@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — k-mers/s ingested into Countgraph (k=20, N=4) on B200, beside the reference CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # our arm
     python bench.py --impl reference [--gpus N] [--steps K] ...    # reference CPU arm (rank 0 only)
 
 Workload (BASELINE.json metric; SURVEY.md §8d): Countgraph/ByteStorage k=20, N=4 tables of ~1e8 bytes
@@ -409,6 +409,37 @@ def secondary_legs(cabi, sk, host, dev, local_rank, n_query=400_000):
     return out
 
 
+DUMP_SAMPLE_PER_TABLE = 1 << 21
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(sk, kmers, out_dir, seed=20240601):
+    """What the last timed step handed its caller, as .npy files for comparing two builds output for output: the k-mers it
+    ingested; n_occupied, n_unique_kmers and the number of bigcount entries; the four counter tables (a histogram of every
+    counter, plus the counters at fixed seeded positions: the full tables are 400 MB); and the bigcount map itself when it
+    has entries (at the bench's 30x coverage no counter reaches 255, so it stays empty)."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    keys, vals = sk.bigcounts()
+    out = {"kmers": np.array([kmers], dtype=np.float64),
+           "stats": np.array(list(sk.stats()) + [len(keys)], dtype=np.float64)}
+    for i in range(N_TABLES):
+        t = sk.table(i)
+        out["table%d_histogram" % i] = np.bincount(t, minlength=256).astype(np.float64)
+        idx = np.sort(rng.choice(len(t), size=min(len(t), DUMP_SAMPLE_PER_TABLE), replace=False))
+        out["table%d_sample" % i] = t[idx].astype(np.float32)
+        del t
+    if len(keys):
+        order = np.argsort(keys, kind="stable")
+        out["bigcount_keys"] = keys[order].astype(np.float64)   # 2-bit hashes of k = 20: below 2**40, exact in float64
+        out["bigcount_values"] = vals[order].astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_MAX_BYTES))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def merge_check(cabi, dist, torch, group_cls, rank, world, local_rank, n_reads=125_000):
     """N > 1: every rank ingests its own fixed batch into a fresh replica, the replicas are merged over NVLink exactly as in
     the timed region; all ranks must then hold identical tables, and rank 0 compares them with ONE sketch fed every rank's
@@ -635,6 +666,14 @@ def run_ours(args):
                "sample": "%d synthetic 150 bp reads (%d k-mers), same table shape, one timed consume_seqfile with %d "
                          "threads sharing one parser" % (args.cpu_reads, kmers_c, threads)}
 
+    if args.dump_outputs and rank == 0:
+        # the tables the last timed step of the hbm leg left behind: replay its job up to that step on an empty sketch
+        last = ((args.warmup + P - 1) // P) * P + args.steps - 1
+        sk.reset()
+        for s in range(last - last % P, last + 1):
+            kmers_last = sk.consume_batch(dev[s % P])
+        dump_outputs(sk, kmers_last, args.dump_outputs)
+
     if rank == 0:
         bases = R * READ_LEN
         line = {
@@ -804,6 +843,7 @@ def main():
     ap.add_argument("--no-file", action="store_true", help="skip the e2e_file and secondary legs")
     ap.add_argument("--check-reads", type=int, default=250_000, help="reads of the parity_check batch")
     ap.add_argument("--file-leg", action="store_true", help="internal: run the e2e_file leg alone and print its dictionary")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     if args.file_leg:
         emit(file_leg(args, int(os.environ.get("KMGPU_DEVICE", "0"))))

@@ -1,6 +1,7 @@
 """Shared parity checks: run one golden case (tests/golden/golden.json, produced by the compiled reference)
 through an implementation and compare every recorded output bit for bit."""
 import hashlib
+import json
 import os
 import struct
 
@@ -22,6 +23,13 @@ def reads_of(fn):
 
 def md5(b):
     return hashlib.md5(bytes(b)).hexdigest()
+
+
+def load_port_golden():
+    """tests/golden/port_golden.json: the reference's outputs for inputs beyond golden.json, written by
+    tests/golden/make_port_golden.py"""
+    with open(os.path.join(HERE, "golden", "port_golden.json")) as fh:
+        return json.load(fh)
 
 
 def f32(hexstr):

@@ -7,7 +7,12 @@ import numpy as np
 import pytest
 
 import oracle_lib as ol
-from common import OracleImpl, check_case, reads_of, md5
+from common import OracleImpl, check_case, load_port_golden, reads_of, md5
+
+
+@pytest.fixture(scope="module")
+def port_golden():
+    return load_port_golden()
 
 
 # ---- known answers held by the reference's own tests ------------------------------------------------
@@ -201,26 +206,47 @@ def test_test_parser_matches_reference_parser(golden):
         assert md5("\n".join(seqs).encode()) == want["md5"], fn
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="compiled reference (oracle/_ref) not built here")
-def test_oracle_vs_live_reference_random(tmp_path):
-    """Differential run against the live reference on fresh random inputs (beyond the committed goldens)."""
+def random_trials():
+    """six fresh random inputs beyond the committed goldens: (class, k, table sizes, reads)"""
     from common import synth_reads
     rng = np.random.default_rng(99)
     for trial in range(6):
         cls = ["Countgraph", "SmallCountgraph", "Nodegraph", "Counttable", "SmallCounttable", "Nodetable"][trial]
         k = int(rng.integers(5, 33))
         sizes = ol.primes_near_x(int(rng.integers(1, 5)), int(rng.integers(500, 20000)))
-        reads = synth_reads(100 + trial, 300, 80, 2000, err=0.02, with_n=True)
+        yield cls, k, sizes, synth_reads(100 + trial, 300, 80, 2000, err=0.02, with_n=True)
+
+
+def random_trial_outputs(cls, k, sizes, reads):
+    """what the oracle port computes for one trial: k-mers consumed, n_unique_kmers, n_occupied, md5 of every table"""
+    o = ol.Oracle(cls, k, sizes)
+    if cls in ("Countgraph", "Counttable"):
+        o.set_use_bigcount(True)
+    kmers = o.consume_reads(reads)
+    return {"kmers": int(kmers), "n_unique_kmers": int(o.n_unique_kmers()), "n_occupied": int(o.n_occupied()),
+            "table_md5": [md5(o.table(i)) for i in range(len(sizes))]}, o
+
+
+def test_oracle_vs_live_reference_random(tmp_path, port_golden):
+    """Differential run against the reference on fresh random inputs (beyond the committed goldens): the reference's outputs
+    stored in tests/golden/port_golden.json, and the live reference too where oracle/_ref is built."""
+    want = port_golden["random"]
+    trials = list(random_trials())
+    assert len(want) == len(trials)
+    for trial, ((cls, k, sizes, reads), w) in enumerate(zip(trials, want)):
+        got, o = random_trial_outputs(cls, k, sizes, reads)
+        assert (cls, k, sizes) == (w["cls"], w["k"], w["sizes"])
+        assert got == {key: w[key] for key in got}, cls
+        if not ol.have_ref():
+            continue
         p = str(tmp_path / ("t%d.fa" % trial))
         with open(p, "w") as fh:
             for i, r in enumerate(reads):
                 fh.write(">%d\n%s\n" % (i, r))
         ref = ol.Ref(cls, k, sizes)
-        o = ol.Oracle(cls, k, sizes)
         if cls in ("Countgraph", "Counttable"):
             ref.set_use_bigcount(True)
-            o.set_use_bigcount(True)
-        assert ref.consume_seqfile(p)[1] == o.consume_reads(reads)
+        assert ref.consume_seqfile(p)[1] == got["kmers"]
         assert ref.n_unique_kmers() == o.n_unique_kmers() and ref.n_occupied() == o.n_occupied()
         for i in range(len(sizes)):
             assert np.array_equal(ref.table(i), o.table(i))
@@ -246,13 +272,30 @@ def test_diginorm_reproduces_reference_script_md5s(datadir):
         assert hashlib.md5(out.encode()).hexdigest() == want
 
 
-def test_hll_registers_restatement_equals_reference(datadir):
-    """ko_hll_consume (the restatement of HLLCounter::add / consume_string) against the compiled reference's HLLCounter:
-    identical registers on random-20-a.fa (consume_seqfile cleans the reads) and on strings fed one by one"""
-    if not ol.have_ref():
-        pytest.skip("oracle/_ref not built")
+HLL_SHAPES = ((20, 14), (32, 10), (41, 16), (5, 4))
+
+
+def hll_outputs(datadir):
+    """the restatement's HLL registers on random-20-a.fa for every (k, p) of HLL_SHAPES: the whole file cleaned, and its first
+    50 reads fed one by one — (reads, k-mers, md5 of the registers) each"""
     reads = ol.read_fastx(os.path.join(datadir, "random-20-a.fa"))
-    for k, p in ((20, 14), (32, 10), (41, 16), (5, 4)):
+    out = []
+    for k, p in HLL_SHAPES:
+        regs, n = ol.hll_consume(reads, k, p, clean=True)
+        regs2, n2 = ol.hll_consume(reads[:50], k, p, clean=True)
+        out.append({"k": k, "p": p, "reads": len(reads), "kmers": int(n), "md5": md5(regs), "kmers_50": int(n2), "md5_50": md5(regs2)})
+    return out
+
+
+def test_hll_registers_restatement_equals_reference(datadir, port_golden):
+    """ko_hll_consume (the restatement of HLLCounter::add / consume_string) against the reference's HLLCounter: identical
+    registers on random-20-a.fa (consume_seqfile cleans the reads) and on strings fed one by one — the reference's registers
+    as stored in tests/golden/port_golden.json, and the compiled reference itself where oracle/_ref is built"""
+    assert hll_outputs(datadir) == port_golden["hll"]
+    if not ol.have_ref():
+        return
+    reads = ol.read_fastx(os.path.join(datadir, "random-20-a.fa"))
+    for k, p in HLL_SHAPES:
         ref = ol.RefHLL(p, k)
         nr, nk = ref.consume_seqfile(os.path.join(datadir, "random-20-a.fa"))
         regs, n = ol.hll_consume(reads, k, p, clean=True)
