@@ -270,7 +270,8 @@ typedef struct kmgpu_shard kmgpu_shard_t;
 int kmgpu_shard_create(int storage, int hash, int ksize, int n_tables, const uint64_t* full_sizes, int device,
                        int rank, int world, uint64_t max_positions_per_route, kmgpu_shard_t** out);
 int kmgpu_shard_destroy(kmgpu_shard_t* s);
-/* the local sketch holding this rank's slices (downloads, queries by local bin work on it as on any sketch) */
+/* the local sketch holding this rank's slices (table downloads work on it as on any sketch; the counts of k-mers come from
+ * query rounds, below) */
 kmgpu_t* kmgpu_shard_local(kmgpu_shard_t* s);
 int kmgpu_shard_slice(kmgpu_shard_t* s, int table, uint64_t* lo, uint64_t* hi);
 /* n_occupied of this rank's slices, this rank's share of n_unique_kmers, bytes of its receive store */
@@ -285,6 +286,32 @@ int kmgpu_shard_offsets(kmgpu_shard_t* s);
 int kmgpu_shard_push(kmgpu_shard_t* s);
 int kmgpu_shard_apply(kmgpu_shard_t* s);
 int kmgpu_shard_count_new(kmgpu_shard_t* s, uint64_t* n_new_out);
+
+/* Query rounds: the counts a single sketch would give the k-mers of every rank's reads (get_count, storage.hh:627-649 / :362-379 /
+ * :207-219: the minimum over the N tables, whose bins live on different ranks).  The first three steps are those of an ingest round:
+ *     kmgpu_shard_route    kmgpu_shard_offsets    kmgpu_shard_push
+ *     kmgpu_shard_lookup   every owner overwrites each record of its arena with the counter it addresses (in place: the answer
+ *                          replaces the bin bits, the position stays); tables, n_occupied and n_unique are not touched.  A round
+ *                          this owner refused fails here with KMGPU_ENOMEM, like kmgpu_shard_apply.
+ *     kmgpu_shard_pull     every sender reads its answered records back from the owners over NVLink and keeps, per position of its
+ *                          reads, the minimum over the tables.  KMGPU_ENOMEM (and no counts) if an owner it sent records to refused.
+ * again with a barrier (provided by the caller) after each step.  The getters below then work on this rank's reads of the round,
+ * as last passed to kmgpu_shard_route (nothing restages the local sketch between the route and them); their layouts and values
+ * equal the single-sketch calls named beside them, without bigcount.  Before a pull they fail with KMGPU_EINVAL. */
+int kmgpu_shard_lookup(kmgpu_shard_t* s);
+int kmgpu_shard_pull(kmgpu_shard_t* s);
+/* kmgpu_kmer_counts: counts_out holds sum(max(0, len_r - k + 1)) entries */
+int kmgpu_shard_kmer_counts(kmgpu_shard_t* s, uint16_t* counts_out, uint64_t* n_kmers_out);
+/* kmgpu_read_medians (each output may be NULL) / kmgpu_median_at_least / kmgpu_trim_batch: one entry per read of the route call */
+int kmgpu_shard_read_medians(kmgpu_shard_t* s, uint16_t* median_out, float* average_out, float* stddev_out, uint32_t* n_kmers_out);
+int kmgpu_shard_median_at_least(kmgpu_shard_t* s, uint32_t cutoff, uint8_t* out);
+int kmgpu_shard_trim(kmgpu_shard_t* s, uint32_t abund, int below, uint32_t* trim_pos_out);
+/* kmgpu_abundance_distribution for one run of reads of this rank, ACCUMULATED into hist (65536 entries): `tracking` (a BIT shard
+ * with the counting shard's hash kind and k) has run an ingest round on the run, up to kmgpu_shard_count_new, and `counts` a query
+ * round on the same run; hist[count] += 1 for every k-mer of the run that was new in `tracking`.  Summed over the ranks and runs
+ * it equals one kmgpu_abundance_distribution fed the rounds in stream order.  KMGPU_EINVAL when the shards live on different
+ * devices, differ in max_positions, hash kind or k, or last routed different reads. */
+int kmgpu_shard_abundance_hist(kmgpu_shard_t* counts, kmgpu_shard_t* tracking, uint64_t* hist);
 
 /* ---- measurement -----------------------------------------------------------------------
  * Device time (ms) and launch count of the ingest kernel accumulated since the last reset, measured

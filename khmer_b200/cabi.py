@@ -37,7 +37,8 @@ SYMBOLS = [
     "kmgpu_timer_start", "kmgpu_timer_stop", "kmgpu_slice_range", "kmgpu_alloc_pinned", "kmgpu_free_pinned",
     "kmgpu_shard_create", "kmgpu_shard_destroy", "kmgpu_shard_local", "kmgpu_shard_slice", "kmgpu_shard_ipc_export",
     "kmgpu_shard_ipc_attach", "kmgpu_shard_attach_local", "kmgpu_shard_route", "kmgpu_shard_offsets", "kmgpu_shard_push", "kmgpu_shard_apply",
-    "kmgpu_shard_count_new", "kmgpu_shard_stats", "kmgpu_hll_create", "kmgpu_hll_destroy", "kmgpu_hll_consume",
+    "kmgpu_shard_count_new", "kmgpu_shard_stats", "kmgpu_shard_lookup", "kmgpu_shard_pull", "kmgpu_shard_kmer_counts",
+    "kmgpu_shard_read_medians", "kmgpu_shard_median_at_least", "kmgpu_shard_trim", "kmgpu_shard_abundance_hist", "kmgpu_hll_create", "kmgpu_hll_destroy", "kmgpu_hll_consume",
     "kmgpu_hll_get_registers", "kmgpu_hll_merge_registers",
 ]
 
@@ -146,6 +147,13 @@ def lib():
         L.kmgpu_shard_push.argtypes = [C.c_void_p]
         L.kmgpu_shard_count_new.argtypes = [C.c_void_p, u64p]
         L.kmgpu_shard_stats.argtypes = [C.c_void_p, u64p, u64p, u64p]
+        L.kmgpu_shard_lookup.argtypes = [C.c_void_p]
+        L.kmgpu_shard_pull.argtypes = [C.c_void_p]
+        L.kmgpu_shard_kmer_counts.argtypes = [C.c_void_p, C.c_void_p, u64p]
+        L.kmgpu_shard_read_medians.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kmgpu_shard_median_at_least.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+        L.kmgpu_shard_trim.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p]
+        L.kmgpu_shard_abundance_hist.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -525,6 +533,8 @@ class Shard:
         arr = (C.c_uint64 * len(self.full_sizes))(*self.full_sizes)
         self.h = C.c_void_p()
         self.storage, self.rank, self.world, self.max_positions = storage, rank, world, max_positions
+        self.ksize = ksize
+        self._routed = np.zeros(1, dtype=np.uint64)   # offsets of the reads of the last route call
         check(lib().kmgpu_shard_create(storage, hashkind, ksize, len(self.full_sizes), arr, device, rank, world, max_positions,
                                        C.byref(self.h)))
         # the local sketch is owned by the shard: wrap it without taking ownership
@@ -563,6 +573,7 @@ class Shard:
     def route(self, reads, clean=True):
         buf, off = as_reads(reads)
         n = C.c_uint64()
+        self._routed = off
         check(lib().kmgpu_shard_route(self.h, _ptr(buf), _ptr(off), len(off) - 1, CLEAN if clean else 0, C.byref(n)))
         return n.value
 
@@ -580,6 +591,42 @@ class Shard:
         n = C.c_uint64()
         check(lib().kmgpu_shard_count_new(self.h, C.byref(n)))
         return n.value
+
+    # -- query rounds: route, offsets, push, then lookup and pull; the getters answer for this rank's reads of the last route
+    def lookup(self):
+        """owner: answer every record this rank was sent with the counter it addresses (tables are not changed)"""
+        check(lib().kmgpu_shard_lookup(self.h))
+
+    def pull(self):
+        """sender: read the answers back; count per k-mer = the minimum over the tables"""
+        check(lib().kmgpu_shard_pull(self.h))
+
+    def kmer_counts(self):
+        off = self._routed
+        lens = (off[1:] - off[:-1]).astype(np.int64)
+        out = np.zeros(max(int(np.maximum(lens - self.ksize + 1, 0).sum()), 1), dtype=np.uint16)
+        n = C.c_uint64()
+        check(lib().kmgpu_shard_kmer_counts(self.h, _ptr(out), C.byref(n)))
+        return out[:n.value]
+
+    def read_medians(self):
+        nr = len(self._routed) - 1
+        med = np.zeros(nr, dtype=np.uint16)
+        avg = np.zeros(nr, dtype=np.float32)
+        sd = np.zeros(nr, dtype=np.float32)
+        nk = np.zeros(nr, dtype=np.uint32)
+        check(lib().kmgpu_shard_read_medians(self.h, _ptr(med), _ptr(avg), _ptr(sd), _ptr(nk)))
+        return med, avg, sd, nk
+
+    def median_at_least(self, cutoff):
+        out = np.zeros(len(self._routed) - 1, dtype=np.uint8)
+        check(lib().kmgpu_shard_median_at_least(self.h, int(cutoff), _ptr(out)))
+        return out
+
+    def trim(self, abund, below=False):
+        out = np.zeros(len(self._routed) - 1, dtype=np.uint32)
+        check(lib().kmgpu_shard_trim(self.h, int(abund), int(below), _ptr(out)))
+        return out
 
     def stats(self):
         """(n_occupied of this rank's slices, this rank's share of n_unique_kmers, bytes of the receive store)"""
@@ -600,6 +647,15 @@ class Shard:
         if self.storage == NIBBLE:
             return t if last else t[: (hi - lo) // 2]
         return t if last else t[: (hi - lo) // 8]
+
+
+def shard_abundance_hist(counts, tracking, hist=None):
+    """abundance_distribution over the run both shards last routed: `tracking` ingested it (up to count_new), `counts` answered it
+    (pull).  Accumulates into hist (uint64[65536])."""
+    if hist is None:
+        hist = np.zeros(65536, dtype=np.uint64)
+    check(lib().kmgpu_shard_abundance_hist(counts.h, tracking.h, _ptr(hist)))
+    return hist
 
 
 def attach_local_shards(shards):

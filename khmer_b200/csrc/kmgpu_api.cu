@@ -2062,6 +2062,22 @@ extern "C" int kmgpu_get_counts(kmgpu_t* h, const uint64_t* hashes, uint64_t n, 
 // ------------------------------------------------------------------------------------------------------
 // per-k-mer and per-read queries over sequences
 // ------------------------------------------------------------------------------------------------------
+// the values of every read's k-mers, read after read, from an array over a chunk's positions (read j starts at offs[j]);
+// returns how many were written
+template <typename T>
+static uint64_t compact_kmers(const T* per_pos, const uint32_t* offs, size_t n_reads, int k, T* out)
+{
+    uint64_t w = 0;
+    for (size_t j = 0; j < n_reads; j++) {
+        const uint32_t s = offs[j], e = offs[j + 1];
+        if (e - s < (uint32_t)k) continue;
+        const uint32_t n = e - s - k + 1;
+        memcpy(out + w, per_pos + s, sizeof(T) * n);
+        w += n;
+    }
+    return w;
+}
+
 static int per_kmer_query(kmgpu_sketch* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
                           uint16_t* counts_out, uint64_t* hashes_out, uint64_t* n_kmers_out)
 {
@@ -2098,14 +2114,11 @@ static int per_kmer_query(kmgpu_sketch* h, const char* seqs, const uint64_t* off
             CK(cudaMemcpyAsync(hh.data(), h->d_hashes.p, 8ull * cd.n_pos, cudaMemcpyDeviceToHost, h->stream));
         }
         CK(cudaStreamSynchronize(h->stream));
-        for (size_t j = 0; j + 1 < c.offs.size(); j++) {
-            uint32_t s = c.offs[j], e = c.offs[j + 1];
-            if (e - s < (uint32_t)h->k) continue;
-            uint32_t n = e - s - h->k + 1;
-            if (want_c) memcpy(counts_out + w, hc.data() + s, 2ull * n);
-            if (hashes_out) memcpy(hashes_out + w, hh.data() + s, 8ull * n);
-            w += n;
-        }
+        const size_t nr = c.offs.size() - 1;
+        uint64_t n = 0;
+        if (want_c) n = compact_kmers(hc.data(), c.offs.data(), nr, h->k, counts_out + w);
+        if (hashes_out) n = compact_kmers(hh.data(), c.offs.data(), nr, h->k, hashes_out + w);
+        w += n;
     }
     if (n_kmers_out) *n_kmers_out = w;
     return KMGPU_OK;
@@ -2127,24 +2140,20 @@ extern "C" int kmgpu_kmer_hashes(kmgpu_t* h, const char* seqs, const uint64_t* o
     return per_kmer_query(h, seqs, offsets, n_reads, flags, nullptr, hashes_out, n_kmers_out);
 }
 
-// one staged chunk of whole reads: counts per position, then one warp per read (median / mean / stddev, or median_at_least)
-static int read_stats_chunk(kmgpu_sketch* h, const ChunkDev& cd, uint64_t r0, uint32_t nb, uint16_t* median_out, float* average_out,
-                            float* stddev_out, uint32_t* n_kmers_out, bool at_least, uint32_t cutoff, uint8_t* at_least_out)
+// one staged chunk of whole reads with its counts per position: one warp per read (median / mean / stddev, or median_at_least),
+// results written from read r0 on
+static int read_stats_counts(kmgpu_sketch* h, const uint16_t* counts, const ChunkDev& cd, uint64_t r0, uint16_t* median_out,
+                             float* average_out, float* stddev_out, uint32_t* n_kmers_out, bool at_least, uint32_t cutoff,
+                             uint8_t* at_least_out)
 {
-    HashCfg H{h->hash, h->k};
     cudaStream_t st = h->stream;
     uint32_t nr = cd.n_reads;
-    CKR(h->d_counts.ensure(std::max<uint32_t>(cd.n_pos, 1)));
-    if (cd.n_pos) {
-        launch_counts(0, h->dev, H, make_input(cd), h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, st);
-        h->all_launches += 1;
-    }
     CKR(h->d_stat_med.ensure(nr));
     CKR(h->d_stat_f.ensure(2ull * nr));
     CKR(h->d_stat_n.ensure(nr));
     CKR(h->d_stat_b.ensure(nr));
     bool want_med = !at_least;
-    k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, want_med ? h->d_stat_med.p : nullptr,
+    k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(counts, cd.offs, nr, h->k, want_med ? h->d_stat_med.p : nullptr,
                                               want_med ? h->d_stat_f.p : nullptr, want_med ? h->d_stat_f.p + nr : nullptr,
                                               h->d_stat_n.p, cutoff, at_least ? h->d_stat_b.p : nullptr);
     h->all_launches += 1;
@@ -2157,6 +2166,34 @@ static int read_stats_chunk(kmgpu_sketch* h, const ChunkDev& cd, uint64_t r0, ui
         CK(cudaMemcpyAsync(at_least_out + r0, h->d_stat_b.p, nr, cudaMemcpyDeviceToHost, st));
     }
     if (n_kmers_out) CK(cudaMemcpyAsync(n_kmers_out + r0, h->d_stat_n.p, 4ull * nr, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return KMGPU_OK;
+}
+
+// one staged chunk of whole reads: counts per position, then read_stats_counts
+static int read_stats_chunk(kmgpu_sketch* h, const ChunkDev& cd, uint64_t r0, uint32_t nb, uint16_t* median_out, float* average_out,
+                            float* stddev_out, uint32_t* n_kmers_out, bool at_least, uint32_t cutoff, uint8_t* at_least_out)
+{
+    HashCfg H{h->hash, h->k};
+    CKR(h->d_counts.ensure(std::max<uint32_t>(cd.n_pos, 1)));
+    if (cd.n_pos) {
+        launch_counts(0, h->dev, H, make_input(cd), h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, h->stream);
+        h->all_launches += 1;
+    }
+    return read_stats_counts(h, h->d_counts.p, cd, r0, median_out, average_out, stddev_out, n_kmers_out, at_least, cutoff, at_least_out);
+}
+
+// the same for trim_on_abundance / trim_below_abundance: the length every read keeps
+static int trim_counts(kmgpu_sketch* h, const uint16_t* counts, const ChunkDev& cd, uint64_t r0, uint32_t abund, int below,
+                       uint32_t* trim_pos_out)
+{
+    cudaStream_t st = h->stream;
+    const uint32_t nr = cd.n_reads;
+    CKR(h->d_stat_n.ensure(nr));
+    k_trim_scan<<<(nr + 7) / 8, 256, 0, st>>>(counts, cd.offs, nr, h->k, abund, below, h->d_stat_n.p);
+    h->all_launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(trim_pos_out + r0, h->d_stat_n.p, 4ull * nr, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return KMGPU_OK;
 }
@@ -2247,20 +2284,14 @@ extern "C" int kmgpu_trim_batch(kmgpu_t* h, const char* seqs, const uint64_t* of
     std::vector<ChunkPlan> plan;
     plan_chunks(offsets, n_reads, h->k, chunk_bases(), plan);
     uint64_t r0 = 0;
-    cudaStream_t st = h->stream;
     for (const ChunkPlan& c : plan) {
         ChunkDev cd;
         CKR(stage_chunk(h, seqs, c, flags, &cd, needs_acgt_check(h, flags)));
-        const uint32_t nr = cd.n_reads;
         CKR(h->d_counts.ensure(std::max<uint32_t>(cd.n_pos, 1)));
-        if (cd.n_pos) launch_counts(0, h->dev, H, make_input(cd), h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, st);
-        CKR(h->d_stat_n.ensure(nr));
-        k_trim_scan<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, abund, below, h->d_stat_n.p);
-        h->all_launches += 2;
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(trim_pos_out + r0, h->d_stat_n.p, 4ull * nr, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        r0 += nr;
+        if (cd.n_pos) launch_counts(0, h->dev, H, make_input(cd), h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, h->stream);
+        h->all_launches += 1;
+        CKR(trim_counts(h, h->d_counts.p, cd, r0, abund, below, trim_pos_out));
+        r0 += cd.n_reads;
     }
     return KMGPU_OK;
 }
@@ -3055,6 +3086,13 @@ struct kmgpu_shard {
     bool exact_s = false;
     bool attached = false, ipc = false;
     uint64_t n_unique = 0;   // k-mers of this rank's reads that were new
+    // the reads of the last route call: they stay staged in slot 0 of the local sketch (nothing else stages there between a
+    // route and the getters of its round); offs covers every read of the call, n_pos its bases
+    ChunkDev q;
+    DevBuf<uint32_t> q_offs;   // those offsets when staging dropped empty reads at either end of the range
+    DevBuf<uint8_t> planes;    // pull: the answers, one byte per (table, position), planes of max_positions bytes
+    bool pulled = false;       // the last route was answered (kmgpu_shard_pull): the local sketch's d_counts hold its counts
+    bool counted = false;      // the last route was ingested up to kmgpu_shard_count_new: its d_newbits hold the new positions
 };
 
 extern "C" int kmgpu_shard_destroy(kmgpu_shard_t* s);
@@ -3182,6 +3220,8 @@ extern "C" int kmgpu_shard_destroy(kmgpu_shard_t* s)
     if (s->recv_off) cudaFree(s->recv_off);
     if (s->flags) cudaFree(s->flags);
     if (s->newbits) cudaFree(s->newbits);
+    s->q_offs.release();
+    s->planes.release();
     s->sb_off.release();
     s->sb_cnt.release();
     s->rec_s.release();
@@ -3310,10 +3350,13 @@ extern "C" int kmgpu_shard_route(kmgpu_shard_t* s, const char* seqs, const uint6
     CK(cudaMemsetAsync(s->cur_s.p, 0, (size_t)n_sb * 4, st));
     CK(cudaMemsetAsync(h->d_ctrl, 0, sizeof(Ctrl), st));
     s->exact_s = false;
+    s->q = ChunkDev{};
+    s->pulled = s->counted = false;
     uint64_t n_kmers = 0;
     if (last > first) {
         ChunkDev cd;
         CKR(stage_range(h, seqs, offsets, n_reads, first, last, flags, &cd, needs_acgt_check(h, flags), 0, st));
+        s->q = cd;
         Input in = make_input(cd);
         CK(cudaEventRecord(h->ev0, st));
         const HashCfg H{h->hash, h->k};
@@ -3372,6 +3415,17 @@ extern "C" int kmgpu_shard_route(kmgpu_shard_t* s, const char* seqs, const uint6
             if (h->h_ctrl->overflow) return fail(KMGPU_ECUDA, "internal: regrouping run overflowed");
         }
         CK(cudaEventRecord(h->ev1, st));
+    }
+    if (s->q.n_reads != n_reads) {
+        // the staged range leaves out empty reads at its ends (or there was nothing to stage): the per-read getters of a query
+        // round need the offsets of every read
+        std::vector<uint32_t> o(n_reads + 1);
+        for (uint64_t r = 0; r <= n_reads; r++) o[r] = (uint32_t)(offsets[r] - first);
+        CKR(s->q_offs.ensure(n_reads + 1));
+        CK(cudaMemcpyAsync(s->q_offs.p, o.data(), (n_reads + 1) * 4, cudaMemcpyHostToDevice, st));
+        CK(cudaStreamSynchronize(st));
+        s->q.offs = s->q_offs.p;
+        s->q.n_reads = (uint32_t)n_reads;
     }
     ShardPeers PP;
     shard_peers(s, &PP);
@@ -3532,7 +3586,178 @@ extern "C" int kmgpu_shard_count_new(kmgpu_shard_t* s, uint64_t* n_new_out)
     CK(cudaGetLastError());
     CKR(read_ctrl(h));
     s->n_unique += h->h_ctrl->n_unique;
+    s->counted = true;
     if (n_new_out) *n_new_out = h->h_ctrl->n_unique;
+    return KMGPU_OK;
+}
+
+// lookup (owner, query rounds): every record of my arena gets the counter it addresses in my slices, in place.  Tables, counters
+// and the new-position bitmap are not touched.
+extern "C" int kmgpu_shard_lookup(kmgpu_shard_t* s)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(set_device(h->device));
+    if (h->kind == BYTE && h->use_bigcount) return fail(KMGPU_EUNSUPPORTED, "bigcount is not maintained by sharded sketches");
+    cudaStream_t st = h->stream;
+    const size_t n_dem = (size_t)s->n_sb_local * s->world;
+    if (s->refused) {
+        // the refusal flag stays up: the senders read it in kmgpu_shard_pull (kmgpu_shard_offsets writes it anew every round)
+        s->refused = false;
+        CK(cudaMemsetAsync(s->demand, 0, n_dem * 4, st));
+        CK(cudaStreamSynchronize(st));
+        return fail(KMGPU_ENOMEM, "rank %d was sent %llu records in one round, its arena holds %llu (this rank owns far more than its share of the "
+                                  "k-mers): the round was not answered; create the shards with a smaller max_positions_per_route",
+                    s->rank, (unsigned long long)s->received, (unsigned long long)s->arena);
+    }
+    if (s->received) {
+        const int sbb = BKT_SHIFT + s->GF.L.sb_shift;
+        const dim3 grid(s->n_sb_local, 8);
+        if (h->kind == BYTE) k_shard_lookup<BYTE><<<grid, 256, 0, st>>>(s->geom, h->dev, s->rec1, s->sb_off.p, s->sb_cnt.p, sbb);
+        else if (h->kind == NIBBLE) k_shard_lookup<NIBBLE><<<grid, 256, 0, st>>>(s->geom, h->dev, s->rec1, s->sb_off.p, s->sb_cnt.p, sbb);
+        else k_shard_lookup<BIT><<<grid, 256, 0, st>>>(s->geom, h->dev, s->rec1, s->sb_off.p, s->sb_cnt.p, sbb);
+        h->all_launches += 1;
+        CK(cudaGetLastError());
+    }
+    CK(cudaMemsetAsync(s->demand, 0, n_dem * 4, st));   // as after an apply: ranks without reads in a later round post nothing
+    CK(cudaStreamSynchronize(st));
+    return KMGPU_OK;
+}
+
+// pull (sender, query rounds): read my answered records back from every owner; count per position = min over the tables
+extern "C" int kmgpu_shard_pull(kmgpu_shard_t* s)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(set_device(h->device));
+    cudaStream_t st = h->stream;
+    s->pulled = false;
+    const uint32_t n_pos = s->q.n_pos;
+    CKR(h->d_counts.ensure(std::max<uint32_t>(n_pos, 1)));
+    if (n_pos) {
+        const uint64_t stride = s->max_positions;
+        if (!try_ensure(s->planes, (size_t)s->nt * stride)) return fail(KMGPU_ENOMEM, "no room for the answers of a query round");
+        ShardPeers PP;
+        shard_peers(s, &PP);
+        const Store src = s->exact_s ? Store{s->rec_s.p, s->off_s.p, s->cur_s.p, 0, 0} : Store{s->rec_s.p, nullptr, s->cur_s.p, s->GF.L.cap1, 0};
+        CK(cudaMemsetAsync(&h->d_ctrl->overflow, 0, sizeof(unsigned long long), st));
+        k_shard_pull<<<dim3(s->GF.n_sb, 8), 256, 0, st>>>(s->geom, src, PP, BKT_SHIFT + s->GF.L.sb_shift,
+                                                         (uint32_t)((uint64_t)s->rank * s->max_positions), stride, s->planes.p,
+                                                         &h->d_ctrl->overflow);
+        h->all_launches += 1;
+        CK(cudaGetLastError());
+        CKR(read_ctrl(h));
+        if (h->h_ctrl->overflow)
+            return fail(KMGPU_ENOMEM, "rank %d: an owner's arena could not hold this round (see its kmgpu_shard_lookup): no counts", s->rank);
+        k_shard_fold<<<(unsigned)std::min<uint32_t>((n_pos + 255) / 256, 148 * 16), 256, 0, st>>>(s->planes.p, s->nt, stride, n_pos,
+                                                                                                   h->d_counts.p);
+        h->all_launches += 1;
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(st));
+    }
+    s->pulled = true;
+    return KMGPU_OK;
+}
+
+static int shard_pulled(const kmgpu_shard* s)
+{
+    if (!s->pulled) return fail(KMGPU_EINVAL, "no query round was pulled since the last kmgpu_shard_route");
+    return KMGPU_OK;
+}
+
+extern "C" int kmgpu_shard_kmer_counts(kmgpu_shard_t* s, uint16_t* counts_out, uint64_t* n_kmers_out)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    if (n_kmers_out) *n_kmers_out = 0;
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(shard_pulled(s));
+    const uint32_t nr = s->q.n_reads;
+    if (nr == 0) return KMGPU_OK;
+    if (!counts_out) return fail(KMGPU_EINVAL, "null output");
+    CKR(set_device(h->device));
+    std::vector<uint32_t> offs(nr + 1);
+    std::vector<uint16_t> hc(s->q.n_pos);
+    CK(cudaMemcpyAsync(offs.data(), s->q.offs, 4ull * (nr + 1), cudaMemcpyDeviceToHost, h->stream));
+    if (s->q.n_pos) CK(cudaMemcpyAsync(hc.data(), h->d_counts.p, 2ull * s->q.n_pos, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const uint64_t w = compact_kmers(hc.data(), offs.data(), nr, h->k, counts_out);
+    if (n_kmers_out) *n_kmers_out = w;
+    return KMGPU_OK;
+}
+
+extern "C" int kmgpu_shard_read_medians(kmgpu_shard_t* s, uint16_t* median_out, float* average_out, float* stddev_out, uint32_t* n_kmers_out)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(shard_pulled(s));
+    if (s->q.n_reads == 0) return KMGPU_OK;
+    CKR(set_device(h->device));
+    return read_stats_counts(h, h->d_counts.p, s->q, 0, median_out, average_out, stddev_out, n_kmers_out, false, 0, nullptr);
+}
+
+extern "C" int kmgpu_shard_median_at_least(kmgpu_shard_t* s, uint32_t cutoff, uint8_t* out)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(shard_pulled(s));
+    if (s->q.n_reads == 0) return KMGPU_OK;
+    if (!out) return fail(KMGPU_EINVAL, "null output");
+    CKR(set_device(h->device));
+    return read_stats_counts(h, h->d_counts.p, s->q, 0, nullptr, nullptr, nullptr, nullptr, true, cutoff, out);
+}
+
+extern "C" int kmgpu_shard_trim(kmgpu_shard_t* s, uint32_t abund, int below, uint32_t* trim_pos_out)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(shard_pulled(s));
+    if (s->q.n_reads == 0) return KMGPU_OK;
+    if (!trim_pos_out) return fail(KMGPU_EINVAL, "null output");
+    CKR(set_device(h->device));
+    return trim_counts(h, h->d_counts.p, s->q, 0, abund, below, trim_pos_out);
+}
+
+// abundance_distribution over one run of reads: `tracking` has ingested it (up to count_new: its local sketch holds this rank's
+// new positions), `counts` has answered it (pull): hist[count] += 1 for every new position
+extern "C" int kmgpu_shard_abundance_hist(kmgpu_shard_t* counts, kmgpu_shard_t* tracking, uint64_t* hist)
+{
+    if (!counts || !tracking || !hist) return fail(KMGPU_EINVAL, "null argument");
+    if (counts == tracking) return fail(KMGPU_EINVAL, "tracking shard must differ from the counting shard");
+    kmgpu_sketch* c = counts->local;
+    kmgpu_sketch* t = tracking->local;
+    if (c->device != t->device) return fail(KMGPU_EINVAL, "shards live on different devices");
+    if (counts->max_positions != tracking->max_positions)
+        return fail(KMGPU_EINVAL, "shards were created for different max_positions (%llu, %llu)", (unsigned long long)counts->max_positions,
+                    (unsigned long long)tracking->max_positions);
+    if (c->hash != t->hash || c->k != t->k) return fail(KMGPU_EINVAL, "the tracking shard must hash k-mers as the counting shard does");
+    kmgpu_sketch* a = c < t ? c : t;
+    kmgpu_sketch* b = c < t ? t : c;
+    std::lock_guard<std::mutex> ga(a->mu);
+    std::lock_guard<std::mutex> gb(b->mu);
+    CKR(shard_pulled(counts));
+    if (!tracking->counted) return fail(KMGPU_EINVAL, "the tracking shard has not counted the new k-mers of its last route (kmgpu_shard_count_new)");
+    if (counts->q.n_pos != tracking->q.n_pos || counts->q.n_reads != tracking->q.n_reads)
+        return fail(KMGPU_EINVAL, "the shards last routed different reads");
+    const uint32_t n_pos = counts->q.n_pos;
+    if (n_pos == 0) return KMGPU_OK;
+    CKR(set_device(c->device));
+    cudaStream_t st = c->stream;
+    CK(cudaStreamSynchronize(t->stream));
+    CKR(c->d_hist.ensure(65536));
+    CK(cudaMemsetAsync(c->d_hist.p, 0, 65536 * 8, st));
+    k_hist<<<148 * 4, 256, 0, st>>>(c->d_counts.p, t->d_newbits.p, n_pos, c->d_hist.p);
+    c->all_launches += 1;
+    CK(cudaGetLastError());
+    std::vector<unsigned long long> hh(65536);
+    CK(cudaMemcpyAsync(hh.data(), c->d_hist.p, 65536 * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (int i = 0; i < 65536; i++) hist[i] += hh[i];
     return KMGPU_OK;
 }
 

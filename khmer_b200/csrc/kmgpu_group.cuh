@@ -1370,5 +1370,79 @@ k_shard_push(const __grid_constant__ ShardGeom G, Store src, const __grid_consta
     for (uint32_t e = blockIdx.y * 256u + threadIdx.x; e < c; e += gridDim.y * 256u) to[e] = __ldcs(from + e);
 }
 
+// ---- query rounds: route, offsets and push as above, then the owner answers every record in place and the sender reads
+//      its answers back.  An answered record keeps its position bits; its low 15 + s bits hold the counter.
+// owner: grid (local super-buckets, Y); the records of super-bucket j are arena[sb_off[j] .. + sb_cnt[j])
+template <int KIND>
+__global__ void __launch_bounds__(256)
+k_shard_lookup(const __grid_constant__ ShardGeom G, const __grid_constant__ SketchDev S, unsigned long long* __restrict__ arena,
+               const unsigned long long* __restrict__ sb_off, const uint32_t* __restrict__ sb_cnt, int sb_bin_shift)
+{
+    const uint32_t j = blockIdx.x;
+    const uint32_t c = sb_cnt[j];
+    if (c == 0) return;
+    int t = 0;
+#pragma unroll 1
+    for (int i = 1; i < G.n_tables; i++)
+        if (j >= G.local_first[i]) t = i;
+    const unsigned long long mask = (1ull << sb_bin_shift) - 1;
+    const uint64_t bin0 = (uint64_t)(j - G.local_first[t]) << sb_bin_shift;
+    const uint8_t* tab = S.tables[t];
+    unsigned long long* rec = arena + sb_off[j];
+    const uint32_t step = gridDim.y * 256u;
+    for (uint32_t e0 = blockIdx.y * 256u + threadIdx.x; e0 < c; e0 += 4 * step) {   // four random table loads in flight per thread
+        unsigned long long r[4];
+        uint32_t v[4];
+#pragma unroll
+        for (int u = 0; u < 4; u++) r[u] = e0 + u * step < c ? rec[e0 + u * step] : 0ull;
+#pragma unroll
+        for (int u = 0; u < 4; u++) v[u] = e0 + u * step < c ? read_counter<KIND>(tab, bin0 | (r[u] & mask)) : 0u;
+#pragma unroll
+        for (int u = 0; u < 4; u++)
+            if (e0 + u * step < c) rec[e0 + u * step] = (r[u] & ~mask) | v[u];
+    }
+}
+
+// sender: grid (global super-buckets, Y), the runs the push wrote; answers land in one byte plane per table (plain stores: every
+// (table, position) has exactly one record).  A run whose owner refused the round sets *refused and is not read.
+__global__ void __launch_bounds__(256)
+k_shard_pull(const __grid_constant__ ShardGeom G, Store src, const __grid_constant__ ShardPeers P, int sb_bin_shift, uint32_t pos_base,
+             uint64_t plane_stride, uint8_t* __restrict__ planes, unsigned long long* refused)
+{
+    const uint32_t g = blockIdx.x;
+    uint32_t c = src.cursor[g];
+    if (c == 0) return;
+    const uint32_t room = src.room(g);
+    if (c > room) c = room;
+    int q;
+    uint32_t j;
+    shard_owner(G, g, &q, &j);
+    if (*P.flags[q] & 1ull) {
+        if (blockIdx.y == 0 && threadIdx.x == 0) atomicOr(refused, 1ull);
+        return;
+    }
+    int t = 0;
+#pragma unroll 1
+    for (int i = 1; i < G.n_tables; i++)
+        if (g >= G.first_sb[i]) t = i;
+    const unsigned long long* from = P.rec[q] + P.recv_off[q][(size_t)j * G.world + G.rank];
+    uint8_t* plane = planes + (size_t)t * plane_stride;
+    const unsigned long long mask = (1ull << sb_bin_shift) - 1;
+    for (uint32_t e = blockIdx.y * 256u + threadIdx.x; e < c; e += gridDim.y * 256u) {
+        const unsigned long long r = __ldcs(from + e);
+        plane[(uint32_t)(r >> sb_bin_shift) - pos_base] = (uint8_t)(r & mask);
+    }
+}
+
+// count per position = min over the tables' planes (get_count, storage.hh:627-649 / :362-379 / :207-219, without bigcount)
+__global__ void k_shard_fold(const uint8_t* __restrict__ planes, int n_tables, uint64_t plane_stride, uint32_t n_pos, uint16_t* __restrict__ counts)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n_pos; p += gridDim.x * blockDim.x) {
+        uint32_t m = planes[p];
+        for (int t = 1; t < n_tables; t++) m = min(m, (uint32_t)planes[(size_t)t * plane_stride + p]);
+        counts[p] = (uint16_t)m;
+    }
+}
+
 }  // namespace kmgpu
 

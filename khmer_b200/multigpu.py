@@ -261,7 +261,9 @@ class ShardedGroup:
     """An address-sharded sketch across ranks: every rank hashes its own reads and groups the counter updates by the owners'
     super-buckets (route), the owners lay out their receive arenas (offsets), the senders write their runs into the owners' HBM
     over NVLink peer memory (push), owners apply what they received (apply); every rank counts which of its k-mers were new
-    (count_new).  Only the barriers between the phases come from `comm`."""
+    (count_new).  A query round takes the same first three steps, then the owners answer every record with its counter in place
+    (lookup) and the senders read the answers back, keeping the minimum over the tables per k-mer (pull).  Only the barriers
+    between the phases come from `comm`."""
 
     def __init__(self, shard, comm=None, device=None):
         self.shard = shard
@@ -277,30 +279,97 @@ class ShardedGroup:
         self.shard.ipc_attach(np.frombuffer(b"".join(parts), dtype=np.uint8).copy())
         self.barrier()
 
-    def consume_reads(self, reads, clean=True):
-        """Collective: every rank passes its own shard of the reads; returns the k-mers this rank hashed."""
+    def _runs(self, reads):
+        """This rank's reads as the runs of its rounds (collective): runs of whole reads of at most max_positions bases, then
+        empty runs up to the number of rounds of the rank with the most — a rank without reads left still takes part."""
         from . import cabi
         buf, off = cabi.as_reads(reads)
         runs = split_by_bases(buf, off, self.shard.max_positions)
         rounds = max(int.from_bytes(p, "little") for p in self.comm.all_gather_bytes(len(runs).to_bytes(8, "little")))
-        kmers = 0
         empty = (np.zeros(0, dtype=np.uint8), np.zeros(1, dtype=np.uint64))
-        for i in range(rounds):
-            if i < len(runs):
-                r0, r1 = runs[i]
-                kmers += self.shard.route((buf, off[r0:r1 + 1]), clean=clean)
-            else:
-                self.shard.route(empty, clean=clean)      # a rank without reads left still posts its (zero) counts
-            self.barrier()          # every owner knows what it will be sent
-            self.shard.offsets()
-            self.barrier()          # every sender can read where its runs go
-            self.shard.push()
-            self.barrier()          # every update of this round sits in its owner's arena
-            self.shard.apply()
-            self.barrier()          # every owner has marked the new positions of the round
-            self.shard.count_new()
-            self.barrier()          # nobody reads a peer's bitmap or store any more: the next round may start
-        return kmers
+        return [(buf, off[r0:r1 + 1]) for r0, r1 in runs] + [empty] * (rounds - len(runs))
+
+    def _ingest_round(self, run, clean):
+        n = self.shard.route(run, clean=clean)
+        self.barrier()          # every owner knows what it will be sent
+        self.shard.offsets()
+        self.barrier()          # every sender can read where its runs go
+        self.shard.push()
+        self.barrier()          # every update of this round sits in its owner's arena
+        self.shard.apply()
+        self.barrier()          # every owner has marked the new positions of the round
+        self.shard.count_new()
+        self.barrier()          # nobody reads a peer's bitmap or store any more: the next round may start
+        return n
+
+    def _query_round(self, run, clean):
+        """route | offsets | push | lookup | pull: afterwards the shard's getters answer for `run`.  A round an owner refused
+        raises on every rank, so that no rank runs on into the next collective alone."""
+        from . import cabi
+        self.shard.route(run, clean=clean)
+        self.barrier()
+        self.shard.offsets()
+        self.barrier()
+        self.shard.push()
+        self.barrier()          # every query of this round sits in its owner's arena
+        err = None
+        try:
+            self.shard.lookup()
+        except cabi.KmgpuError as e:
+            err = e
+        self.barrier()          # every record is answered
+        if err is None:
+            try:
+                self.shard.pull()
+            except cabi.KmgpuError as e:
+                err = e
+        # (also the barrier after pull: no owner's arena or refusal flag is rewritten before every sender has read it)
+        if self.comm.all_reduce_sum(err is not None):
+            raise err or cabi.KmgpuError(4, "another rank's arena could not hold this query round")
+
+    def _query(self, reads, clean, get, dtypes):
+        parts = []
+        for run in self._runs(reads):
+            self._query_round(run, clean)
+            got = get()
+            parts.append(got if isinstance(got, tuple) else (got,))
+        out = tuple(np.concatenate([p[i] for p in parts]) if parts else np.zeros(0, dtype=dt) for i, dt in enumerate(dtypes))
+        return out if len(out) > 1 else out[0]
+
+    def consume_reads(self, reads, clean=True):
+        """Collective: every rank passes its own shard of the reads; returns the k-mers this rank hashed."""
+        return sum(self._ingest_round(run, clean) for run in self._runs(reads))
+
+    # -- queries (collective): every rank passes its own reads and gets the answers for them, in read order.  The reads go in the
+    #    same rounds as consume_reads would take them.
+    def kmer_counts(self, reads, clean=False):
+        """Hashtable::get_kmer_counts over all of this rank's reads: counts of read 0's k-mers, then read 1's, ..."""
+        return self._query(reads, clean, self.shard.kmer_counts, (np.uint16,))
+
+    def read_medians(self, reads, clean=False):
+        """Hashtable::get_median_count per read: (median uint16, average float32, stddev float32, n_kmers uint32)"""
+        return self._query(reads, clean, self.shard.read_medians, (np.uint16, np.float32, np.float32, np.uint32))
+
+    def median_at_least(self, reads, cutoff, clean=False):
+        """Hashtable::median_at_least per read: 0 / 1, 2 for a read without k-mers"""
+        return self._query(reads, clean, lambda: self.shard.median_at_least(cutoff), (np.uint8,))
+
+    def trim(self, reads, abund, below=False, clean=False):
+        """trim_on_abundance (below=False) / trim_below_abundance (below=True) per read: the length each read keeps"""
+        return self._query(reads, clean, lambda: self.shard.trim(abund, below), (np.uint32,))
+
+    def abundance_distribution(self, tracking_group, reads, clean=True):
+        """Hashtable::abundance_distribution with this group's sketch as the counts and `tracking_group`'s (a Bloom filter of the
+        same hash kind, on the same devices and ranks) as the tracking filter: returns the histogram summed over the ranks, which
+        equals ONE abundance_distribution fed the rounds in stream order (run i of rank 0, of rank 1, ..., then run i + 1)."""
+        from . import cabi
+        hist = np.zeros(65536, dtype=np.uint64)
+        for run in self._runs(reads):
+            tracking_group._ingest_round(run, clean)
+            self._query_round(run, clean)
+            cabi.shard_abundance_hist(self.shard, tracking_group.shard, hist)
+        parts = self.comm.all_gather_bytes(hist.tobytes())
+        return np.sum([np.frombuffer(p, dtype=np.uint64) for p in parts], axis=0).astype(np.uint64)
 
     def stats(self):
         """(n_occupied, n_unique_kmers) of the whole sketch (collective)."""
