@@ -1,8 +1,8 @@
 // C ABI (include/kmgpu.h) + host orchestration of the kernels in kmgpu_kernels.cuh.
 //
 // One handle = one sketch resident in HBM.  Reads are processed in chunks of at most CHUNK_BASES stream
-// positions; per chunk: H2D (ASCII or packed) -> k_pack -> k_ingest -> [only when the chunk occupied new
-// bins] exact first-toucher resolution -> [only when bytes saturated] bigcount events to the host map.
+// positions; per chunk: H2D (ASCII or packed) -> k_pack -> one of the bins, delta or grouped paths (choose_path)
+// -> [only when bytes saturated] bigcount events to the host map.
 #include <algorithm>
 #include <cstdarg>
 #include <cstdio>
@@ -195,7 +195,6 @@ struct kmgpu_sketch {
     Ctrl* d_ctrl_copy = nullptr;
     Ctrl* h_ctrl_copy = nullptr;  // pinned
     // workspace
-    DevBuf<uint32_t> d_flags;
     DevBuf<uint32_t> d_newbits;
     DevBuf<uint32_t> d_filter;
     DevBuf<uint32_t> d_rank;
@@ -249,7 +248,6 @@ struct kmgpu_sketch {
     DevBuf<unsigned long long> d_hist;
     Ctrl* d_ctrl = nullptr;
     Ctrl* h_ctrl = nullptr;  // pinned
-    PinBuf<Event> h_events;
 
     // profile
     double ingest_ms = 0;
@@ -294,70 +292,6 @@ static Input make_hash_input(const uint64_t* d_hashes, uint32_t n)
 }
 
 static inline unsigned n_tiles(uint32_t n_pos) { return (n_pos + TILE - 1) / TILE; }
-
-template <int KIND, int HK, int SRC>
-static void launch_ingest_nt(const SketchDev& S, const SketchDev& M, HashCfg H, const Pred& P, bool pred, const Input& in,
-                             uint32_t* flags, Ctrl* ctrl, cudaStream_t st)
-{
-    unsigned g = n_tiles(in.n_pos);
-    if (pred) {
-        k_ingest<KIND, HK, SRC, 0, true><<<g, THREADS, 0, st>>>(S, M, H, P, in, flags, ctrl);
-    } else if (S.n_tables == 4) {
-        k_ingest<KIND, HK, SRC, 4, false><<<g, THREADS, 0, st>>>(S, M, H, P, in, flags, ctrl);
-    } else if (S.n_tables == 2) {
-        k_ingest<KIND, HK, SRC, 2, false><<<g, THREADS, 0, st>>>(S, M, H, P, in, flags, ctrl);
-    } else {
-        k_ingest<KIND, HK, SRC, 0, false><<<g, THREADS, 0, st>>>(S, M, H, P, in, flags, ctrl);
-    }
-}
-
-template <int KIND>
-static void launch_ingest_kind(int hk, int src, const SketchDev& S, const SketchDev& M, HashCfg H, const Pred& P, bool pred,
-                               const Input& in, uint32_t* flags, Ctrl* ctrl, cudaStream_t st)
-{
-    if (src == 1) launch_ingest_nt<KIND, TWOBIT, 1>(S, M, H, P, pred, in, flags, ctrl, st);
-    else if (hk == TWOBIT) launch_ingest_nt<KIND, TWOBIT, 0>(S, M, H, P, pred, in, flags, ctrl, st);
-    else launch_ingest_nt<KIND, MURMUR, 0>(S, M, H, P, pred, in, flags, ctrl, st);
-}
-
-static void launch_ingest(int src, const SketchDev& S, const SketchDev& M, HashCfg H, const Pred& P, bool pred, const Input& in,
-                          uint32_t* flags, Ctrl* ctrl, cudaStream_t st)
-{
-    if (S.kind == BYTE) launch_ingest_kind<BYTE>(H.kind, src, S, M, H, P, pred, in, flags, ctrl, st);
-    else if (S.kind == NIBBLE) launch_ingest_kind<NIBBLE>(H.kind, src, S, M, H, P, pred, in, flags, ctrl, st);
-    else launch_ingest_kind<BIT>(H.kind, src, S, M, H, P, pred, in, flags, ctrl, st);
-}
-
-template <int KIND>
-static void launch_pass_kind(int hk, int src, const SketchDev& S, int table, uint64_t lo, uint64_t hi, int first, const SketchDev& M,
-                             HashCfg H, const Pred& P, bool pred, const Input& in, uint32_t* flags, Ctrl* ctrl, cudaStream_t st)
-{
-    unsigned g = n_tiles(in.n_pos);
-#define LP(HK, SRC)                                                                                                       \
-    do {                                                                                                                  \
-        if (pred) k_ingest_pass<KIND, HK, SRC, true><<<g, THREADS, 0, st>>>(S, table, lo, hi, first, M, H, P, in, flags, ctrl);  \
-        else k_ingest_pass<KIND, HK, SRC, false><<<g, THREADS, 0, st>>>(S, table, lo, hi, first, M, H, P, in, flags, ctrl);      \
-    } while (0)
-    if (src == 1) LP(TWOBIT, 1);
-    else if (hk == TWOBIT) LP(TWOBIT, 0);
-    else LP(MURMUR, 0);
-#undef LP
-}
-
-static void launch_pass(int src, const SketchDev& S, int table, uint64_t lo, uint64_t hi, int first, const SketchDev& M, HashCfg H,
-                        const Pred& P, bool pred, const Input& in, uint32_t* flags, Ctrl* ctrl, cudaStream_t st)
-{
-    if (S.kind == BYTE) launch_pass_kind<BYTE>(H.kind, src, S, table, lo, hi, first, M, H, P, pred, in, flags, ctrl, st);
-    else if (S.kind == NIBBLE) launch_pass_kind<NIBBLE>(H.kind, src, S, table, lo, hi, first, M, H, P, pred, in, flags, ctrl, st);
-    else launch_pass_kind<BIT>(H.kind, src, S, table, lo, hi, first, M, H, P, pred, in, flags, ctrl, st);
-}
-
-#define DISPATCH_HK_SRC(KERNEL, hk, src, grid, st, ...)                                        \
-    do {                                                                                       \
-        if ((src) == 1) KERNEL<TWOBIT, 1><<<grid, THREADS, 0, st>>>(__VA_ARGS__);              \
-        else if ((hk) == TWOBIT) KERNEL<TWOBIT, 0><<<grid, THREADS, 0, st>>>(__VA_ARGS__);     \
-        else KERNEL<MURMUR, 0><<<grid, THREADS, 0, st>>>(__VA_ARGS__);                         \
-    } while (0)
 
 static void launch_counts(int src, const SketchDev& S, HashCfg H, const Input& in, const uint64_t* bk, const uint16_t* bv,
                           uint32_t nb, uint16_t* counts, uint64_t* hashes, const uint32_t* only_bits, cudaStream_t st)
@@ -520,13 +454,12 @@ extern "C" int kmgpu_destroy(kmgpu_t* h)
     if (h->d_ctrl_copy) cudaFree(h->d_ctrl_copy);
     if (h->h_ctrl_copy) cudaFreeHost(h->h_ctrl_copy);
     if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    h->d_flags.release(); h->d_newbits.release(); h->d_filter.release(); h->d_rank.release(); h->d_records.release(); h->d_cursors.release(); h->d_rec1.release(); h->d_cur1.release(); h->d_off1.release(); h->d_off2.release(); h->d_hash64.release(); h->d_newmask.release(); for (auto& sg : h->ft_segs) cudaFree(sg.first); h->ft_segs.clear(); h->d_readbits.release(); h->d_upos.release(); h->d_uc0.release(); h->d_nslot.release(); h->d_ncnt.release(); h->d_nfill.release(); h->d_nhits.release(); h->d_nstate.release(); h->d_biglist.release(); h->d_bins.release(); h->d_delta.release(); h->d_binlist.release(); h->d_sel.release(); h->d_recslot.release();
+    h->d_newbits.release(); h->d_filter.release(); h->d_rank.release(); h->d_records.release(); h->d_cursors.release(); h->d_rec1.release(); h->d_cur1.release(); h->d_off1.release(); h->d_off2.release(); h->d_hash64.release(); h->d_newmask.release(); for (auto& sg : h->ft_segs) cudaFree(sg.first); h->ft_segs.clear(); h->d_readbits.release(); h->d_upos.release(); h->d_uc0.release(); h->d_nslot.release(); h->d_ncnt.release(); h->d_nfill.release(); h->d_nhits.release(); h->d_nstate.release(); h->d_biglist.release(); h->d_bins.release(); h->d_delta.release(); h->d_binlist.release(); h->d_sel.release(); h->d_recslot.release();
     h->d_evkeys.release(); h->d_evvals.release(); h->d_evout.release(); h->h_evout.release();
     for (int i = 0; i < MAX_TABLES; i++) h->d_satbits[i].release();
     h->d_htkeys.release(); h->d_htvals.release(); h->d_events.release(); h->d_counts.release(); h->d_hashes.release();
     h->d_hashin.release(); h->d_stat_med.release(); h->d_stat_f.release(); h->d_stat_n.release(); h->d_stat_b.release();
     h->d_hist.release(); h->big_keys.release(); h->big_vals.release();
-    h->h_events.release();
     if (h->d_ctrl) cudaFree(h->d_ctrl);
     if (h->h_ctrl) cudaFreeHost(h->h_ctrl);
     if (h->ev0) cudaEventDestroy(h->ev0);
@@ -713,15 +646,6 @@ extern "C" int kmgpu_bigcount_import(kmgpu_t* h, const uint64_t* hashes, const u
     return KMGPU_OK;
 }
 
-// ByteStorage::add tail (storage.hh:606-617)
-static inline void big_event(kmgpu_sketch* h, uint64_t hash)
-{
-    uint16_t& v = h->big[hash];
-    if (v == 0) v = 256;
-    else if (v < 65535) v++;
-    h->big_dirty = true;
-}
-
 static int sync_big_to_device(kmgpu_sketch* h)
 {
     if (!h->big_dirty) return KMGPU_OK;
@@ -759,160 +683,6 @@ static int read_ctrl(kmgpu_sketch* h)
     return KMGPU_OK;
 }
 
-// first-toucher resolution for the chunk whose flags are in d_flags: leaves the "new" bitmap in
-// d_newbits and returns the number of new k-mers.
-static int resolve_new(kmgpu_sketch* h, int src, const SketchDev& S, HashCfg H, const Input& in, uint64_t n_keys, uint64_t* n_new)
-{
-    cudaStream_t st = h->stream;
-    uint64_t slots = pow2_at_least(2 * n_keys);
-    CKR(h->d_htkeys.ensure(slots));
-    CKR(h->d_htvals.ensure(slots));
-    size_t nb_words = (in.n_pos + 31) / 32;
-    CKR(h->d_newbits.ensure(nb_words));
-    CK(cudaMemsetAsync(h->d_htkeys.p, 0xFF, slots * 8, st));
-    CK(cudaMemsetAsync(h->d_htvals.p, 0xFF, slots * 4, st));
-    CK(cudaMemsetAsync(h->d_newbits.p, 0, nb_words * 4, st));
-    CK(cudaMemsetAsync(&h->d_ctrl->n_unique, 0, sizeof(unsigned long long), st));
-    unsigned g = n_tiles(in.n_pos);
-    // bitmap prefilter of the registered bins; pointless once it would be mostly ones
-    uint32_t* filter = nullptr;
-    if (n_keys < (uint64_t)S.n_tables * FILTER_BITS / 4) {
-        CKR(h->d_filter.ensure((size_t)S.n_tables * FILTER_WORDS));
-        CK(cudaMemsetAsync(h->d_filter.p, 0, (size_t)S.n_tables * FILTER_WORDS * 4, st));
-        filter = h->d_filter.p;
-    }
-    DISPATCH_HK_SRC(k_register, H.kind, src, g, st, S, H, in, h->d_flags.p, 0, h->d_htkeys.p, slots - 1, filter);
-    DISPATCH_HK_SRC(k_replay, H.kind, src, g, st, S, H, in, h->d_flags.p, h->d_htkeys.p, h->d_htvals.p, slots - 1, filter);
-    unsigned gm = (unsigned)std::min<uint64_t>((slots + 255) / 256, 148 * 8);
-    k_mark<<<gm, 256, 0, st>>>(h->d_htkeys.p, h->d_htvals.p, slots, h->d_newbits.p, h->d_ctrl);
-    h->all_launches += 3;
-    CK(cudaGetLastError());
-    CKR(read_ctrl(h));
-    *n_new = h->h_ctrl->n_unique;
-    return KMGPU_OK;
-}
-
-// bigcount after a chunk (ByteStorage with use_bigcount).  See DESIGN.md "bigcount exactness".
-static int resolve_bigcount(kmgpu_sketch* h, int src, HashCfg H, const Input& in, uint64_t n_allsat, uint64_t n_cross)
-{
-    cudaStream_t st = h->stream;
-    const SketchDev& S = h->dev;
-    unsigned g = n_tiles(in.n_pos);
-    std::vector<Event> certain;
-    if (n_allsat) {
-        CKR(h->d_events.ensure(n_allsat));
-        CKR(h->h_events.ensure(n_allsat));
-        CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
-        DISPATCH_HK_SRC(k_events, H.kind, src, g, st, S, H, in, h->d_flags.p, h->d_events.p, h->d_ctrl);
-        h->all_launches += 1;
-        CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(h->h_events.p, h->d_events.p, n_allsat * sizeof(Event), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        certain.assign(h->h_events.p, h->h_events.p + n_allsat);
-        std::sort(certain.begin(), certain.end(), [](const Event& a, const Event& b) { return a.pos < b.pos; });
-    }
-    if (!n_cross) {
-        // every saturated bin was saturated before the chunk began: memory order == stream order for the test
-        for (const Event& e : certain) big_event(h, e.hash);
-        return KMGPU_OK;
-    }
-    // some bins reached 255 inside this chunk: rebuild, per such bin, the stream position T of the update
-    // that saturated it.  If E updates of the chunk found the bin already saturated (a count that does not
-    // depend on the order), T is the update with exactly E later updates of that bin.
-    uint64_t slots = pow2_at_least(2 * n_cross);
-    CKR(h->d_htkeys.ensure(slots));
-    CK(cudaMemsetAsync(h->d_htkeys.p, 0xFF, slots * 8, st));
-    DISPATCH_HK_SRC(k_register, H.kind, src, g, st, S, H, in, h->d_flags.p, 20, h->d_htkeys.p, slots - 1, (uint32_t*)nullptr);
-    uint64_t cap = in.n_pos;
-    CKR(h->d_events.ensure(cap));
-    CKR(h->h_events.ensure(cap));
-    CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
-    DISPATCH_HK_SRC(k_cross_replay, H.kind, src, g, st, S, H, in, h->d_flags.p, h->d_htkeys.p, slots - 1, h->d_events.p,
-                    (unsigned long long)cap, h->d_ctrl);
-    h->all_launches += 2;
-    CK(cudaGetLastError());
-    CKR(read_ctrl(h));
-    uint64_t n_rec = h->h_ctrl->n_events;
-    if (n_rec > cap) return fail(KMGPU_ECUDA, "internal: cross replay overflow");
-    if (n_rec) {
-        CK(cudaMemcpyAsync(h->h_events.p, h->d_events.p, n_rec * sizeof(Event), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    }
-    std::vector<Event> recs(h->h_events.p, h->h_events.p + n_rec);
-    std::sort(recs.begin(), recs.end(), [](const Event& a, const Event& b) { return a.pos < b.pos; });
-    struct BinInfo {
-        std::vector<uint32_t> touches;
-        uint64_t later = 0;  // E
-        uint32_t T = 0;
-    };
-    std::unordered_map<uint64_t, BinInfo> bins;  // key = bin << 8 | table
-    for (const Event& e : recs) {
-        uint32_t cross = e.info & 0x3ff, sat = (e.info >> 10) & 0x3ff;
-        for (int i = 0; i < h->nt; i++) {
-            if (!(cross >> i & 1)) continue;
-            BinInfo& b = bins[((e.hash % h->sizes[i]) << 8) | (uint64_t)i];
-            b.touches.push_back(e.pos);  // ascending
-            b.later += (sat >> i) & 1;
-        }
-    }
-    for (auto& kv : bins) {
-        BinInfo& b = kv.second;
-        if (b.later >= b.touches.size()) return fail(KMGPU_ECUDA, "internal: inconsistent saturation record");
-        b.T = b.touches[b.touches.size() - 1 - b.later];
-    }
-    // merge: records decide k-mers touching a crossing bin, `certain` decides the rest
-    std::vector<Event> events;
-    size_t ci = 0;
-    for (const Event& e : recs) {
-        while (ci < certain.size() && certain[ci].pos < e.pos) events.push_back(certain[ci++]);
-        if (ci < certain.size() && certain[ci].pos == e.pos) ci++;  // decided here instead
-        if (!(e.info >> 30 & 1)) continue;
-        bool after_all = true;
-        uint32_t cross = e.info & 0x3ff;
-        for (int i = 0; i < h->nt && after_all; i++) {
-            if (!(cross >> i & 1)) continue;
-            const BinInfo& b = bins[((e.hash % h->sizes[i]) << 8) | (uint64_t)i];
-            if (!(e.pos > b.T)) after_all = false;
-        }
-        if (after_all) events.push_back(e);
-    }
-    while (ci < certain.size()) events.push_back(certain[ci++]);
-    for (const Event& e : events) big_event(h, e.hash);
-    return KMGPU_OK;
-}
-
-// ------------------------------------------------------------------------------------------------------
-// L2-blocked passes.  A sketch that is neither small enough to sit in L2 as a whole nor hopelessly larger
-// than L2 is ingested one table (or one address range of a table) at a time, so that each pass's counters
-// stay L2-resident (profiles/r1_atomic_ceiling.txt: random updates run 2-5x faster at <= ~100 MB).
-// ------------------------------------------------------------------------------------------------------
-struct PassPlan {
-    int table;
-    uint64_t lo, hi;  // bins
-};
-
-static uint64_t l2_block_bytes()
-{
-    uint64_t b = env_u64("KMGPU_L2_BLOCK_BYTES", ~0ull);  // test hook: force passes on tiny tables
-    return b != ~0ull ? b : env_u64("KMGPU_L2_BLOCK_MB", 104) * 1000000ull;
-}
-
-static void plan_passes(const kmgpu_sketch* h, std::vector<PassPlan>& out)
-{
-    out.clear();
-    const uint64_t block = l2_block_bytes();
-    const uint64_t max_passes = env_u64("KMGPU_MAX_PASSES", 16);
-    uint64_t total = 0;
-    for (int i = 0; i < h->nt; i++) total += h->nbytes[i];
-    if (block == 0 || total <= block) return;  // single pass: everything is L2-resident anyway
-    for (int i = 0; i < h->nt; i++) {
-        uint64_t r = (h->nbytes[i] + block - 1) / block;
-        uint64_t per = (h->sizes[i] + r - 1) / r;
-        for (uint64_t j = 0; j < r; j++) out.push_back(PassPlan{i, j * per, std::min(h->sizes[i], (j + 1) * per)});
-    }
-    if (out.size() > max_passes) out.clear();  // far larger than L2: one pass, HBM-bound either way
-}
-
 struct ChunkResult {
     uint64_t n_kmers = 0, n_new = 0;
     bool have_newbits = false;
@@ -942,7 +712,6 @@ static uint64_t delta_block_bins(int kind)
 static bool plan_delta(const kmgpu_sketch* h, std::vector<DeltaPass>& out)
 {
     out.clear();
-    if (!env_u64("KMGPU_DELTA", 1)) return false;
     const uint64_t block = delta_block_bins(h->kind);
     const uint64_t gran = h->kind == BIT ? 128 : 8;
     for (int i = 0; i < h->nt; i++) {
@@ -1398,61 +1167,83 @@ static int ingest_chunk_delta(kmgpu_sketch* h, const std::vector<DeltaPass>& pas
     return KMGPU_OK;
 }
 
-// ingest one staged chunk into sketch `h` (hash config may come from another sketch: abundance tracking)
-static int ingest_chunk(kmgpu_sketch* h, int src, HashCfg H, const Input& in, const Pred& P, bool pred, const SketchDev* M,
-                        ChunkResult* res, const Between& between = Between())
+// ------------------------------------------------------------------------------------------------------
+// path of a chunk
+// ------------------------------------------------------------------------------------------------------
+// Bins: k_hashbins + k_bucketize + k_apply (ingest_chunk_delta; a bucket that overflows sends the chunk through the delta passes)
+// Delta: k_hashbins + k_scatter + k_fold per table block (ingest_chunk_delta)
+// Grouped: k_part + k_apply2 / k_apply_sparse (ingest_chunk_grouped)
+enum class Path { Choose, Unsupported, Bins, Delta, Grouped };
+
+constexpr size_t PREFER_DELTA_MAX_BLOCKS = 12;
+
+// The path of a chunk of n_pos positions; G (optional) receives the grouped layout.  `first_touch`: the sketch keeps a first-touch
+// log, which only the grouped path writes.
+static Path choose_path(const kmgpu_sketch* h, uint32_t n_pos, bool first_touch, GroupPlan* G = nullptr)
 {
-    if (in.n_pos == 0) return between ? between() : KMGPU_OK;
-    {
-        GroupPlan G;
-        if (plan_group(h, in.n_pos, h->nt > F_MAXT || h->ft_on, &G))
-            return ingest_chunk_grouped(h, G, src, H, std::vector<Part>(1, Part{in, 0u, nullptr}), P, pred, M, res, between);
-        if (h->nt > F_MAXT) return fail(KMGPU_EUNSUPPORTED, "sketches with more than %d tables need the grouped path, which this shape cannot take", F_MAXT);
-        std::vector<DeltaPass> dp;
-        if (plan_delta(h, dp)) return ingest_chunk_delta(h, dp, src, H, std::vector<Part>(1, Part{in, 0u, nullptr}), P, pred, M, res, between);
+    GroupPlan own;
+    if (!G) G = &own;
+    if (h->nt > F_MAXT || first_touch) return plan_group(h, n_pos, G) ? Path::Grouped : Path::Unsupported;
+    std::vector<DeltaPass> dp;
+    const bool delta = plan_delta(h, dp);
+    BucketLayout BL;
+    const bool bins = delta && plan_buckets(h, n_pos, &BL);
+    const uint64_t min_buckets = env_u64("KMGPU_GROUP_MIN_BUCKETS", 1024);
+    // tests steer small shapes onto the grouped path
+    const bool hooked = !env_u64("KMGPU_PREFER_BINS", 1) || env_u64("KMGPU_FORCE_TWO_LEVEL", 0) || min_buckets == 0;
+    // Shapes the bins path can take (every table within 6144 buckets, <= 65535 records per bucket and chunk) stay with it: hashing
+    // once per position into the bins[] array and grouping with k_bucketize measures faster there than the fused kernel
+    // (profiles/r2_grouping_variants.txt), at the price of 37 B per k-mer more DRAM traffic
+    if (!hooked && bins) return Path::Bins;
+    // ... and shapes the delta + fold passes cover in a dozen L2-sized blocks (config C2's Bloom filter: 18.3 against 10.1
+    // G k-mers/s) measure faster there than through two grouping levels; with more blocks (SmallCountgraph at 4 x 4e8: 16
+    // blocks, 9.1 against 10.7) the grouped path wins
+    if (!hooked && delta && dp.size() <= PREFER_DELTA_MAX_BLOCKS) return Path::Delta;
+    const bool grouped = plan_group(h, n_pos, G);
+    if (grouped && G->n_buckets >= min_buckets) return Path::Grouped;
+    if (delta) return bins ? Path::Bins : Path::Delta;   // a handful of buckets cannot fill the machine
+    return grouped ? Path::Grouped : Path::Unsupported;
+}
+
+// Ingest one chunk into sketch `h` (hash config may come from another sketch: abundance tracking).  `path`: the caller's
+// choice; by default it is chosen here for the chunk's extent.
+static int ingest_chunk(kmgpu_sketch* h, int src, HashCfg H, const std::vector<Part>& parts, const Pred& P, bool pred, const SketchDev* M,
+                        ChunkResult* res, const Between& between = Between(), Path path = Path::Choose)
+{
+    uint32_t n_pos = 0;
+    for (const Part& pt : parts) n_pos = std::max(n_pos, pt.pos_off + pt.in.n_pos);
+    if (n_pos == 0) return between ? between() : KMGPU_OK;
+    GroupPlan G;   // the regions are sized for this chunk's positions
+    if (path == Path::Choose) path = choose_path(h, n_pos, h->ft_on, &G);
+    else if (path == Path::Grouped && !plan_group(h, n_pos, &G)) return fail(KMGPU_ECUDA, "internal: grouped plan changed between chunks");
+    if (path == Path::Grouped) return ingest_chunk_grouped(h, G, src, H, parts, P, pred, M, res, between);
+    std::vector<DeltaPass> dp;
+    if (path == Path::Unsupported || !plan_delta(h, dp))
+        return fail(KMGPU_EUNSUPPORTED, "no ingestion path can take this sketch (%d tables; more than %d need the grouped path)", h->nt, F_MAXT);
+    return ingest_chunk_delta(h, dp, src, H, parts, P, pred, M, res, between);
+}
+
+// Positions per chunk for this sketch.  A chunk costs one pass over every bucket of the sketch; where the two-level grouped path is
+// taken (tables of billions of bins) that pass is what dominates, so chunks grow to what half of the free device memory holds in
+// record stores (two levels of 8-byte records with their slack, plus hashes and bitmaps).  The first-touch log, which takes every
+// chunk onto the grouped path, does not change the chunk size.
+static uint64_t sketch_chunk_bases(kmgpu_sketch* h)
+{
+    if (getenv("KMGPU_CHUNK_BASES")) return chunk_bases();
+    if (h->chunk_cap) return h->chunk_cap;
+    uint64_t cap = chunk_bases();
+    GroupPlan G;
+    if (choose_path(h, (uint32_t)cap, false, &G) == Path::Grouped && G.L.two_level) {
+        size_t fr = 0, tot = 0;
+        if (cudaMemGetInfo(&fr, &tot) == cudaSuccess) {
+            const uint64_t per_pos = (uint64_t)h->nt * 21 + 16;
+            uint64_t p = std::min<uint64_t>((fr / 2) / per_pos, 1ull << 30);
+            cap = std::max<uint64_t>(cap, (p / TILE) * TILE);
+        }
+        cudaGetLastError();
     }
-    cudaStream_t st = h->stream;
-    CKR(h->d_flags.ensure(in.n_pos));
-    CK(cudaMemsetAsync(h->d_ctrl, 0, sizeof(Ctrl), st));
-    std::vector<PassPlan> passes;
-    plan_passes(h, passes);
-    CK(cudaEventRecord(h->ev0, st));
-    if (passes.empty()) {
-        launch_ingest(src, h->dev, M ? *M : h->dev, H, P, pred, in, h->d_flags.p, h->d_ctrl, st);
-    } else {
-        for (size_t pi = 0; pi < passes.size(); pi++)
-            launch_pass(src, h->dev, passes[pi].table, passes[pi].lo, passes[pi].hi, pi == 0, M ? *M : h->dev, H, P, pred, in,
-                        h->d_flags.p, h->d_ctrl, st);
-    }
-    CK(cudaEventRecord(h->ev1, st));
-    CK(cudaGetLastError());
-    if (between) CKR(between());
-    CKR(read_ctrl(h));
-    float ms = 0;
-    CK(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-    h->ingest_ms += ms;
-    size_t nl = passes.empty() ? 1 : passes.size();
-    h->ingest_launches += nl;
-    h->all_launches += nl;
-    if (!passes.empty() && h->kind == BYTE && h->use_bigcount && h->h_ctrl->n_sat) {
-        k_count_allsat<<<148 * 8, 256, 0, st>>>(h->d_flags.p, in.n_pos, (1u << h->nt) - 1, h->d_ctrl);
-        h->all_launches += 1;
-        CK(cudaGetLastError());
-        CKR(read_ctrl(h));
-    }
-    Ctrl c = *h->h_ctrl;
-    res->n_kmers += c.n_kmers;
-    h->n_occupied += c.n_z0;
-    if (c.n_zbits) {
-        uint64_t n_new = 0;
-        CKR(resolve_new(h, src, h->dev, H, in, c.n_zbits, &n_new));
-        h->n_unique += n_new;
-        res->n_new += n_new;
-        res->have_newbits = true;
-    }
-    if (h->kind == BYTE && h->use_bigcount && (c.n_allsat || c.n_cross))
-        CKR(resolve_bigcount(h, src, H, in, c.n_allsat, c.n_cross));
-    return KMGPU_OK;
+    h->chunk_cap = cap;
+    return cap;
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -1693,8 +1484,6 @@ static int consume_host(kmgpu_t* h, const char* seqs, const uint64_t* packed, ui
         // large as for device-resident input, but it is uploaded, packed, hashed and bucketized part by part, so that only
         // the first part's trip over PCIe is exposed.  All of a chunk's copies are queued on the copy stream at once (one
         // staging slot per part, two sets of slots: the next chunk's parts are queued while this chunk is being applied).
-        std::vector<DeltaPass> dp;
-        BucketLayout BL;
         const uint64_t total = last - first, cap = sketch_chunk_bases(h);
         const uint64_t n_chunks = (total + cap - 1) / cap;
         const uint64_t per_chunk = (((total + n_chunks - 1) / n_chunks) + 31) & ~31ull;
@@ -1702,10 +1491,9 @@ static int consume_host(kmgpu_t* h, const char* seqs, const uint64_t* packed, ui
         const uint64_t part_cap = (std::max<uint64_t>(std::min<uint64_t>(env_u64("KMGPU_PART_BASES", 24ull << 20), per_chunk),
                                                       (per_chunk + kmgpu_sketch::MAX_PARTS - 1) / kmgpu_sketch::MAX_PARTS) + 31) & ~31ull;
         const uint64_t worst_pos = per_chunk + (uint64_t)kmgpu_sketch::MAX_PARTS * h->k;
-        GroupPlan GP;
-        const bool grouped = worst_pos < (1ull << 31) && plan_group(h, (uint32_t)worst_pos, h->nt > F_MAXT || h->ft_on, &GP);
-        if (env_u64("KMGPU_PARTS", 1) && total > part_cap && worst_pos < (1ull << 31) &&
-            (grouped || (h->nt <= F_MAXT && plan_delta(h, dp) && plan_buckets(h, (uint32_t)worst_pos, &BL)))) {
+        // the path is kept for every chunk of the call: a short last chunk that the bins path could take stays grouped
+        const Path path = worst_pos < (1ull << 31) ? choose_path(h, (uint32_t)worst_pos, h->ft_on) : Path::Unsupported;
+        if (env_u64("KMGPU_PARTS", 1) && total > part_cap && (path == Path::Bins || path == Path::Grouped)) {
             struct Staged { std::vector<Part> parts; };
             Staged set[2];
             auto stage_chunk_parts = [&](uint64_t ci, Staged* out) -> int {
@@ -1735,15 +1523,7 @@ static int consume_host(kmgpu_t* h, const char* seqs, const uint64_t* packed, ui
                 if (set[ci & 1].parts.empty()) break;
                 const Between next = [&]() -> int { return ci + 1 < n_chunks ? stage_chunk_parts(ci + 1, &set[(ci + 1) & 1]) : KMGPU_OK; };
                 ChunkResult cr;
-                if (grouped) {
-                    uint32_t np = 0;
-                    for (const Part& pt : set[ci & 1].parts) np = std::max(np, pt.pos_off + pt.in.n_pos);
-                    GroupPlan G;   // the regions are sized for this chunk's positions
-                    if (!plan_group(h, np, true, &G)) return fail(KMGPU_ECUDA, "internal: grouped plan changed between chunks");
-                    CKR(ingest_chunk_grouped(h, G, 0, H, set[ci & 1].parts, P, pred, M, &cr, next));
-                } else {
-                    CKR(ingest_chunk_delta(h, dp, 0, H, set[ci & 1].parts, P, pred, M, &cr, next));
-                }
+                CKR(ingest_chunk(h, 0, H, set[ci & 1].parts, P, pred, M, &cr, next, path));
                 res.n_kmers += cr.n_kmers;
                 res.n_new += cr.n_new;
                 if (newbits_out && cr.have_newbits) {
@@ -1804,7 +1584,7 @@ static int consume_host(kmgpu_t* h, const char* seqs, const uint64_t* packed, ui
     for (uint64_t i = 0; i < n_chunks; i++) {
         CK(cudaStreamWaitEvent(h->stream, h->stage[i & 1].ready, 0));
         ChunkResult cr;
-        CKR(ingest_chunk(h, 0, H, make_input(cd[i & 1]), P, pred, M, &cr, [&]() -> int {
+        CKR(ingest_chunk(h, 0, H, {Part{make_input(cd[i & 1]), 0u, nullptr}}, P, pred, M, &cr, [&]() -> int {
             if (i + 1 < n_chunks) {
                 int ns = (int)((i + 1) & 1);
                 uint64_t c0, c1;
@@ -1987,11 +1767,10 @@ extern "C" int kmgpu_consume_batch(kmgpu_t* h, const kmgpu_batch_t* b, const kmg
             pos += p.n_pos;
             j++;
         }
-        GroupPlan G;
-        if (parts.size() > 1 && pos < (1ull << 31) && plan_group(h, (uint32_t)pos, h->nt > F_MAXT || h->ft_on, &G)) {
-            CKR(ingest_chunk_grouped(h, G, 0, H, parts, P, pred, M, &res, Between()));
+        if (parts.size() > 1 && pos < (1ull << 31) && choose_path(h, (uint32_t)pos, h->ft_on) == Path::Grouped) {
+            CKR(ingest_chunk(h, 0, H, parts, P, pred, M, &res));
         } else {
-            for (const Part& pt : parts) CKR(ingest_chunk(h, 0, H, pt.in, P, pred, M, &res));
+            for (const Part& pt : parts) CKR(ingest_chunk(h, 0, H, {Part{pt.in, 0u, nullptr}}, P, pred, M, &res));
         }
         i = j;
     }
@@ -2019,7 +1798,7 @@ extern "C" int kmgpu_add_hashes(kmgpu_t* h, const uint64_t* hashes, uint64_t n, 
         CKR(h->d_hashin.ensure(m));
         CK(cudaMemcpyAsync(h->d_hashin.p, hashes + i0, 8ull * m, cudaMemcpyHostToDevice, h->stream));
         ChunkResult res;
-        CKR(ingest_chunk(h, 1, H, make_hash_input(h->d_hashin.p, m), P, false, nullptr, &res));
+        CKR(ingest_chunk(h, 1, H, {Part{make_hash_input(h->d_hashin.p, m), 0u, nullptr}}, P, false, nullptr, &res));
         if (is_new_out) {
             if (res.have_newbits) {
                 bits.resize((m + 31) / 32);
@@ -2331,11 +2110,11 @@ extern "C" int kmgpu_abundance_distribution(kmgpu_t* counts, kmgpu_t* tracking, 
         if (cd.n_pos == 0) continue;
         ChunkResult res;
         Input in = make_input(cd);
+        const std::vector<Part> one(1, Part{in, 0u, nullptr});
         t->ft_defer = t->ft_on;   // first-touch log: the entries of this chunk carry the k-mers' counts, known below
-        int rc = ingest_chunk(t, 0, H, in, P, false, nullptr, &res);
+        int rc = ingest_chunk(t, 0, H, one, P, false, nullptr, &res);
         t->ft_defer = false;
         CKR(rc);
-        const std::vector<Part> one(1, Part{in, 0u, nullptr});
         if (!res.have_newbits || res.n_new == 0) {
             if (t->ft_on) CKR(ft_emit(t, 0, H, one, nullptr));
             continue;
@@ -2651,7 +2430,7 @@ extern "C" int kmgpu_normalize_batch(kmgpu_t* h, const char* seqs, const uint64_
                     Input ink = make_input(cd);
                     ink.read_keep = h->d_readbits.p;
                     ChunkResult res;
-                    CKR(ingest_chunk(h, 0, H, ink, P0, false, nullptr, &res));
+                    CKR(ingest_chunk(h, 0, H, {Part{ink, 0u, nullptr}}, P0, false, nullptr, &res));
                     kmers_total += res.n_kmers;
                     kept_total += nk_reads;
                 }
@@ -3124,7 +2903,7 @@ extern "C" int kmgpu_shard_create(int storage, int hash, int ksize, int n_tables
         full_shape.nt = n_tables;
         full_shape.kind = storage;
         for (int i = 0; i < n_tables; i++) full_shape.sizes[i] = full_sizes[i];
-        if (!plan_group(&full_shape, (uint32_t)max_positions, true, &s->GF, true) || !s->GF.L.two_level) {
+        if (!plan_group(&full_shape, (uint32_t)max_positions, &s->GF, true) || !s->GF.L.two_level) {
             delete s;
             return fail(KMGPU_EUNSUPPORTED, "tables of this size cannot be grouped");
         }
@@ -3164,7 +2943,7 @@ extern "C" int kmgpu_shard_create(int storage, int hash, int ksize, int n_tables
         nominal_shape.nt = n_tables;
         nominal_shape.kind = storage;
         for (int i = 0; i < n_tables; i++) nominal_shape.sizes[i] = nominal[i];
-        const bool ok = plan_group(&nominal_shape, (uint32_t)max_positions, true, &s->G, true, PART_MAXP, (uint64_t)world * max_positions, shift);
+        const bool ok = plan_group(&nominal_shape, (uint32_t)max_positions, &s->G, true, PART_MAXP, (uint64_t)world * max_positions, shift);
         if (!ok || !s->G.L.two_level || s->G.n_sb != s->n_sb_local) {
             kmgpu_shard_destroy(s);
             return fail(KMGPU_EUNSUPPORTED, "slices of this size cannot be grouped");

@@ -1,5 +1,5 @@
 // Device-side building blocks: 2-bit stream access, the two hash functions, modulo by an
-// arbitrary table size, and the three saturating counter updates.  sm_100a only.
+// arbitrary table size, and the three counter reads.  sm_100a only.
 #pragma once
 #include <cstdint>
 #include <cuda_fp16.h>
@@ -196,69 +196,23 @@ __device__ __forceinline__ uint64_t hash_murmur(const uint64_t* __restrict__ w, 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Counter updates.  Each returns the value the counter held BEFORE this update in the order the memory
-// system serialised the updates of that bin (0 => this update occupied the bin).
+// Counter reads.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t ld_cg_u32(const uint32_t* p) { return __ldcg(p); }
-
-// ByteStorage::add core (storage.hh:577-603): +1 while < 255.  The byte lives in a 32-bit word that is
-// updated with compare-and-swap so that a saturated byte never carries into its neighbour.
-__device__ __forceinline__ uint32_t update_byte(uint8_t* table, uint64_t bin)
-{
-    uint32_t* word = reinterpret_cast<uint32_t*>(table + (bin & ~3ull));
-    uint32_t sh = (uint32_t)(bin & 3) * 8;
-    uint32_t cur = ld_cg_u32(word);
-    while (true) {
-        uint32_t b = (cur >> sh) & 255u;
-        if (b == 255u) return 255u;
-        uint32_t seen = atomicCAS(word, cur, cur + (1u << sh));
-        if (seen == cur) return b;
-        cur = seen;
-    }
-}
+// ByteStorage: one byte per bin.
 __device__ __forceinline__ uint32_t read_byte(const uint8_t* table, uint64_t bin) { return __ldcg(table + bin); }
 
-// NibbleStorage::add core (storage.hh:325-351): even bin -> high nibble (helpers :259-272), clamp 15.
-__device__ __forceinline__ uint32_t update_nibble(uint8_t* table, uint64_t bin)
-{
-    uint64_t byte = bin >> 1;
-    uint32_t* word = reinterpret_cast<uint32_t*>(table + (byte & ~3ull));
-    uint32_t sh = (uint32_t)(byte & 3) * 8 + ((bin & 1) ? 0 : 4);
-    uint32_t cur = ld_cg_u32(word);
-    while (true) {
-        uint32_t b = (cur >> sh) & 15u;
-        if (b == 15u) return 15u;
-        uint32_t seen = atomicCAS(word, cur, cur + (1u << sh));
-        if (seen == cur) return b;
-        cur = seen;
-    }
-}
+// NibbleStorage: even bin -> high nibble (storage.hh:259-272).
 __device__ __forceinline__ uint32_t read_nibble(const uint8_t* table, uint64_t bin)
 {
     return (__ldcg(table + (bin >> 1)) >> ((bin & 1) ? 0 : 4)) & 15u;
 }
 
-// BitStorage::test_and_set_bits core (storage.hh:176-184): bit (bin % 8) of byte bin / 8, i.e. bit
-// (bin % 32) of little-endian word bin / 32.  Already-set bits are not written again.
-__device__ __forceinline__ uint32_t update_bit(uint8_t* table, uint64_t bin)
-{
-    uint32_t* word = reinterpret_cast<uint32_t*>(table) + (bin >> 5);
-    uint32_t bit = 1u << (bin & 31);
-    if (ld_cg_u32(word) & bit) return 1u;
-    return (atomicOr(word, bit) & bit) ? 1u : 0u;
-}
+// BitStorage: bit (bin % 8) of byte bin / 8 (storage.hh:176-184).
 __device__ __forceinline__ uint32_t read_bit(const uint8_t* table, uint64_t bin)
 {
     return (__ldcg(table + (bin >> 3)) >> (bin & 7)) & 1u;
 }
 
-template <int KIND>
-__device__ __forceinline__ uint32_t update_counter(uint8_t* t, uint64_t bin)
-{
-    if (KIND == BYTE) return update_byte(t, bin);
-    if (KIND == NIBBLE) return update_nibble(t, bin);
-    return update_bit(t, bin);
-}
 template <int KIND>
 __device__ __forceinline__ uint32_t read_counter(const uint8_t* t, uint64_t bin)
 {
@@ -270,85 +224,6 @@ template <int KIND>
 __device__ __forceinline__ uint32_t counter_cap()
 {
     return KIND == BYTE ? 255u : KIND == NIBBLE ? 15u : 1u;
-}
-
-// ------------------------------------------------------------------------------------------------
-// U independent updates issued together: all loads first, then all compare-and-swaps, then the (rare)
-// retries.  Each update is two dependent L2 round trips; interleaving U of them per thread is what keeps
-// the L2 atomic units busy (profiles/r1_atomic_ceiling.txt: one-at-a-time ld+CAS reaches a third of the
-// L2-resident atomic rate).  Semantics per update are exactly update_counter<KIND>.
-// ------------------------------------------------------------------------------------------------
-template <int KIND, int U>
-__device__ __forceinline__ void multi_update(uint8_t* const* tab, const uint64_t* bin, const bool* act, uint32_t* old)
-{
-    uint32_t* word[U];
-    uint32_t sh[U], cur[U];
-    bool pend[U];
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-        pend[u] = false;
-        old[u] = 1u;  // inactive slots report "occupied, not saturated"
-        if (!act[u]) continue;
-        if (KIND == BYTE) {
-            word[u] = reinterpret_cast<uint32_t*>(tab[u] + (bin[u] & ~3ull));
-            sh[u] = (uint32_t)(bin[u] & 3) * 8;
-        } else if (KIND == NIBBLE) {
-            uint64_t byte = bin[u] >> 1;
-            word[u] = reinterpret_cast<uint32_t*>(tab[u] + (byte & ~3ull));
-            sh[u] = (uint32_t)(byte & 3) * 8 + ((bin[u] & 1) ? 0 : 4);
-        } else {
-            word[u] = reinterpret_cast<uint32_t*>(tab[u]) + (bin[u] >> 5);
-            sh[u] = (uint32_t)(bin[u] & 31);
-        }
-        cur[u] = ld_cg_u32(word[u]);
-    }
-    constexpr uint32_t CAP = KIND == BYTE ? 255u : KIND == NIBBLE ? 15u : 1u;
-    // issue every atomic before looking at any result, so the U round trips overlap
-    uint32_t seen[U];
-    bool tried[U];
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-        uint32_t b = (cur[u] >> sh[u]) & CAP;
-        tried[u] = act[u] && b != CAP;
-        seen[u] = cur[u];
-        if (tried[u]) {
-            if (KIND == BIT) seen[u] = atomicOr(word[u], 1u << sh[u]);
-            else seen[u] = atomicCAS(word[u], cur[u], cur[u] + (1u << sh[u]));
-        }
-    }
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-        if (!act[u]) continue;
-        uint32_t b = (cur[u] >> sh[u]) & CAP;
-        if (!tried[u]) {
-            old[u] = CAP;
-        } else if (KIND == BIT) {
-            old[u] = (seen[u] >> sh[u]) & 1u;
-        } else if (seen[u] == cur[u]) {
-            old[u] = b;
-        } else {
-            cur[u] = seen[u];
-            pend[u] = true;
-        }
-    }
-    if (KIND != BIT) {
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            while (pend[u]) {
-                uint32_t b = (cur[u] >> sh[u]) & CAP;
-                if (b == CAP) {
-                    old[u] = CAP;
-                    pend[u] = false;
-                } else {
-                    uint32_t seen = atomicCAS(word[u], cur[u], cur[u] + (1u << sh[u]));
-                    if (seen == cur[u]) {
-                        old[u] = b;
-                        pend[u] = false;
-                    } else cur[u] = seen;
-                }
-            }
-        }
-    }
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -454,19 +454,11 @@ __host__ __device__ constexpr uint32_t slice_bytes_full() { return KIND == BYTE 
 template <int KIND, int SPLIT>
 constexpr size_t apply2_smem() { return ((size_t)BKT_BINS * 2 + (size_t)BKT_BINS * 4 + slice_bytes_full<KIND>()) / SPLIT + 64; }
 
-template <int KIND>
-__device__ __forceinline__ bool slice_empty(const uint8_t* slice, uint32_t lb)
-{
-    if (KIND == BYTE) return slice[lb] == 0;
-    if (KIND == NIBBLE) return ((slice[lb >> 1] >> ((lb & 1) ? 0 : 4)) & 15u) == 0;
-    return !((slice[lb >> 3] >> (lb & 7)) & 1u);
-}
-
 template <int KIND, int SPLIT>
 __global__ void __launch_bounds__(1024 / SPLIT, SPLIT == 4 ? 3 : SPLIT)
 k_apply2(const __grid_constant__ SketchDev S, const __grid_constant__ GroupLayout L, Store st, uint32_t bucket0, uint32_t* __restrict__ newbits,
          uint64_t* __restrict__ binlist, unsigned long long list_cap, Ctrl* ctrl, int want_cross, const __grid_constant__ SatBitsG sb,
-         unsigned long long ovf_mask, uint32_t* __restrict__ newmask, int gate, const uint32_t* __restrict__ bucket_list)
+         unsigned long long ovf_mask, uint32_t* __restrict__ newmask, const uint32_t* __restrict__ bucket_list)
 {
     extern __shared__ __align__(128) unsigned char ap_raw[];
     constexpr uint32_t SUB_BINS = BKT_BINS / SPLIT, NTHR = 1024 / SPLIT, SUB_BYTES = slice_bytes_full<KIND>() / SPLIT;
@@ -507,29 +499,11 @@ k_apply2(const __grid_constant__ SketchDev S, const __grid_constant__ GroupLayou
         uint4* f = reinterpret_cast<uint4*>(minpos);
         for (uint32_t i = tid; i < SUB_BINS / 4; i += NTHR) f[i] = make_uint4(~0u, ~0u, ~0u, ~0u);
     }
-    if (gate) mbar_wait(bar, 0);   // ungated: the slice is first needed by the sweep, its load hides behind the record loop
+    // the slice is first needed by the sweep: its load hides behind the record loop
     constexpr int GPT = SUB_BINS / 8 / NTHR;
     if (KIND != BIT) {
-        // touch lanes start at 0, with bit 15 set for bins that hold a count already: the value atomicAdd returns then tells
-        // every record, at no extra cost, whether its bin was empty before the chunk — only those records can be a new k-mer's
-        // first toucher and pay the atomicMin below
 #pragma unroll
-        for (int q = 0; q < GPT; q++) {
-            const uint32_t g = q * NTHR + tid;
-            uint32_t w[4] = {0, 0, 0, 0};
-            if (gate && (uint64_t)g * (KIND == BYTE ? 8 : 4) < sbytes) {
-                if (KIND == BYTE) {
-                    const uint64_t old64 = *reinterpret_cast<const uint64_t*>(slice + (size_t)g * 8);
-#pragma unroll
-                    for (int j = 0; j < 8; j++) w[j >> 1] |= ((old64 >> (8 * j)) & 255u) ? (0x8000u << ((j & 1) * 16)) : 0u;
-                } else {
-                    const uint32_t old32 = *reinterpret_cast<const uint32_t*>(slice + (size_t)g * 4);
-#pragma unroll
-                    for (int j = 0; j < 8; j++) w[j >> 1] |= ((old32 >> ((j >> 1) * 8 + ((j & 1) ? 0 : 4))) & 15u) ? (0x8000u << ((j & 1) * 16)) : 0u;
-                }
-            }
-            reinterpret_cast<uint4*>(cnt)[g] = make_uint4(w[0], w[1], w[2], w[3]);
-        }
+        for (int q = 0; q < GPT; q++) reinterpret_cast<uint4*>(cnt)[q * NTHR + tid] = make_uint4(0, 0, 0, 0);
     }
     __syncthreads();
     const unsigned long long* src = st.rec + st.base(b);
@@ -556,36 +530,26 @@ k_apply2(const __grid_constant__ SketchDev S, const __grid_constant__ GroupLayou
                     if (lb / SUB_BINS != sub) continue;
                     lb &= SUB_BINS - 1;
                 }
-                if (KIND == BIT) {
-                    // a Bloom bit that is set already changes nothing
-                    if (!gate || slice_empty<KIND>(slice, lb)) atomicMin(&minpos[lb], (uint32_t)(v[j] >> BKT_SHIFT));
-                } else if (gate) {
-                    const uint32_t was = atomicAdd(&cnt[lb >> 1], (lb & 1) ? 0x10000u : 1u);
-                    if (!((lb & 1) ? was >> 31 : (was >> 15) & 1u)) atomicMin(&minpos[lb], (uint32_t)(v[j] >> BKT_SHIFT));
-                } else {
-                    // ungated: both updates leave at once, nothing waits for a result (the sweep ignores positions of bins that were occupied)
-                    atomicAdd(&cnt[lb >> 1], (lb & 1) ? 0x10000u : 1u);
-                    atomicMin(&minpos[lb], (uint32_t)(v[j] >> BKT_SHIFT));
-                }
+                // both updates leave at once, nothing waits for a result (the sweep ignores positions of bins that were occupied)
+                if (KIND != BIT) atomicAdd(&cnt[lb >> 1], (lb & 1) ? 0x10000u : 1u);
+                atomicMin(&minpos[lb], (uint32_t)(v[j] >> BKT_SHIFT));
             }
         }
-        // More records than a lane can count (15 bits when bit 15 is the "was occupied" flag, else 16): clamp every lane after each
-        // 16 Ki (32 Ki) records to a value the next round cannot push into the flag bit or the neighbouring lane — any value >=
-        // the counter's cap saturates it just the same.
-        const bool clamp_now = gate ? n > 32767u : (n > 65535u && (e0 / ITER_REC) % CLAMP_EVERY == CLAMP_EVERY - 1);
-        if (KIND != BIT && clamp_now) {
-            const uint32_t lim = gate ? 0x3FFFu : 0x7FFFu, keep = gate ? 0x80008000u : 0u, msk = gate ? 0x7FFFu : 0xFFFFu;
+        // More records than a 16-bit lane can count: clamp every lane after each 32 Ki records to a value the next round cannot
+        // push into the neighbouring lane — any value >= the counter's cap saturates it just the same.
+        if (KIND != BIT && n > 65535u && (e0 / ITER_REC) % CLAMP_EVERY == CLAMP_EVERY - 1) {
+            const uint32_t lim = 0x7FFFu;
             __syncthreads();
             for (uint32_t i = tid; i < SUB_BINS / 2; i += NTHR) {
                 const uint32_t w = cnt[i];
-                const uint32_t lo = w & msk, hi = (w >> 16) & msk;
-                cnt[i] = (w & keep) | (lo > lim ? lim : lo) | ((hi > lim ? lim : hi) << 16);
+                const uint32_t lo = w & 0xFFFFu, hi = w >> 16;
+                cnt[i] = (lo > lim ? lim : lo) | ((hi > lim ? lim : hi) << 16);
             }
             __syncthreads();
         }
     }
     __syncthreads();
-    if (!gate) mbar_wait(bar, 0);
+    mbar_wait(bar, 0);
     unsigned n_new = 0, n_sat = 0, n_cross = 0;
 #pragma unroll
     for (int q = 0; q < GPT; q++) {
@@ -610,8 +574,7 @@ k_apply2(const __grid_constant__ SketchDev S, const __grid_constant__ GroupLayou
                 }
             continue;
         }
-        uint4 c4 = reinterpret_cast<const uint4*>(cnt)[g];
-        if (gate) { c4.x &= 0x7FFF7FFFu; c4.y &= 0x7FFF7FFFu; c4.z &= 0x7FFF7FFFu; c4.w &= 0x7FFF7FFFu; }   // touches without the "was occupied" flags
+        const uint4 c4 = reinterpret_cast<const uint4*>(cnt)[g];
         if (!(c4.x | c4.y | c4.z | c4.w)) continue;
         const uint32_t cw[4] = {c4.x, c4.y, c4.z, c4.w};
         unsigned crossm = 0;

@@ -30,31 +30,23 @@ def test_gpu_matches_reference_golden(golden, name):
     check_case(make_gpu, rec)
 
 
-def test_gpu_golden_cases_in_pass_mode():
-    """All reference goldens again with the L2-blocked pass kernel forced (block of 3 kB, small chunks)."""
-    import subprocess, sys
-    env = dict(os.environ, KMGPU_DELTA="0", KMGPU_L2_BLOCK_BYTES="3000", KMGPU_MAX_PASSES="100000", KMGPU_CHUNK_BASES="65536")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", os.path.abspath(__file__), "-k",
-                        "test_gpu_matches_reference_golden and not C1 and not 25k"], env=env, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-
-
-def test_gpu_golden_cases_cas_single_pass():
-    """All reference goldens through the compare-and-swap kernel (the path huge tables take)."""
-    import subprocess, sys
-    env = dict(os.environ, KMGPU_DELTA="0")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", os.path.abspath(__file__), "-k",
-                        "test_gpu_matches_reference_golden and not C1 and not 25k"], env=env, capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-
-
 def test_gpu_golden_cases_grouped_path():
-    """The large-table goldens (C1 and the other 25k cases, 1e8-bin tables) through the grouped path (fused hash + grouping); by
-    default these shapes take the bins[] + k_bucketize path."""
+    """All reference goldens through the grouped path (fused hash + grouping), the small tables included; by default these
+    shapes take the bins[] + k_bucketize path or the delta passes."""
     import subprocess, sys
-    env = dict(os.environ, KMGPU_PREFER_BINS="0")
+    env = dict(os.environ, KMGPU_PREFER_BINS="0", KMGPU_GROUP_MIN_BUCKETS="0")
     r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", os.path.abspath(__file__), "-k",
-                        "test_gpu_matches_reference_golden and (C1 or 25k)"], env=env, capture_output=True, text=True)
+                        "test_gpu_matches_reference_golden"], env=env, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
+
+
+def test_gpu_golden_cases_no_delta_plan():
+    """All reference goldens with delta blocks so small that no table has a delta plan: the shapes the bins path could take
+    go to the grouped path instead, since the bins path needs the delta passes for a bucket that overflows."""
+    import subprocess, sys
+    env = dict(os.environ, KMGPU_DELTA_BLOCK_BINS="256", KMGPU_DELTA_MAX_PASSES="1", KMGPU_CHUNK_BASES="65536")
+    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", os.path.abspath(__file__), "-k",
+                        "test_gpu_matches_reference_golden and not C1 and not 25k"], env=env, capture_output=True, text=True)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
 
 
@@ -75,7 +67,7 @@ def _same_state(g, o, n_tables):
 
 
 @pytest.mark.parametrize("cls", list(ol.CLASSES))
-@pytest.mark.parametrize("chunk", [None, 4096, "cas-8192", "passes", "delta-blocks", "delta-cold", "delta-cold-stamps", "buckets",
+@pytest.mark.parametrize("chunk", [None, 4096, "bins-no-delta", "bins-no-delta-parts", "delta-blocks", "delta-cold", "delta-cold-stamps", "buckets",
                                    "buckets-overflow", "buckets-whole", "group", "group-whole", "group-regroup", "group-two",
                                    "group-two-regroup", "group-turns", "group-t16k", "count-passes"])
 def test_gpu_vs_oracle_random(cls, chunk, monkeypatch):
@@ -84,10 +76,10 @@ def test_gpu_vs_oracle_random(cls, chunk, monkeypatch):
     if chunk is not None:
         import subprocess, sys
         env = dict(os.environ, KMGPU_TEST_CLS=cls)
-        if chunk == "passes":   # compare-and-swap path, L2-blocked multi-pass mode forced on tiny tables
-            env.update(KMGPU_DELTA="0", KMGPU_L2_BLOCK_BYTES="1500", KMGPU_MAX_PASSES="64", KMGPU_CHUNK_BASES="16384")
-        elif chunk == "cas-8192":   # compare-and-swap path, all tables in one pass
-            env.update(KMGPU_DELTA="0", KMGPU_CHUNK_BASES="8192")
+        if chunk == "bins-no-delta":   # tables the bins path could take, too many delta blocks for its overflow fallback: grouped path
+            env.update(KMGPU_DELTA_BLOCK_BINS="256", KMGPU_DELTA_MAX_PASSES="1", KMGPU_CHUNK_BASES="16384")
+        elif chunk == "bins-no-delta-parts":   # same, host input in 16 parts per chunk (every chunk of a call keeps the grouped path)
+            env.update(KMGPU_DELTA_BLOCK_BINS="256", KMGPU_DELTA_MAX_PASSES="1", KMGPU_CHUNK_BASES="16384", KMGPU_PART_BASES="1000")
         elif chunk == "delta-cold":   # delta+fold path, per-block ("cold chunk") ranked-bitmap resolution forced
             env.update(KMGPU_DELTA_BLOCK_BINS="2000", KMGPU_COLD_MIN_NEW="1", KMGPU_CHUNK_BASES="32768", KMGPU_BUCKETS="0")
         elif chunk == "buckets":   # bucket path (records grouped by 32 Ki-bin bucket, applied in shared memory)
