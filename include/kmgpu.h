@@ -183,6 +183,31 @@ int kmgpu_normalize_batch(kmgpu_t* h, const char* seqs, const uint64_t* offsets,
                           const uint8_t* pair_with_next, uint32_t cutoff, uint8_t* keep_out, uint64_t* n_kept_out,
                           uint64_t* n_kmers_out);
 
+/* per-read outcome of the streaming trimmer (kmgpu_trim_low_abund_pass1 / pass2) */
+enum { KMGPU_TLA_DROP = 0,   /* no k-mer (shorter than k): the script's reader removes it; never makes its bundle consumed */
+       KMGPU_TLA_SKIP = 1,   /* pass 1, --diginorm: med >= D */
+       KMGPU_TLA_SAVE = 2,   /* pass 1: consumed, saved for pass 2 */
+       KMGPU_TLA_TRIM = 3,   /* trim_pos_out[r] = the length trim_on_abundance(read, C) keeps */
+       KMGPU_TLA_KEEP = 4 }; /* pass 2 with variable coverage: written untrimmed */
+
+/* The first pass of scripts/trim-low-abund.py:196-238 (Trimmer.pass1) for a batch of reads in stream order, bundles as in
+ * kmgpu_normalize_batch.  With med = the bundle's minimum get_median_count in the table as it is when the bundle arrives:
+ * med >= diginorm_coverage (0 = off) -> SKIP; else med >= trim_at_coverage -> TRIM against the table at arrival with cutoff;
+ * else every read of the bundle is consumed and SAVEd.  May be called on consecutive batches of one stream.  Results equal the
+ * serial loop: actions, trim lengths, tables, n_occupied, n_unique_kmers, bigcount map.  n_kmers_out: k-mers consumed.
+ * Cutoffs above 255 on a bigcount ByteStorage are not supported. */
+int kmgpu_trim_low_abund_pass1(kmgpu_t* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
+                               const uint8_t* pair_with_next, uint32_t trim_at_coverage, uint32_t cutoff,
+                               uint32_t diginorm_coverage /* 0 = off */, uint8_t* action_out, uint32_t* trim_pos_out,
+                               uint64_t* n_kmers_out);
+
+/* The second pass (Trimmer.pass2, scripts/trim-low-abund.py:240-271) over the saved reads against the current table: TRIM, or
+ * with variable_coverage != 0, TRIM a bundle whose every read has median_at_least(trim_at_coverage) and KEEP the others.
+ * The table is not changed. */
+int kmgpu_trim_low_abund_pass2(kmgpu_t* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
+                               const uint8_t* pair_with_next, uint32_t trim_at_coverage, uint32_t cutoff, int variable_coverage,
+                               uint8_t* action_out, uint32_t* trim_pos_out);
+
 /* ---- state -----------------------------------------------------------------------------
  * Storage::n_occupied / n_unique_kmers / n_tables / get_tablesizes (storage.hh:65-74). */
 int kmgpu_stats(kmgpu_t* h, uint64_t* n_occupied, uint64_t* n_unique_kmers);

@@ -39,8 +39,11 @@ SYMBOLS = [
     "kmgpu_shard_ipc_attach", "kmgpu_shard_attach_local", "kmgpu_shard_route", "kmgpu_shard_offsets", "kmgpu_shard_push", "kmgpu_shard_apply",
     "kmgpu_shard_count_new", "kmgpu_shard_stats", "kmgpu_shard_lookup", "kmgpu_shard_pull", "kmgpu_shard_kmer_counts",
     "kmgpu_shard_read_medians", "kmgpu_shard_median_at_least", "kmgpu_shard_trim", "kmgpu_shard_abundance_hist", "kmgpu_hll_create", "kmgpu_hll_destroy", "kmgpu_hll_consume",
-    "kmgpu_hll_get_registers", "kmgpu_hll_merge_registers",
+    "kmgpu_hll_get_registers", "kmgpu_hll_merge_registers", "kmgpu_trim_low_abund_pass1", "kmgpu_trim_low_abund_pass2",
 ]
+
+# per-read outcomes of the streaming trimmer (KMGPU_TLA_*)
+TLA_DROP, TLA_SKIP, TLA_SAVE, TLA_TRIM, TLA_KEEP = 0, 1, 2, 3, 4
 
 
 class Band(C.Structure):
@@ -101,6 +104,10 @@ def lib():
         L.kmgpu_trim_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, C.c_void_p]
         L.kmgpu_normalize_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32,
                                             C.c_void_p, u64p, u64p]
+        L.kmgpu_trim_low_abund_pass1.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32,
+                                                 C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, u64p]
+        L.kmgpu_trim_low_abund_pass2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32,
+                                                 C.c_uint32, C.c_int, C.c_void_p, C.c_void_p]
         L.kmgpu_consume_reads_new.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, u64p, u64p]
         L.kmgpu_first_touch_log.argtypes = [C.c_void_p, C.c_int]
         L.kmgpu_first_touch_resolve.argtypes = [C.c_void_p, u64p, u64p, C.c_void_p]
@@ -429,6 +436,37 @@ class Sketch:
                                           _ptr(pw) if pw is not None else None, int(cutoff), _ptr(keep), C.byref(kept),
                                           C.byref(kmers)))
         return keep[:nr], kmers.value
+
+    def trim_low_abund_pass1(self, reads, trim_at_coverage, cutoff, diginorm_coverage=None, paired=None, clean=False):
+        """Pass 1 of trim-low-abund (scripts/trim-low-abund.py:196-238) on a batch in stream order: per-read actions (TLA_*), trim
+        lengths (for TLA_TRIM) and the number of k-mers consumed.  `paired` as in normalize_batch."""
+        buf, off = as_reads(reads)
+        nr = len(off) - 1
+        act = np.zeros(max(nr, 1), dtype=np.uint8)
+        pos = np.zeros(max(nr, 1), dtype=np.uint32)
+        pw = None
+        if paired is not None:
+            pw = np.ascontiguousarray(paired, dtype=np.uint8)
+            assert len(pw) == nr
+        kmers = C.c_uint64()
+        check(lib().kmgpu_trim_low_abund_pass1(self.h, _ptr(buf), _ptr(off), nr, CLEAN if clean else 0, _ptr(pw), int(trim_at_coverage),
+                                               int(cutoff), int(diginorm_coverage or 0), _ptr(act), _ptr(pos), C.byref(kmers)))
+        return act[:nr], pos[:nr], kmers.value
+
+    def trim_low_abund_pass2(self, reads, trim_at_coverage, cutoff, variable_coverage=False, paired=None, clean=False):
+        """Pass 2 (scripts/trim-low-abund.py:240-271) over saved reads: per-read actions (TLA_TRIM / TLA_KEEP / TLA_DROP) and trim
+        lengths.  The table is not changed."""
+        buf, off = as_reads(reads)
+        nr = len(off) - 1
+        act = np.zeros(max(nr, 1), dtype=np.uint8)
+        pos = np.zeros(max(nr, 1), dtype=np.uint32)
+        pw = None
+        if paired is not None:
+            pw = np.ascontiguousarray(paired, dtype=np.uint8)
+            assert len(pw) == nr
+        check(lib().kmgpu_trim_low_abund_pass2(self.h, _ptr(buf), _ptr(off), nr, CLEAN if clean else 0, _ptr(pw), int(trim_at_coverage),
+                                               int(cutoff), int(bool(variable_coverage)), _ptr(act), _ptr(pos)))
+        return act[:nr], pos[:nr]
 
     # -- state
     def stats(self):

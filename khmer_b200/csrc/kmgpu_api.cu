@@ -239,6 +239,7 @@ struct kmgpu_sketch {
     DevBuf<uint32_t> d_htvals;
     DevBuf<Event> d_events;
     DevBuf<uint16_t> d_counts;
+    DevBuf<uint16_t> d_ocounts;             // normalization: counts under the overlay (d_counts keeps the window's start)
     DevBuf<uint64_t> d_hashes;
     DevBuf<uint64_t> d_hashin;
     DevBuf<uint16_t> d_stat_med;
@@ -2136,6 +2137,315 @@ extern "C" int kmgpu_abundance_distribution(kmgpu_t* counts, kmgpu_t* tracking, 
 // ------------------------------------------------------------------------------------------------------
 // digital normalization
 // ------------------------------------------------------------------------------------------------------
+// KMGPU_DEBUG: wall clock per phase of normalize_batch / trim_low_abund_pass1 (every phase ends in a synchronisation)
+struct NormClock {
+    const bool dbg = env_u64("KMGPU_DEBUG", 0) != 0;
+    // stage + first test, overlay test, in-between resolution, ingest of the kept reads, host loops;
+    // 5..8: parts of the in-between resolution; 9: refinement of trim-low-abund's pass 1
+    double t[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    double mark = dbg ? now() : 0;
+    static double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+    void lap(int i)
+    {
+        if (!dbg) return;
+        const double x = now();
+        t[i] += x - mark;
+        mark = x;
+    }
+};
+
+// one bit per read -> d_readbits
+static int upload_read_bits(kmgpu_sketch* h, const std::vector<uint8_t>& flag, uint32_t nr)
+{
+    std::vector<uint32_t> bits((nr + 31) / 32, 0u);
+    for (uint32_t r = 0; r < nr; r++)
+        if (flag[r]) bits[r >> 5] |= 1u << (r & 31);
+    CKR(h->d_readbits.ensure(bits.size()));
+    CK(cudaMemcpyAsync(h->d_readbits.p, bits.data(), bits.size() * 4, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));   // `bits` goes
+    return KMGPU_OK;
+}
+
+// end of the bundle that starts at read r of a window (pw: the window's pair flags, or null)
+static uint32_t bundle_end(const uint8_t* pw, uint32_t nr, uint32_t r)
+{
+    uint32_t e = r + 1;
+    while (e < nr && pw && pw[e - 1]) e++;
+    return e;
+}
+
+// A window of whole bundles, at most W reads and max_bases bases, from read r0 on; staged on the device.
+static int stage_window(kmgpu_sketch* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
+                        const uint8_t* pair_with_next, uint64_t r0, uint64_t W, ChunkPlan& c, ChunkDev& cd, uint64_t* r1_out)
+{
+    const uint64_t max_bases = chunk_bases() / 2;
+    uint64_t r1 = r0;
+    while (r1 < n_reads && r1 - r0 < W && offsets[r1 + 1] - offsets[r0] <= max_bases) r1++;
+    if (r1 == r0) r1 = r0 + 1;
+    while (r1 < n_reads && pair_with_next && pair_with_next[r1 - 1]) r1++;   // do not cut a pair
+    const uint32_t nr = (uint32_t)(r1 - r0);
+    c.base0 = offsets[r0];
+    c.base1 = offsets[r1];
+    c.offs.resize(nr + 1);
+    for (uint32_t r = 0; r <= nr; r++) c.offs[r] = (uint32_t)(offsets[r0 + r] - offsets[r0]);
+    *r1_out = r1;
+    return stage_chunk(h, seqs, c, flags, &cd, needs_acgt_check(h, flags));
+}
+
+// Steps 1-3 of digital normalization for one staged window with k-mers (cd.n_pos > 0): keep[r] = 1 iff read r's bundle is kept,
+// i.e. consumed in stream order.  h->d_counts keeps step 1's counts (the table at the window's start).  *any_cand: some bundle
+// was a candidate (steps 2-3 ran); *n_unsure: in-between reads.  *too_large: the in-between lists would pass 32 bits (refused).
+// `fl`: room to reserve for the lists from the start (large calls).
+static int norm_window_decide(kmgpu_sketch* h, const ChunkPlan& c, const ChunkDev& cd, const uint8_t* pw, uint32_t cutoff, size_t fl,
+                              NormClock& clk, std::vector<uint8_t>& keep, bool* any_cand, uint64_t* n_unsure_out, bool* too_large)
+{
+    cudaStream_t st = h->stream;
+    const HashCfg H{h->hash, h->k};
+    const int N = h->nt;
+    const uint32_t cap_c = h->kind == BYTE ? 255u : h->kind == NIBBLE ? 15u : 1u;
+    const uint32_t nr = cd.n_reads;
+    *any_cand = false;
+    *n_unsure_out = 0;
+    *too_large = false;
+    keep.assign(nr, 0);
+    Input in = make_input(cd);
+    // 1. median_at_least of every read in the table as it is at the window's start
+    if (h->kind == BYTE && h->use_bigcount) CKR(sync_big_to_device(h));
+    const uint32_t nb = (h->kind == BYTE && h->use_bigcount) ? h->n_big_dev : 0;
+    CKR(h->d_counts.ensure(cd.n_pos));
+    CKR(h->d_stat_n.ensure(nr));
+    CKR(h->d_stat_b.ensure(nr));
+    launch_counts(0, h->dev, H, in, h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, st);
+    k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, nullptr, nullptr, nullptr, h->d_stat_n.p, cutoff, h->d_stat_b.p);
+    h->all_launches += 2;
+    CK(cudaGetLastError());
+    std::vector<uint8_t> al1(nr), al2;
+    CK(cudaMemcpyAsync(al1.data(), h->d_stat_b.p, nr, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    clk.lap(0);
+    // candidates: bundles with a read below the cutoff (a read without k-mers never makes its bundle a candidate)
+    std::vector<uint8_t> cand(nr, 0);
+    uint64_t cand_bases = 0, n_cand = 0;
+    for (uint32_t r = 0; r < nr;) {
+        const uint32_t e = bundle_end(pw, nr, r);
+        bool below = false;
+        for (uint32_t q = r; q < e; q++) below |= al1[q] == 0;
+        if (below)
+            for (uint32_t q = r; q < e; q++) {
+                cand[q] = 1;
+                cand_bases += c.offs[q + 1] - c.offs[q];
+                n_cand++;
+            }
+        r = e;
+    }
+    if (!n_cand) return KMGPU_OK;
+    *any_cand = true;
+    // 2. the same test with every candidate of the window added on top (overlay): still below => kept for good.  The overlay's
+    //    counts go to their own buffer.
+    CKR(upload_read_bits(h, cand, nr));
+    const uint64_t slots = pow2_at_least(2 * cand_bases * (uint64_t)N);
+    CKR(h->d_htkeys.ensure(slots));
+    CKR(h->d_htvals.ensure(slots));
+    CKR(h->d_ocounts.ensure(cd.n_pos));
+    CK(cudaMemsetAsync(h->d_htkeys.p, 0xFF, slots * 8, st));
+    CK(cudaMemsetAsync(h->d_htvals.p, 0, slots * 4, st));
+    in.read_keep = h->d_readbits.p;
+    const unsigned gt = n_tiles(cd.n_pos);
+    if (H.kind == TWOBIT) k_norm_overlay_add<TWOBIT, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1);
+    else k_norm_overlay_add<MURMUR, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1);
+#define NORM_COUNTS(KIND)                                                                                                                  \
+    do {                                                                                                                                   \
+        if (H.kind == TWOBIT) k_norm_counts_overlay<KIND, TWOBIT, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1, h->d_ocounts.p); \
+        else k_norm_counts_overlay<KIND, MURMUR, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1, h->d_ocounts.p);                 \
+    } while (0)
+    if (h->kind == BYTE) NORM_COUNTS(BYTE);
+    else if (h->kind == NIBBLE) NORM_COUNTS(NIBBLE);
+    else NORM_COUNTS(BIT);
+#undef NORM_COUNTS
+    k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(h->d_ocounts.p, cd.offs, nr, h->k, nullptr, nullptr, nullptr, h->d_stat_n.p, cutoff, h->d_stat_b.p);
+    h->all_launches += 3;
+    CK(cudaGetLastError());
+    al2.resize(nr);
+    CK(cudaMemcpyAsync(al2.data(), h->d_stat_b.p, nr, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    clk.lap(1);
+    std::vector<uint8_t> sure(nr, 0), unsure(nr, 0);
+    uint64_t n_unsure = 0, up_total = 0;
+    for (uint32_t r = 0; r < nr;) {
+        const uint32_t e = bundle_end(pw, nr, r);
+        if (cand[r]) {
+            bool below = false;
+            for (uint32_t q = r; q < e; q++) below |= al2[q] == 0;
+            for (uint32_t q = r; q < e; q++) {
+                (below ? sure : unsure)[q] = 1;
+                if (!below) {
+                    n_unsure++;
+                    const uint32_t len = c.offs[q + 1] - c.offs[q];
+                    if (len >= (uint32_t)h->k) up_total += len - h->k + 1;
+                }
+            }
+        }
+        r = e;
+    }
+    keep = sure;
+    *n_unsure_out = n_unsure;
+    if (n_unsure) {
+        // 3. in-between bundles: the state each of them meets is the window's start + the candidates kept before it.
+        //    Gather, for every k-mer of theirs, the counters at the window's start and the touches of its bins by the
+        //    window's candidates (position, read); then decide in rounds on the device (k_norm_resolve).
+        h->n_norm_unsure += n_unsure;
+        std::vector<uint32_t> upos, meta_ub, meta_start, meta_ur, meta_read;
+        upos.reserve(up_total);
+        meta_ur.push_back(0);
+        for (uint32_t r = 0; r < nr;) {
+            const uint32_t e = bundle_end(pw, nr, r);
+            if (unsure[r]) {
+                meta_ub.push_back((uint32_t)meta_read.size());
+                meta_start.push_back(c.offs[r]);
+                for (uint32_t q = r; q < e; q++) {
+                    const uint32_t s0 = c.offs[q], len = c.offs[q + 1] - s0;
+                    for (uint32_t i = 0; i + h->k <= len; i++) upos.push_back(s0 + i);
+                    meta_read.push_back(q);
+                    meta_ur.push_back((uint32_t)upos.size());
+                }
+            }
+            r = e;
+        }
+        meta_ub.push_back((uint32_t)meta_read.size());
+        const uint32_t n_up = (uint32_t)upos.size(), n_ub = (uint32_t)meta_start.size();
+        std::vector<uint8_t> state(nr, 0);
+        for (uint32_t r = 0; r < nr; r++) state[r] = sure[r] ? 1 : unsure[r] ? 2 : 0;
+        double t_sub = clk.dbg ? NormClock::now() : 0;
+        auto sub = [&](int i) {
+            if (!clk.dbg) return;
+            const double t = NormClock::now();
+            clk.t[i] += t - t_sub;
+            t_sub = t;
+        };
+        sub(5);   // host: the lists of the in-between bundles
+        if (n_up) {
+            const uint64_t slots2 = pow2_at_least(2 * (uint64_t)n_up * N);
+            if (slots2 > (1ull << 32)) {
+                *too_large = true;
+                return fail(KMGPU_EUNSUPPORTED, "normalize_batch: window too large");
+            }
+            // one upload: upos | ub_first | ub_start | ur_first | ur_read
+            std::vector<uint32_t> pack;
+            pack.reserve((size_t)n_up + meta_ub.size() + meta_start.size() + meta_ur.size() + meta_read.size());
+            pack.insert(pack.end(), upos.begin(), upos.end());
+            const size_t o_ub = pack.size();
+            pack.insert(pack.end(), meta_ub.begin(), meta_ub.end());
+            const size_t o_st = pack.size();
+            pack.insert(pack.end(), meta_start.begin(), meta_start.end());
+            const size_t o_ur = pack.size();
+            pack.insert(pack.end(), meta_ur.begin(), meta_ur.end());
+            const size_t o_rd = pack.size();
+            pack.insert(pack.end(), meta_read.begin(), meta_read.end());
+            // large calls: room for a typical window's in-between reads from the start (growing these buffers window
+            // by window costs a cudaFree + cudaMalloc each time, milliseconds apiece on some hosts)
+            CKR(h->d_upos.ensure(std::max(pack.size(), fl + fl / 8)));
+            CKR(h->d_nslot.ensure(std::max((size_t)n_up, fl) * N));
+            CKR(h->d_uc0.ensure(std::max((size_t)n_up, fl) * N));
+            CKR(h->d_evkeys.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
+            CKR(h->d_ncnt.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
+            CKR(h->d_nfill.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
+            CKR(h->d_nstate.ensure(std::max<size_t>(nr, fl ? (size_t)1 << 17 : 0)));
+            CK(cudaMemcpyAsync(h->d_upos.p, pack.data(), pack.size() * 4, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(h->d_nstate.p, state.data(), nr, cudaMemcpyHostToDevice, st));
+            CK(cudaMemsetAsync(h->d_evkeys.p, 0xFF, slots2 * 8, st));
+            CK(cudaMemsetAsync(h->d_ncnt.p, 0, slots2 * 4, st));
+            CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
+            uint64_t* keys2 = reinterpret_cast<uint64_t*>(h->d_evkeys.p);
+            Input in0 = make_input(cd);
+#define NORM_GATHER(KIND)                                                                                                                                    \
+    do {                                                                                                                                                     \
+        if (H.kind == TWOBIT) k_norm_gather<KIND, TWOBIT><<<(n_up + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, n_up, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1); \
+        else k_norm_gather<KIND, MURMUR><<<(n_up + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, n_up, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1);               \
+    } while (0)
+            if (h->kind == BYTE) NORM_GATHER(BYTE);
+            else if (h->kind == NIBBLE) NORM_GATHER(NIBBLE);
+            else NORM_GATHER(BIT);
+#undef NORM_GATHER
+            Input inc = make_input(cd);
+            inc.read_keep = h->d_readbits.p;   // still the candidates' bits (uploaded for the overlay)
+            if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
+            else k_norm_hits<MURMUR, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
+            k_norm_hit_offsets<<<148 * 8, 256, 0, st>>>(h->d_ncnt.p, h->d_nfill.p, slots2, &h->d_ctrl->n_events);
+            h->all_launches += 3;
+            CK(cudaGetLastError());
+            CKR(read_ctrl(h));   // synchronises: the host vectors above may go
+            sub(6);   // uploads, gather, counting pass of the hits
+            const uint64_t n_hits = h->h_ctrl->n_events;
+            if (n_hits >= (1ull << 32)) {
+                *too_large = true;
+                return fail(KMGPU_EUNSUPPORTED, "normalize_batch: window too large");
+            }
+            CKR(h->d_nhits.ensure(std::max<uint64_t>(std::max<uint64_t>(n_hits, 1), 8 * (uint64_t)fl)));
+            if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
+            else k_norm_hits<MURMUR, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
+            h->all_launches += 1;
+            NormResolve R;
+            R.ub_first = h->d_upos.p + o_ub;
+            R.ub_start = h->d_upos.p + o_st;
+            R.ur_first = h->d_upos.p + o_ur;
+            R.ur_read = h->d_upos.p + o_rd;
+            R.slot = h->d_nslot.p;
+            R.c0 = h->d_uc0.p;
+            R.cnt = h->d_ncnt.p;
+            R.fill = h->d_nfill.p;
+            R.hits = h->d_nhits.p;
+            R.state = h->d_nstate.p;
+            R.n_tables = N;
+            R.cutoff = cutoff;
+            R.cap = cap_c;
+            unsigned int* n_left = reinterpret_cast<unsigned int*>(&h->d_ctrl->n_events);
+            if (clk.dbg) CK(cudaStreamSynchronize(st));
+            sub(7);   // fill pass of the hits
+            for (uint64_t round = 0;; round++) {
+                // two rounds per look at the counter (a round is a few microseconds, the look a round trip)
+                CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
+                k_norm_resolve<<<(n_ub + 7) / 8, 256, 0, st>>>(R, n_ub, n_left);
+                CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
+                k_norm_resolve<<<(n_ub + 7) / 8, 256, 0, st>>>(R, n_ub, n_left);
+                h->all_launches += 2;
+                h->n_norm_rounds += 2;
+                CK(cudaGetLastError());
+                CKR(read_ctrl(h));
+                if (h->h_ctrl->n_events == 0) break;
+                if (round > n_ub) return fail(KMGPU_ECUDA, "normalize_batch: the in-between resolution does not converge");
+            }
+            CK(cudaMemcpyAsync(state.data(), h->d_nstate.p, nr, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            sub(8);   // rounds
+        } else {
+            // in-between bundles without a single k-mer cannot be "below": never kept (they were no candidates at all)
+            for (uint32_t r = 0; r < nr; r++)
+                if (state[r] == 2) state[r] = 0;
+        }
+        for (uint32_t r = 0; r < nr; r++) keep[r] = state[r] == 1;
+    }
+    clk.lap(2);
+    return KMGPU_OK;
+}
+
+// 4. the kept reads of a window are consumed in stream order (one ordinary ingest with a read mask); adds the k-mers consumed
+static int norm_window_ingest(kmgpu_sketch* h, const ChunkDev& cd, const std::vector<uint8_t>& keep, uint64_t* n_kmers)
+{
+    const uint32_t nr = cd.n_reads;
+    uint64_t nk_reads = 0;
+    for (uint32_t r = 0; r < nr; r++) nk_reads += keep[r];
+    if (!nk_reads) return KMGPU_OK;
+    CKR(upload_read_bits(h, keep, nr));
+    Input ink = make_input(cd);
+    ink.read_keep = h->d_readbits.p;
+    ChunkResult res;
+    Pred P0;
+    memset(&P0, 0, sizeof P0);
+    CKR(ingest_chunk(h, 0, HashCfg{h->hash, h->k}, {Part{ink, 0u, nullptr}}, P0, false, nullptr, &res));
+    *n_kmers += res.n_kmers;
+    return KMGPU_OK;
+}
+
 extern "C" int kmgpu_normalize_batch(kmgpu_t* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
                                      const uint8_t* pair_with_next, uint32_t cutoff, uint8_t* keep_out, uint64_t* n_kept_out,
                                      uint64_t* n_kmers_out)
@@ -2153,302 +2463,287 @@ extern "C" int kmgpu_normalize_batch(kmgpu_t* h, const char* seqs, const uint64_
     if (pair_with_next && pair_with_next[n_reads - 1]) return fail(KMGPU_EINVAL, "the last read cannot be paired with a next one");
     std::lock_guard<std::mutex> g(h->mu);
     CKR(set_device(h->device));
-    cudaStream_t st = h->stream;
-    const HashCfg H{h->hash, h->k};
-    const int N = h->nt;
-    const uint32_t cap_c = h->kind == BYTE ? 255u : h->kind == NIBBLE ? 15u : 1u;
     // reads per window: fixed by KMGPU_NORM_WINDOW, else adapted so that only a small share of a window's bundles is "in between"
     // (their number grows with the coverage a window adds; they are resolved one by one on the host)
     const uint64_t W_fixed = env_u64("KMGPU_NORM_WINDOW", 0);
     uint64_t W = W_fixed ? std::max<uint64_t>(2, W_fixed) : 32768;
     uint64_t n_windows = 0;
     const uint64_t unsure0 = h->n_norm_unsure, rounds0 = h->n_norm_rounds;
-    // KMGPU_DEBUG: wall clock per phase (every phase ends in a synchronisation)
-    const bool dbg = env_u64("KMGPU_DEBUG", 0) != 0;
-    double t_phase[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // stage + first test, overlay test, in-between resolution, ingest of the kept reads,
-                                                          // host loops; 5..8: parts of the in-between resolution
-    auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    double t_mark = dbg ? now() : 0;
-    auto lap = [&](int i) {
-        if (!dbg) return;
-        const double t = now();
-        t_phase[i] += t - t_mark;
-        t_mark = t;
-    };
-    const uint64_t max_bases = chunk_bases() / 2;
-    Pred P0;
-    memset(&P0, 0, sizeof P0);
+    NormClock clk;
+    const size_t fl = n_reads >= 100000 ? ((size_t)1 << 21) : 0;
     uint64_t kept_total = 0, kmers_total = 0;
-    std::vector<uint8_t> al1, al2;
-    std::vector<uint32_t> bits;
-    auto upload_bits = [&](const std::vector<uint8_t>& flag, uint32_t nr) -> int {   // one bit per read -> d_readbits
-        bits.assign((nr + 31) / 32, 0u);
-        for (uint32_t r = 0; r < nr; r++)
-            if (flag[r]) bits[r >> 5] |= 1u << (r & 31);
-        CKR(h->d_readbits.ensure(bits.size()));
-        CK(cudaMemcpyAsync(h->d_readbits.p, bits.data(), bits.size() * 4, cudaMemcpyHostToDevice, st));
-        CK(cudaStreamSynchronize(st));   // `bits` is reused
-        return KMGPU_OK;
-    };
+    std::vector<uint8_t> keep;
     for (uint64_t r0 = 0; r0 < n_reads;) {
-        // window of whole bundles, at most W reads and max_bases bases
-        uint64_t r1 = r0;
-        while (r1 < n_reads && r1 - r0 < W && offsets[r1 + 1] - offsets[r0] <= max_bases) r1++;
-        if (r1 == r0) r1 = r0 + 1;
-        while (r1 < n_reads && pair_with_next && pair_with_next[r1 - 1]) r1++;   // do not cut a pair
+        ChunkPlan c;
+        ChunkDev cd;
+        uint64_t r1;
+        CKR(stage_window(h, seqs, offsets, n_reads, flags, pair_with_next, r0, W, c, cd, &r1));
         const uint32_t nr = (uint32_t)(r1 - r0);
         n_windows++;
-        ChunkPlan c;
-        c.base0 = offsets[r0];
-        c.base1 = offsets[r1];
-        c.offs.resize(nr + 1);
-        for (uint32_t r = 0; r <= nr; r++) c.offs[r] = (uint32_t)(offsets[r0 + r] - offsets[r0]);
-        ChunkDev cd;
-        CKR(stage_chunk(h, seqs, c, flags, &cd, needs_acgt_check(h, flags)));
-        auto bundle_end = [&](uint32_t r) { uint32_t e = r + 1; while (e < nr && pair_with_next && pair_with_next[r0 + e - 1]) e++; return e; };
-        std::vector<uint8_t> keep(nr, 0);
+        keep.assign(nr, 0);
         if (cd.n_pos) {
-            Input in = make_input(cd);
-            // 1. median_at_least of every read in the table as it is at the window's start
-            if (h->kind == BYTE && h->use_bigcount) CKR(sync_big_to_device(h));
-            const uint32_t nb = (h->kind == BYTE && h->use_bigcount) ? h->n_big_dev : 0;
-            CKR(h->d_counts.ensure(cd.n_pos));
-            CKR(h->d_stat_n.ensure(nr));
-            CKR(h->d_stat_b.ensure(nr));
-            launch_counts(0, h->dev, H, in, h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, st);
-            k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, nullptr, nullptr, nullptr, h->d_stat_n.p, cutoff, h->d_stat_b.p);
-            h->all_launches += 2;
-            CK(cudaGetLastError());
-            al1.resize(nr);
-            CK(cudaMemcpyAsync(al1.data(), h->d_stat_b.p, nr, cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            lap(0);
-            // candidates: bundles with a read below the cutoff (a read without k-mers never makes its bundle a candidate)
-            std::vector<uint8_t> cand(nr, 0);
-            uint64_t cand_bases = 0, n_cand = 0;
-            for (uint32_t r = 0; r < nr;) {
-                const uint32_t e = bundle_end(r);
-                bool below = false;
-                for (uint32_t q = r; q < e; q++) below |= al1[q] == 0;
-                if (below)
-                    for (uint32_t q = r; q < e; q++) {
-                        cand[q] = 1;
-                        cand_bases += c.offs[q + 1] - c.offs[q];
-                        n_cand++;
-                    }
-                r = e;
-            }
-            if (n_cand) {
-                // 2. the same test with every candidate of the window added on top (overlay): still below => kept for good
-                CKR(upload_bits(cand, nr));
-                const uint64_t slots = pow2_at_least(2 * cand_bases * (uint64_t)N);
-                CKR(h->d_htkeys.ensure(slots));
-                CKR(h->d_htvals.ensure(slots));
-                CK(cudaMemsetAsync(h->d_htkeys.p, 0xFF, slots * 8, st));
-                CK(cudaMemsetAsync(h->d_htvals.p, 0, slots * 4, st));
-                in.read_keep = h->d_readbits.p;
-                const unsigned gt = n_tiles(cd.n_pos);
-                if (H.kind == TWOBIT) k_norm_overlay_add<TWOBIT, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1);
-                else k_norm_overlay_add<MURMUR, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1);
-#define NORM_COUNTS(KIND)                                                                                                                  \
-    do {                                                                                                                                   \
-        if (H.kind == TWOBIT) k_norm_counts_overlay<KIND, TWOBIT, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1, h->d_counts.p); \
-        else k_norm_counts_overlay<KIND, MURMUR, 0><<<gt, THREADS, 0, st>>>(h->dev, H, in, h->d_htkeys.p, h->d_htvals.p, slots - 1, h->d_counts.p);                 \
-    } while (0)
-                if (h->kind == BYTE) NORM_COUNTS(BYTE);
-                else if (h->kind == NIBBLE) NORM_COUNTS(NIBBLE);
-                else NORM_COUNTS(BIT);
-#undef NORM_COUNTS
-                k_read_stats<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, nullptr, nullptr, nullptr, h->d_stat_n.p, cutoff, h->d_stat_b.p);
-                h->all_launches += 3;
-                CK(cudaGetLastError());
-                al2.resize(nr);
-                CK(cudaMemcpyAsync(al2.data(), h->d_stat_b.p, nr, cudaMemcpyDeviceToHost, st));
-                CK(cudaStreamSynchronize(st));
-                lap(1);
-                std::vector<uint8_t> sure(nr, 0), unsure(nr, 0);
-                uint64_t n_unsure = 0, up_total = 0;
-                for (uint32_t r = 0; r < nr;) {
-                    const uint32_t e = bundle_end(r);
-                    if (cand[r]) {
-                        bool below = false;
-                        for (uint32_t q = r; q < e; q++) below |= al2[q] == 0;
-                        for (uint32_t q = r; q < e; q++) {
-                            (below ? sure : unsure)[q] = 1;
-                            if (!below) {
-                                n_unsure++;
-                                const uint32_t len = c.offs[q + 1] - c.offs[q];
-                                if (len >= (uint32_t)h->k) up_total += len - h->k + 1;
-                            }
-                        }
-                    }
-                    r = e;
-                }
-                keep = sure;
+            bool any_cand, too_large;
+            uint64_t n_unsure;
+            CKR(norm_window_decide(h, c, cd, pair_with_next ? pair_with_next + r0 : nullptr, cutoff, fl, clk, keep, &any_cand, &n_unsure,
+                                   &too_large));
+            if (any_cand) {
                 if (!W_fixed) {
                     // a window costs ~1 ms of launches and round trips whatever its size; the in-between bundles (their number grows
                     // with the square of the window) cost a few rounds of k_norm_resolve over their k-mers
                     if (n_unsure > 8192) W = std::max<uint64_t>(2048, W / 2);
                     else if (n_unsure < 2048) W = std::min<uint64_t>(1u << 17, W * 2);
                 }
-                if (n_unsure) {
-                    // 3. in-between bundles: the state each of them meets is the window's start + the candidates kept before it.
-                    //    Gather, for every k-mer of theirs, the counters at the window's start and the touches of its bins by the
-                    //    window's candidates (position, read); then decide in rounds on the device (k_norm_resolve).
-                    h->n_norm_unsure += n_unsure;
-                    std::vector<uint32_t> upos, meta_ub, meta_start, meta_ur, meta_read;
-                    upos.reserve(up_total);
-                    meta_ur.push_back(0);
-                    for (uint32_t r = 0; r < nr;) {
-                        const uint32_t e = bundle_end(r);
-                        if (unsure[r]) {
-                            meta_ub.push_back((uint32_t)meta_read.size());
-                            meta_start.push_back(c.offs[r]);
-                            for (uint32_t q = r; q < e; q++) {
-                                const uint32_t s0 = c.offs[q], len = c.offs[q + 1] - s0;
-                                for (uint32_t i = 0; i + h->k <= len; i++) upos.push_back(s0 + i);
-                                meta_read.push_back(q);
-                                meta_ur.push_back((uint32_t)upos.size());
-                            }
-                        }
-                        r = e;
-                    }
-                    meta_ub.push_back((uint32_t)meta_read.size());
-                    const uint32_t n_up = (uint32_t)upos.size(), n_ub = (uint32_t)meta_start.size(), n_ur = (uint32_t)meta_read.size();
-                    std::vector<uint8_t> state(nr, 0);
-                    for (uint32_t r = 0; r < nr; r++) state[r] = sure[r] ? 1 : unsure[r] ? 2 : 0;
-                    double t_sub = dbg ? now() : 0;
-                    auto sub = [&](int i) {
-                        if (!dbg) return;
-                        const double t = now();
-                        t_phase[i] += t - t_sub;
-                        t_sub = t;
-                    };
-                    sub(5);   // host: the lists of the in-between bundles
-                    if (n_up) {
-                        const uint64_t slots2 = pow2_at_least(2 * (uint64_t)n_up * N);
-                        if (slots2 > (1ull << 32)) return fail(KMGPU_EUNSUPPORTED, "normalize_batch: window too large");
-                        // one upload: upos | ub_first | ub_start | ur_first | ur_read
-                        std::vector<uint32_t> pack;
-                        pack.reserve((size_t)n_up + meta_ub.size() + meta_start.size() + meta_ur.size() + meta_read.size());
-                        pack.insert(pack.end(), upos.begin(), upos.end());
-                        const size_t o_ub = pack.size();
-                        pack.insert(pack.end(), meta_ub.begin(), meta_ub.end());
-                        const size_t o_st = pack.size();
-                        pack.insert(pack.end(), meta_start.begin(), meta_start.end());
-                        const size_t o_ur = pack.size();
-                        pack.insert(pack.end(), meta_ur.begin(), meta_ur.end());
-                        const size_t o_rd = pack.size();
-                        pack.insert(pack.end(), meta_read.begin(), meta_read.end());
-                        // large calls: room for a typical window's in-between reads from the start (growing these buffers window
-                        // by window costs a cudaFree + cudaMalloc each time, milliseconds apiece on some hosts)
-                        const size_t fl = n_reads >= 100000 ? ((size_t)1 << 21) : 0;
-                        CKR(h->d_upos.ensure(std::max(pack.size(), fl + fl / 8)));
-                        CKR(h->d_nslot.ensure(std::max((size_t)n_up, fl) * N));
-                        CKR(h->d_uc0.ensure(std::max((size_t)n_up, fl) * N));
-                        CKR(h->d_evkeys.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
-                        CKR(h->d_ncnt.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
-                        CKR(h->d_nfill.ensure(std::max<uint64_t>(slots2, pow2_at_least(2 * (uint64_t)fl * N))));
-                        CKR(h->d_nstate.ensure(std::max<size_t>(nr, fl ? (size_t)1 << 17 : 0)));
-                        CK(cudaMemcpyAsync(h->d_upos.p, pack.data(), pack.size() * 4, cudaMemcpyHostToDevice, st));
-                        CK(cudaMemcpyAsync(h->d_nstate.p, state.data(), nr, cudaMemcpyHostToDevice, st));
-                        CK(cudaMemsetAsync(h->d_evkeys.p, 0xFF, slots2 * 8, st));
-                        CK(cudaMemsetAsync(h->d_ncnt.p, 0, slots2 * 4, st));
-                        CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
-                        uint64_t* keys2 = reinterpret_cast<uint64_t*>(h->d_evkeys.p);
-                        Input in0 = make_input(cd);
-#define NORM_GATHER(KIND)                                                                                                                                    \
-    do {                                                                                                                                                     \
-        if (H.kind == TWOBIT) k_norm_gather<KIND, TWOBIT><<<(n_up + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, n_up, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1); \
-        else k_norm_gather<KIND, MURMUR><<<(n_up + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, n_up, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1);               \
-    } while (0)
-                        if (h->kind == BYTE) NORM_GATHER(BYTE);
-                        else if (h->kind == NIBBLE) NORM_GATHER(NIBBLE);
-                        else NORM_GATHER(BIT);
-#undef NORM_GATHER
-                        Input inc = make_input(cd);
-                        inc.read_keep = h->d_readbits.p;   // still the candidates' bits (uploaded for the overlay)
-                        if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
-                        else k_norm_hits<MURMUR, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
-                        k_norm_hit_offsets<<<148 * 8, 256, 0, st>>>(h->d_ncnt.p, h->d_nfill.p, slots2, &h->d_ctrl->n_events);
-                        h->all_launches += 3;
-                        CK(cudaGetLastError());
-                        CKR(read_ctrl(h));   // synchronises: the host vectors above may go
-                        sub(6);   // uploads, gather, counting pass of the hits
-                        const uint64_t n_hits = h->h_ctrl->n_events;
-                        if (n_hits >= (1ull << 32)) return fail(KMGPU_EUNSUPPORTED, "normalize_batch: window too large");
-                        CKR(h->d_nhits.ensure(std::max<uint64_t>(std::max<uint64_t>(n_hits, 1), 8 * (uint64_t)fl)));
-                        if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
-                        else k_norm_hits<MURMUR, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
-                        h->all_launches += 1;
-                        NormResolve R;
-                        R.ub_first = h->d_upos.p + o_ub;
-                        R.ub_start = h->d_upos.p + o_st;
-                        R.ur_first = h->d_upos.p + o_ur;
-                        R.ur_read = h->d_upos.p + o_rd;
-                        R.slot = h->d_nslot.p;
-                        R.c0 = h->d_uc0.p;
-                        R.cnt = h->d_ncnt.p;
-                        R.fill = h->d_nfill.p;
-                        R.hits = h->d_nhits.p;
-                        R.state = h->d_nstate.p;
-                        R.n_tables = N;
-                        R.cutoff = cutoff;
-                        R.cap = cap_c;
-                        unsigned int* n_left = reinterpret_cast<unsigned int*>(&h->d_ctrl->n_events);
-                        if (dbg) CK(cudaStreamSynchronize(st));
-                        sub(7);   // fill pass of the hits
-                        for (uint64_t round = 0;; round++) {
-                            // two rounds per look at the counter (a round is a few microseconds, the look a round trip)
-                            CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
-                            k_norm_resolve<<<(n_ub + 7) / 8, 256, 0, st>>>(R, n_ub, n_left);
-                            CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
-                            k_norm_resolve<<<(n_ub + 7) / 8, 256, 0, st>>>(R, n_ub, n_left);
-                            h->all_launches += 2;
-                            h->n_norm_rounds += 2;
-                            CK(cudaGetLastError());
-                            CKR(read_ctrl(h));
-                            if (h->h_ctrl->n_events == 0) break;
-                            if (round > n_ub) return fail(KMGPU_ECUDA, "normalize_batch: the in-between resolution does not converge");
-                        }
-                        CK(cudaMemcpyAsync(state.data(), h->d_nstate.p, nr, cudaMemcpyDeviceToHost, st));
-                        CK(cudaStreamSynchronize(st));
-                        sub(8);   // rounds
-                    } else {
-                        // in-between bundles without a single k-mer cannot be "below": never kept (they were no candidates at all)
-                        for (uint32_t r = 0; r < nr; r++)
-                            if (state[r] == 2) state[r] = 0;
-                    }
-                    for (uint32_t r = 0; r < nr; r++) keep[r] = state[r] == 1;
-                }
-                lap(2);
-                // 4. the kept reads are consumed in stream order (one ordinary ingest with a read mask)
-                uint64_t nk_reads = 0;
-                for (uint32_t r = 0; r < nr; r++) nk_reads += keep[r];
-                if (nk_reads) {
-                    CKR(upload_bits(keep, nr));
-                    Input ink = make_input(cd);
-                    ink.read_keep = h->d_readbits.p;
-                    ChunkResult res;
-                    CKR(ingest_chunk(h, 0, H, {Part{ink, 0u, nullptr}}, P0, false, nullptr, &res));
-                    kmers_total += res.n_kmers;
-                    kept_total += nk_reads;
-                }
-                lap(3);
+                CKR(norm_window_ingest(h, cd, keep, &kmers_total));
+                for (uint32_t r = 0; r < nr; r++) kept_total += keep[r];
+                clk.lap(3);
             }
         }
         memcpy(keep_out + r0, keep.data(), nr);
-        lap(4);
+        clk.lap(4);
         r0 = r1;
     }
     if (n_kept_out) *n_kept_out = kept_total;
     if (n_kmers_out) *n_kmers_out = kmers_total;
-    if (dbg)
+    if (clk.dbg)
         fprintf(stderr, "[kmgpu] normalize_batch: %llu reads in %llu windows (last %llu reads), %llu in-between reads, %llu resolve rounds; "
                         "seconds: first test %.3f, overlay test %.3f, in-between %.3f (lists %.3f, gather + count %.3f, fill %.3f, rounds %.3f), ingest %.3f, other %.3f\n",
                 (unsigned long long)n_reads, (unsigned long long)n_windows, (unsigned long long)W,
-                (unsigned long long)(h->n_norm_unsure - unsure0), (unsigned long long)(h->n_norm_rounds - rounds0), t_phase[0], t_phase[1], t_phase[2],
-                t_phase[5], t_phase[6], t_phase[7], t_phase[8], t_phase[3], t_phase[4]);
+                (unsigned long long)(h->n_norm_unsure - unsure0), (unsigned long long)(h->n_norm_rounds - rounds0), clk.t[0], clk.t[1], clk.t[2],
+                clk.t[5], clk.t[6], clk.t[7], clk.t[8], clk.t[3], clk.t[4]);
+    return KMGPU_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------
+// trim-low-abund (scripts/trim-low-abund.py:196-271, khmer/trimming.py:36-66)
+// ------------------------------------------------------------------------------------------------------
+extern "C" int kmgpu_trim_low_abund_pass1(kmgpu_t* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
+                                          const uint8_t* pair_with_next, uint32_t trim_at_coverage, uint32_t cutoff,
+                                          uint32_t diginorm_coverage, uint8_t* action_out, uint32_t* trim_pos_out, uint64_t* n_kmers_out)
+{
+    if (!h) return fail(KMGPU_EINVAL, "null handle");
+    if (n_kmers_out) *n_kmers_out = 0;
+    if (n_reads == 0) return KMGPU_OK;
+    if (!seqs || !offsets || !action_out || !trim_pos_out) return fail(KMGPU_EINVAL, "null argument");
+    const uint32_t Z = trim_at_coverage, C = cutoff, D = diginorm_coverage;
+    if (h->kind == BYTE && h->use_bigcount && (Z > 255 || C > 255 || D > 255))
+        return fail(KMGPU_EUNSUPPORTED, "trim_low_abund_pass1: coverages and cutoffs above 255 on a bigcount table are not supported");
+    for (uint64_t r = 0; r < n_reads; r++)
+        if (offsets[r + 1] - offsets[r] > chunk_bases() / 4)
+            return fail(KMGPU_EUNSUPPORTED, "read %llu is too long for a trimming window", (unsigned long long)r);
+    if (pair_with_next && pair_with_next[n_reads - 1]) return fail(KMGPU_EINVAL, "the last read cannot be paired with a next one");
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(set_device(h->device));
+    cudaStream_t st = h->stream;
+    const HashCfg H{h->hash, h->k};
+    const int N = h->nt;
+    const uint32_t cap_c = h->kind == BYTE ? 255u : h->kind == NIBBLE ? 15u : 1u;
+    // a bundle is consumed iff some read of it has median_at_least(min(Z, D)) false: normalization's keep rule.  The others are
+    // skipped (med >= D) or trimmed (Z <= med < D); with D <= Z all of them are skipped.  Their judgement compares counts with C
+    // (trim) and D (the skip test when Z < D): counts at or above R = the larger of the two need no refinement.
+    const uint32_t cut = D ? std::min(Z, D) : Z;
+    const bool judge = !(D && D <= Z);
+    const bool test_d = D && Z < D;
+    const uint32_t R = test_d ? std::max(C, D) : C;
+    const uint64_t W_fixed = env_u64("KMGPU_NORM_WINDOW", 0);
+    uint64_t W = W_fixed ? std::max<uint64_t>(2, W_fixed) : 32768;
+    uint64_t n_windows = 0, n_refined = 0;
+    NormClock clk;
+    const size_t fl = n_reads >= 100000 ? ((size_t)1 << 21) : 0;
+    uint64_t kmers_total = 0;
+    std::vector<uint8_t> keep, al;
+    std::vector<uint32_t> bstart;
+    for (uint64_t r0 = 0; r0 < n_reads;) {
+        ChunkPlan c;
+        ChunkDev cd;
+        uint64_t r1;
+        CKR(stage_window(h, seqs, offsets, n_reads, flags, pair_with_next, r0, W, c, cd, &r1));
+        const uint32_t nr = (uint32_t)(r1 - r0);
+        const uint8_t* pw = pair_with_next ? pair_with_next + r0 : nullptr;
+        uint8_t* act = action_out + r0;
+        uint32_t* tpos = trim_pos_out + r0;
+        n_windows++;
+        keep.assign(nr, 0);
+        bool too_large = false;
+        if (cd.n_pos) {
+            bool any_cand;
+            uint64_t n_unsure;
+            const int rc = norm_window_decide(h, c, cd, pw, cut, fl, clk, keep, &any_cand, &n_unsure, &too_large);
+            if (rc != KMGPU_OK && !too_large) return rc;
+            if (!too_large && any_cand && !W_fixed) {
+                if (n_unsure > 8192) W = std::max<uint64_t>(2048, W / 2);
+                else if (n_unsure < 2048) W = std::min<uint64_t>(1u << 17, W * 2);
+            }
+        }
+        // reads that were not consumed: their judgement.  Positions to refine: those of such reads whose window-start count is
+        // below R, when a consumed bundle may come before them.
+        uint64_t n_cons = 0, cap_up = 0;
+        bool any_judged = false;
+        bstart.assign(nr, ~0u);
+        for (uint32_t r = 0; r < nr && !too_large;) {
+            const uint32_t e = bundle_end(pw, nr, r);
+            for (uint32_t q = r; q < e; q++) {
+                const uint32_t len = c.offs[q + 1] - c.offs[q];
+                if (keep[q]) n_cons++;
+                else if (len >= (uint32_t)h->k) {
+                    bstart[q] = c.offs[r];
+                    cap_up += len - h->k + 1;
+                    any_judged = true;
+                }
+            }
+            r = e;
+        }
+        if (!too_large && judge && any_judged) {
+            if (n_cons && R) {
+                CKR(upload_read_bits(h, keep, nr));
+                CKR(h->d_upos.ensure(2 * cap_up));
+                CKR(h->d_nstate.ensure(4ull * nr));
+                uint32_t* d_bstart = reinterpret_cast<uint32_t*>(h->d_nstate.p);
+                CK(cudaMemcpyAsync(d_bstart, bstart.data(), 4ull * nr, cudaMemcpyHostToDevice, st));
+                CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
+                k_tla_refine_list<<<(nr + 7) / 8, 256, 0, st>>>(h->d_counts.p, cd.offs, nr, h->k, d_bstart, R, h->d_upos.p, h->d_upos.p + cap_up,
+                                                               &h->d_ctrl->n_events);
+                h->all_launches += 1;
+                CK(cudaGetLastError());
+                CKR(read_ctrl(h));
+                const uint64_t n_up = h->h_ctrl->n_events;
+                const uint64_t slots2 = pow2_at_least(2 * n_up * N);
+                if (slots2 > (1ull << 32)) too_large = true;
+                if (n_up && !too_large) {
+                    n_refined += n_up;
+                    CKR(h->d_nslot.ensure(n_up * N));
+                    CKR(h->d_uc0.ensure(n_up * N));
+                    CKR(h->d_evkeys.ensure(slots2));
+                    CKR(h->d_ncnt.ensure(slots2));
+                    CKR(h->d_nfill.ensure(slots2));
+                    CK(cudaMemsetAsync(h->d_evkeys.p, 0xFF, slots2 * 8, st));
+                    CK(cudaMemsetAsync(h->d_ncnt.p, 0, slots2 * 4, st));
+                    CK(cudaMemsetAsync(&h->d_ctrl->n_events, 0, sizeof(unsigned long long), st));
+                    uint64_t* keys2 = reinterpret_cast<uint64_t*>(h->d_evkeys.p);
+                    const Input in0 = make_input(cd);
+                    const uint32_t nu = (uint32_t)n_up;
+#define TLA_GATHER(KIND)                                                                                                                                    \
+    do {                                                                                                                                                    \
+        if (H.kind == TWOBIT) k_norm_gather<KIND, TWOBIT><<<(nu + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, nu, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1); \
+        else k_norm_gather<KIND, MURMUR><<<(nu + 255) / 256, 256, 0, st>>>(h->dev, H, in0, h->d_upos.p, nu, h->d_nslot.p, h->d_uc0.p, keys2, slots2 - 1);               \
+    } while (0)
+                    if (h->kind == BYTE) TLA_GATHER(BYTE);
+                    else if (h->kind == NIBBLE) TLA_GATHER(NIBBLE);
+                    else TLA_GATHER(BIT);
+#undef TLA_GATHER
+                    Input inc = make_input(cd);
+                    inc.read_keep = h->d_readbits.p;   // the consumed reads
+                    const unsigned gt = n_tiles(cd.n_pos);
+                    if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
+                    else k_norm_hits<MURMUR, 0, 0><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_ncnt.p, nullptr);
+                    k_norm_hit_offsets<<<148 * 8, 256, 0, st>>>(h->d_ncnt.p, h->d_nfill.p, slots2, &h->d_ctrl->n_events);
+                    h->all_launches += 3;
+                    CK(cudaGetLastError());
+                    CKR(read_ctrl(h));
+                    const uint64_t n_hits = h->h_ctrl->n_events;
+                    if (n_hits >= (1ull << 32)) too_large = true;
+                    if (!too_large) {
+                        CKR(h->d_nhits.ensure(std::max<uint64_t>(n_hits, 1)));
+                        if (H.kind == TWOBIT) k_norm_hits<TWOBIT, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
+                        else k_norm_hits<MURMUR, 0, 1><<<gt, THREADS, 0, st>>>(h->dev, H, inc, keys2, slots2 - 1, h->d_nfill.p, h->d_nhits.p);
+                        k_tla_refine<<<(nu + 255) / 256, 256, 0, st>>>(h->d_upos.p, h->d_upos.p + cap_up, nu, h->d_nslot.p, h->d_uc0.p, h->d_ncnt.p,
+                                                                      h->d_nfill.p, h->d_nhits.p, N, R, cap_c, h->d_counts.p);
+                        h->all_launches += 2;
+                        CK(cudaGetLastError());
+                    }
+                }
+            }
+            if (!too_large) {
+                // d_counts: every judged read's counts as its bundle meets the table (exact below R)
+                if (test_d) {
+                    al.resize(nr);
+                    CKR(read_stats_counts(h, h->d_counts.p, cd, 0, nullptr, nullptr, nullptr, nullptr, true, D, al.data()));
+                }
+                CKR(trim_counts(h, h->d_counts.p, cd, 0, C, 0, tpos));
+                clk.lap(9);
+            }
+        }
+        if (too_large) {
+            // the refinement's lists would pass 32 bits: the same reads in smaller windows (the table has not changed)
+            if (nr < 2) return fail(KMGPU_EUNSUPPORTED, "trim_low_abund_pass1: a window of one bundle is too large");
+            W = std::max<uint64_t>(1, nr / 2);
+            continue;
+        }
+        for (uint32_t r = 0; r < nr;) {
+            const uint32_t e = bundle_end(pw, nr, r);
+            bool skip = !judge;
+            if (test_d) {
+                skip = true;
+                for (uint32_t q = r; q < e; q++)
+                    if (!keep[q] && bstart[q] != ~0u && al[q] == 0) skip = false;
+            }
+            for (uint32_t q = r; q < e; q++) {
+                const bool kmers = c.offs[q + 1] - c.offs[q] >= (uint32_t)h->k;
+                act[q] = !kmers ? KMGPU_TLA_DROP : keep[q] ? KMGPU_TLA_SAVE : skip ? KMGPU_TLA_SKIP : KMGPU_TLA_TRIM;
+                if (act[q] != KMGPU_TLA_TRIM) tpos[q] = 0;
+            }
+            r = e;
+        }
+        CKR(norm_window_ingest(h, cd, keep, &kmers_total));
+        clk.lap(3);
+        r0 = r1;
+    }
+    if (n_kmers_out) *n_kmers_out = kmers_total;
+    if (clk.dbg)
+        fprintf(stderr, "[kmgpu] trim_low_abund_pass1: %llu reads in %llu windows (last %llu reads), %llu refined positions; "
+                        "seconds: first test %.3f, overlay test %.3f, in-between %.3f, refinement + judgement %.3f, ingest %.3f, other %.3f\n",
+                (unsigned long long)n_reads, (unsigned long long)n_windows, (unsigned long long)W, (unsigned long long)n_refined,
+                clk.t[0], clk.t[1], clk.t[2], clk.t[9], clk.t[3], clk.t[4]);
+    return KMGPU_OK;
+}
+
+extern "C" int kmgpu_trim_low_abund_pass2(kmgpu_t* h, const char* seqs, const uint64_t* offsets, uint64_t n_reads, uint32_t flags,
+                                          const uint8_t* pair_with_next, uint32_t trim_at_coverage, uint32_t cutoff, int variable_coverage,
+                                          uint8_t* action_out, uint32_t* trim_pos_out)
+{
+    if (!h) return fail(KMGPU_EINVAL, "null handle");
+    if (n_reads == 0) return KMGPU_OK;
+    if (!seqs || !offsets || !action_out || !trim_pos_out) return fail(KMGPU_EINVAL, "null argument");
+    for (uint64_t r = 0; r < n_reads; r++)
+        if (offsets[r + 1] - offsets[r] > chunk_bases())
+            return fail(KMGPU_EUNSUPPORTED, "read %llu is longer than a device chunk", (unsigned long long)r);
+    if (pair_with_next && pair_with_next[n_reads - 1]) return fail(KMGPU_EINVAL, "the last read cannot be paired with a next one");
+    std::lock_guard<std::mutex> g(h->mu);
+    CKR(set_device(h->device));
+    if (h->kind == BYTE && h->use_bigcount) CKR(sync_big_to_device(h));
+    const uint32_t nb = (h->kind == BYTE && h->use_bigcount) ? h->n_big_dev : 0;
+    const HashCfg H{h->hash, h->k};
+    // one count per k-mer: median_at_least (variable coverage) and the trim scan read the same counts
+    std::vector<uint8_t> al(variable_coverage ? n_reads : 0);
+    std::vector<ChunkPlan> plan;
+    plan_chunks(offsets, n_reads, h->k, chunk_bases(), plan);
+    uint64_t r0 = 0;
+    for (const ChunkPlan& c : plan) {
+        ChunkDev cd;
+        CKR(stage_chunk(h, seqs, c, flags, &cd, needs_acgt_check(h, flags)));
+        if (variable_coverage) {
+            CKR(read_stats_chunk(h, cd, r0, nb, nullptr, nullptr, nullptr, nullptr, true, trim_at_coverage, al.data()));
+        } else {
+            CKR(h->d_counts.ensure(std::max<uint32_t>(cd.n_pos, 1)));
+            if (cd.n_pos) launch_counts(0, h->dev, H, make_input(cd), h->big_keys.p, h->big_vals.p, nb, h->d_counts.p, nullptr, nullptr, h->stream);
+            h->all_launches += 1;
+        }
+        CKR(trim_counts(h, h->d_counts.p, cd, r0, cutoff, 0, trim_pos_out));
+        r0 += cd.n_reads;
+    }
+    // bundles: ReadBundle.coverages_at_least (khmer/utils.py:178-180) over the reads with k-mers
+    for (uint64_t r = 0; r < n_reads;) {
+        uint64_t e = r + 1;
+        while (e < n_reads && pair_with_next && pair_with_next[e - 1]) e++;
+        bool trim = true;
+        if (variable_coverage)
+            for (uint64_t q = r; q < e; q++) trim &= al[q] != 0;
+        for (uint64_t q = r; q < e; q++) {
+            const bool kmers = offsets[q + 1] - offsets[q] >= (uint64_t)h->k;
+            action_out[q] = !kmers ? KMGPU_TLA_DROP : trim ? KMGPU_TLA_TRIM : KMGPU_TLA_KEEP;
+            if (action_out[q] != KMGPU_TLA_TRIM) trim_pos_out[q] = 0;
+        }
+        r = e;
+    }
     return KMGPU_OK;
 }
 

@@ -1092,6 +1092,63 @@ __global__ void k_norm_keep_bits(const uint8_t* __restrict__ state, uint32_t n_r
     bits[w] = m;
 }
 
+// =====================================================================================================================
+// 6. Trim-low-abund, pass 1 (scripts/trim-low-abund.py:196-238).  The consumed bundles of a window are normalization's kept
+//    ones (cutoff min(Z, D)); every other bundle is judged against the table as it arrives, whose count for a k-mer at chunk
+//    position p of a bundle starting at s is min over tables of min(cap, c0 + touches of its bin by consumed reads before s).
+//    Only k-mers whose window-start count is below R (the largest threshold a judgement compares with) can differ in outcome.
+// =====================================================================================================================
+
+// one warp per read: the positions of read r's k-mers whose count is below R, with the start of r's bundle (bstart[r] = ~0u:
+// nothing to refine in that read)
+__global__ void __launch_bounds__(256)
+k_tla_refine_list(const uint16_t* __restrict__ counts, const uint32_t* __restrict__ offs, uint32_t n_reads, int k,
+                  const uint32_t* __restrict__ bstart, uint32_t R, uint32_t* __restrict__ out_pos, uint32_t* __restrict__ out_start,
+                  unsigned long long* n_out)
+{
+    const int lane = threadIdx.x & 31;
+    const uint32_t r = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (r >= n_reads || bstart[r] == ~0u) return;
+    const uint32_t s = offs[r], e = offs[r + 1];
+    const uint32_t n = e - s >= (uint32_t)k ? e - s - k + 1 : 0;
+    for (uint32_t i0 = 0; i0 < n; i0 += 32) {
+        const uint32_t i = i0 + lane;
+        const bool low = i < n && counts[s + i] < R;
+        const unsigned m = __ballot_sync(0xffffffffu, low);
+        if (!m) continue;
+        uint32_t base = 0;
+        if (lane == 0) base = (uint32_t)atomicAdd(n_out, (unsigned long long)__popc(m));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (low) {
+            const uint32_t at = base + __popc(m & ((1u << lane) - 1u));
+            out_pos[at] = s + i;
+            out_start[at] = bstart[r];
+        }
+    }
+}
+
+// per listed position: its count as the bundle meets it (hits before the bundle's start; a table stops counting at R), written
+// over the window-start count
+__global__ void __launch_bounds__(256)
+k_tla_refine(const uint32_t* __restrict__ upos, const uint32_t* __restrict__ ustart, uint32_t n_up, const uint32_t* __restrict__ slot,
+             const uint16_t* __restrict__ c0, const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ fill,
+             const uint2* __restrict__ hits, int n_tables, uint32_t R, uint32_t cap, uint16_t* __restrict__ counts)
+{
+    const uint32_t j = blockIdx.x * 256u + threadIdx.x;
+    if (j >= n_up) return;
+    const uint32_t bstart = ustart[j];
+    uint32_t mn = cap;
+    for (int t = 0; t < n_tables; t++) {
+        const size_t at = (size_t)j * n_tables + t;
+        const uint32_t sl = slot[at];
+        uint32_t v = c0[at];
+        const uint32_t end = fill[sl];
+        for (uint32_t x = end - cnt[sl]; x < end && v < R; x++) v += hits[x].x < bstart;
+        mn = v < mn ? v : mn;
+    }
+    counts[upos[j]] = (uint16_t)mn;
+}
+
 }  // namespace kmgpu
 
 namespace kmgpu {

@@ -740,6 +740,40 @@ unsigned long long Hashtable::normalize_batch(const std::vector<std::string>& se
     return kmers;
 }
 
+unsigned long long Hashtable::trim_low_abund_pass1(const std::vector<std::string>& seqs, unsigned int trim_at_coverage, unsigned int cutoff,
+                                                   unsigned int diginorm_coverage, const std::vector<uint8_t>& pair_with_next, bool clean,
+                                                   std::vector<uint8_t>& action, std::vector<uint32_t>& trim_pos)
+{
+    std::string buf;
+    std::vector<uint64_t> offs;
+    pack_strings(seqs, buf, offs);
+    action.assign(seqs.size(), 0);
+    trim_pos.assign(seqs.size(), 0);
+    if (seqs.empty()) return 0;
+    if (!pair_with_next.empty() && pair_with_next.size() != seqs.size()) throw oxli_value_exception("pair flags: one per read");
+    uint64_t kmers = 0;
+    check(kmgpu_trim_low_abund_pass1(store->handle(), buf.data(), offs.data(), seqs.size(), clean ? KMGPU_CLEAN : 0,
+                                     pair_with_next.empty() ? nullptr : pair_with_next.data(), trim_at_coverage, cutoff, diginorm_coverage,
+                                     action.data(), trim_pos.data(), &kmers));
+    return kmers;
+}
+
+void Hashtable::trim_low_abund_pass2(const std::vector<std::string>& seqs, unsigned int trim_at_coverage, unsigned int cutoff, bool variable_coverage,
+                                     const std::vector<uint8_t>& pair_with_next, bool clean, std::vector<uint8_t>& action,
+                                     std::vector<uint32_t>& trim_pos)
+{
+    std::string buf;
+    std::vector<uint64_t> offs;
+    pack_strings(seqs, buf, offs);
+    action.assign(seqs.size(), 0);
+    trim_pos.assign(seqs.size(), 0);
+    if (seqs.empty()) return;
+    if (!pair_with_next.empty() && pair_with_next.size() != seqs.size()) throw oxli_value_exception("pair flags: one per read");
+    check(kmgpu_trim_low_abund_pass2(store->handle(), buf.data(), offs.data(), seqs.size(), clean ? KMGPU_CLEAN : 0,
+                                     pair_with_next.empty() ? nullptr : pair_with_next.data(), trim_at_coverage, cutoff, variable_coverage ? 1 : 0,
+                                     action.data(), trim_pos.data()));
+}
+
 BoundedCounterType Hashtable::get_min_count(const std::string& s)
 {
     std::vector<BoundedCounterType> counts;

@@ -342,6 +342,14 @@ public:
     // digital normalization of a batch in stream order (scripts/normalize-by-median.py:155-179); returns the k-mers consumed
     unsigned long long normalize_batch(const std::vector<std::string>& seqs, unsigned int cutoff, const std::vector<uint8_t>& pair_with_next,
                                        std::vector<uint8_t>& keep);
+    // trim-low-abund's two passes for a batch in stream order (scripts/trim-low-abund.py:196-271): per-read actions (KMGPU_TLA_*) and
+    // trim lengths; pass 1 returns the k-mers consumed.  clean: Read::set_clean_seq on the device.
+    unsigned long long trim_low_abund_pass1(const std::vector<std::string>& seqs, unsigned int trim_at_coverage, unsigned int cutoff,
+                                            unsigned int diginorm_coverage, const std::vector<uint8_t>& pair_with_next, bool clean,
+                                            std::vector<uint8_t>& action, std::vector<uint32_t>& trim_pos);
+    void trim_low_abund_pass2(const std::vector<std::string>& seqs, unsigned int trim_at_coverage, unsigned int cutoff, bool variable_coverage,
+                              const std::vector<uint8_t>& pair_with_next, bool clean, std::vector<uint8_t>& action,
+                              std::vector<uint32_t>& trim_pos);
     unsigned long trim_on_abundance(std::string seq, BoundedCounterType min_abund) const;
     unsigned long trim_below_abundance(std::string seq, BoundedCounterType max_abund) const;
     std::vector<unsigned int> find_spectral_error_positions(std::string seq, BoundedCounterType min_abund) const;

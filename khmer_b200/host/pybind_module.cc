@@ -294,6 +294,29 @@ PYBIND11_MODULE(_oxli, m)
             }
             return py::make_tuple(keep, kmers);
         }, py::arg("seqs"), py::arg("cutoff"), py::arg("paired") = std::vector<uint8_t>())
+        .def("trim_low_abund_pass1", [](Hashtable& h, const std::vector<std::string>& seqs, unsigned trim_at_coverage, unsigned cutoff,
+                                        unsigned diginorm_coverage, const std::vector<uint8_t>& paired, bool clean) {
+            std::vector<uint8_t> action;
+            std::vector<uint32_t> trim_pos;
+            unsigned long long kmers;
+            {
+                py::gil_scoped_release nogil;
+                kmers = h.trim_low_abund_pass1(seqs, trim_at_coverage, cutoff, diginorm_coverage, paired, clean, action, trim_pos);
+            }
+            return py::make_tuple(py::bytes(reinterpret_cast<const char*>(action.data()), action.size()), trim_pos, kmers);
+        }, py::arg("seqs"), py::arg("trim_at_coverage"), py::arg("cutoff"), py::arg("diginorm_coverage") = 0,
+           py::arg("paired") = std::vector<uint8_t>(), py::arg("clean") = false)
+        .def("trim_low_abund_pass2", [](Hashtable& h, const std::vector<std::string>& seqs, unsigned trim_at_coverage, unsigned cutoff,
+                                        bool variable_coverage, const std::vector<uint8_t>& paired, bool clean) {
+            std::vector<uint8_t> action;
+            std::vector<uint32_t> trim_pos;
+            {
+                py::gil_scoped_release nogil;
+                h.trim_low_abund_pass2(seqs, trim_at_coverage, cutoff, variable_coverage, paired, clean, action, trim_pos);
+            }
+            return py::make_tuple(py::bytes(reinterpret_cast<const char*>(action.data()), action.size()), trim_pos);
+        }, py::arg("seqs"), py::arg("trim_at_coverage"), py::arg("cutoff"), py::arg("variable_coverage") = false,
+           py::arg("paired") = std::vector<uint8_t>(), py::arg("clean") = false)
         .def("n_unique_kmers", &Hashtable::n_unique_kmers)
         .def("n_occupied", &Hashtable::n_occupied)
         .def("n_tables", &Hashtable::n_tables)
