@@ -287,10 +287,21 @@ int kmgpu_first_touch_resolve(kmgpu_t* h, uint64_t* n_new_out, uint64_t* n_local
  * exact); a round is refused (KMGPU_ENOMEM from kmgpu_shard_apply on that rank, nothing applied there) only if one owner is sent
  * more than 1.5 x what its share of the bins receives on average in a full round.
  * Table bytes and n_occupied are exact (concatenated slices / summed counters equal the single sketch); n_unique_kmers is the
- * sum of the ranks' shares (kmgpu_shard_stats); bigcount is not maintained in this mode.  The saved table is the
- * concatenation of the ranks' slices in rank order (kmgpu_shard_slice + the local sketch's kmgpu_download_table). */
+ * sum of the ranks' shares (kmgpu_shard_stats).  The saved table is the concatenation of the ranks' slices in rank order
+ * (kmgpu_shard_slice + the local sketch's kmgpu_download_table).
+ * Bigcount (ByteStorage, at most 30 tables): kmgpu_set_use_bigcount on every rank's kmgpu_shard_local, the same value on all ranks
+ * (it may change between rounds).  Then kmgpu_shard_apply also marks, in its arena, which touches found their byte at 255 (bit 1
+ * of its refusal word tells the senders), and each round gains two steps after kmgpu_shard_count_new:
+ *     kmgpu_shard_bigcount_events  every sender reads the marks of its records back and lists its k-mers whose N bytes were all 255
+ *                                  before they arrived (ByteStorage::add, storage.hh:606-617): one entry per distinct hash with
+ *                                  its number of events, in the order of its first event.  KMGPU_ENOMEM if an owner it sent
+ *                                  records to refused the round.  hashes == NULL asks for the number only; the list stays
+ *                                  until the next route.  Call it before the barrier that ends the round.
+ *     kmgpu_shard_bigcount_apply   every rank applies ALL ranks' lists, concatenated in rank order, to its local sketch's map
+ * so that every rank holds the map of one sketch fed the rounds in stream order — same entries, same iteration order
+ * (kmgpu_bigcount_export on kmgpu_shard_local).  Query rounds then give counts above 255 from that map. */
 typedef struct kmgpu_shard kmgpu_shard_t;
-#define KMGPU_SHARD_IPC_HANDLES 5 /* receive arena, demand table, receive offsets, refusal word, new-position bitmap */
+#define KMGPU_SHARD_IPC_HANDLES 5 /* receive arena, demand table, receive offsets, refusal / bigcount word, new-position bitmap */
 #define KMGPU_MAX_WORLD 16
 int kmgpu_shard_create(int storage, int hash, int ksize, int n_tables, const uint64_t* full_sizes, int device,
                        int rank, int world, uint64_t max_positions_per_route, kmgpu_shard_t** out);
@@ -311,6 +322,8 @@ int kmgpu_shard_offsets(kmgpu_shard_t* s);
 int kmgpu_shard_push(kmgpu_shard_t* s);
 int kmgpu_shard_apply(kmgpu_shard_t* s);
 int kmgpu_shard_count_new(kmgpu_shard_t* s, uint64_t* n_new_out);
+int kmgpu_shard_bigcount_events(kmgpu_shard_t* s, uint64_t* hashes, uint32_t* counts, uint64_t cap, uint64_t* n_out);
+int kmgpu_shard_bigcount_apply(kmgpu_shard_t* s, const uint64_t* hashes, const uint32_t* counts, uint64_t n);
 
 /* Query rounds: the counts a single sketch would give the k-mers of every rank's reads (get_count, storage.hh:627-649 / :362-379 /
  * :207-219: the minimum over the N tables, whose bins live on different ranks).  The first three steps are those of an ingest round:
@@ -322,7 +335,8 @@ int kmgpu_shard_count_new(kmgpu_shard_t* s, uint64_t* n_new_out);
  *                          reads, the minimum over the tables.  KMGPU_ENOMEM (and no counts) if an owner it sent records to refused.
  * again with a barrier (provided by the caller) after each step.  The getters below then work on this rank's reads of the round,
  * as last passed to kmgpu_shard_route (nothing restages the local sketch between the route and them); their layouts and values
- * equal the single-sketch calls named beside them, without bigcount.  Before a pull they fail with KMGPU_EINVAL. */
+ * equal the single-sketch calls named beside them (with bigcount on, a count of 255 is the map's value where the map holds the
+ * k-mer).  Before a pull they fail with KMGPU_EINVAL. */
 int kmgpu_shard_lookup(kmgpu_shard_t* s);
 int kmgpu_shard_pull(kmgpu_shard_t* s);
 /* kmgpu_kmer_counts: counts_out holds sum(max(0, len_r - k + 1)) entries */

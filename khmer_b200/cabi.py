@@ -38,7 +38,8 @@ SYMBOLS = [
     "kmgpu_shard_create", "kmgpu_shard_destroy", "kmgpu_shard_local", "kmgpu_shard_slice", "kmgpu_shard_ipc_export",
     "kmgpu_shard_ipc_attach", "kmgpu_shard_attach_local", "kmgpu_shard_route", "kmgpu_shard_offsets", "kmgpu_shard_push", "kmgpu_shard_apply",
     "kmgpu_shard_count_new", "kmgpu_shard_stats", "kmgpu_shard_lookup", "kmgpu_shard_pull", "kmgpu_shard_kmer_counts",
-    "kmgpu_shard_read_medians", "kmgpu_shard_median_at_least", "kmgpu_shard_trim", "kmgpu_shard_abundance_hist", "kmgpu_hll_create", "kmgpu_hll_destroy", "kmgpu_hll_consume",
+    "kmgpu_shard_read_medians", "kmgpu_shard_median_at_least", "kmgpu_shard_trim", "kmgpu_shard_abundance_hist",
+    "kmgpu_shard_bigcount_events", "kmgpu_shard_bigcount_apply", "kmgpu_hll_create", "kmgpu_hll_destroy", "kmgpu_hll_consume",
     "kmgpu_hll_get_registers", "kmgpu_hll_merge_registers", "kmgpu_trim_low_abund_pass1", "kmgpu_trim_low_abund_pass2",
 ]
 
@@ -161,6 +162,8 @@ def lib():
         L.kmgpu_shard_median_at_least.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
         L.kmgpu_shard_trim.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p]
         L.kmgpu_shard_abundance_hist.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kmgpu_shard_bigcount_events.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, u64p]
+        L.kmgpu_shard_bigcount_apply.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
         _lib = L
     return _lib
 
@@ -629,6 +632,33 @@ class Shard:
         n = C.c_uint64()
         check(lib().kmgpu_shard_count_new(self.h, C.byref(n)))
         return n.value
+
+    # -- bigcount (ByteStorage): the switch and the map are the local sketch's; every rank must use the same setting
+    def set_use_bigcount(self, on):
+        self.local.set_use_bigcount(on)
+
+    def get_use_bigcount(self):
+        return self.local.get_use_bigcount()
+
+    def bigcount_events(self):
+        """after every rank has applied the round (and before the next route): this rank's k-mers whose N bytes were all 255
+        before they arrived, one per distinct hash in the order of its first event -> (hashes uint64, event counts uint32)"""
+        n = C.c_uint64()
+        check(lib().kmgpu_shard_bigcount_events(self.h, None, None, 0, C.byref(n)))
+        keys = np.zeros(max(n.value, 1), dtype=np.uint64)
+        counts = np.zeros(max(n.value, 1), dtype=np.uint32)
+        check(lib().kmgpu_shard_bigcount_events(self.h, _ptr(keys), _ptr(counts), n.value, C.byref(n)))
+        return keys[:n.value], counts[:n.value]
+
+    def bigcount_apply(self, hashes, counts):
+        """apply every rank's events of the round, concatenated in rank order, to this rank's bigcount map"""
+        hashes = np.ascontiguousarray(hashes, dtype=np.uint64)
+        counts = np.ascontiguousarray(counts, dtype=np.uint32)
+        check(lib().kmgpu_shard_bigcount_apply(self.h, _ptr(hashes), _ptr(counts), len(hashes)))
+
+    def bigcounts(self):
+        """the bigcount map (the same on every rank), in its iteration order: (hashes uint64, counts uint16)"""
+        return self.local.bigcounts()
 
     # -- query rounds: route, offsets, push, then lookup and pull; the getters answer for this rank's reads of the last route
     def lookup(self):

@@ -3139,7 +3139,7 @@ struct kmgpu_shard {
     unsigned long long* rec1 = nullptr;    // arena
     uint32_t* demand = nullptr;            // [local super-bucket * world + sender]
     unsigned long long* recv_off = nullptr;
-    unsigned long long* flags = nullptr;   // bit 0: this round does not fit the arena
+    unsigned long long* flags = nullptr;   // bit 0: this round does not fit the arena; bit 1: the arena holds bigcount answers
     uint32_t* newbits = nullptr;           // one bit per global position of a round: marked new by this owner
     struct PeerQ {
         unsigned long long* rec1;
@@ -3167,6 +3167,10 @@ struct kmgpu_shard {
     DevBuf<uint8_t> planes;    // pull: the answers, one byte per (table, position), planes of max_positions bytes
     bool pulled = false;       // the last route was answered (kmgpu_shard_pull): the local sketch's d_counts hold its counts
     bool counted = false;      // the last route was ingested up to kmgpu_shard_count_new: its d_newbits hold the new positions
+    // bigcount (ingest rounds): the owner's (position, crossing-bin slot) pairs, and this rank's events of the last round
+    DevBuf<uint2> sel_pairs;
+    std::vector<EvOut> big_ev;
+    bool big_ev_ready = false;
 };
 
 extern "C" int kmgpu_shard_destroy(kmgpu_shard_t* s);
@@ -3298,6 +3302,7 @@ extern "C" int kmgpu_shard_destroy(kmgpu_shard_t* s)
     s->planes.release();
     s->sb_off.release();
     s->sb_cnt.release();
+    s->sel_pairs.release();
     s->rec_s.release();
     s->off_s.release();
     s->cur_s.release();
@@ -3425,7 +3430,7 @@ extern "C" int kmgpu_shard_route(kmgpu_shard_t* s, const char* seqs, const uint6
     CK(cudaMemsetAsync(h->d_ctrl, 0, sizeof(Ctrl), st));
     s->exact_s = false;
     s->q = ChunkDev{};
-    s->pulled = s->counted = false;
+    s->pulled = s->counted = s->big_ev_ready = false;
     uint64_t n_kmers = 0;
     if (last > first) {
         ChunkDev cd;
@@ -3569,18 +3574,78 @@ extern "C" int kmgpu_shard_push(kmgpu_shard_t* s)
     return KMGPU_OK;
 }
 
+// bigcount (owner, after the apply): every record of my arena is answered with "its byte was 255 before it arrived" (k_shard_satmark),
+// and bit 1 of my flags tells the senders to read the answers.  A bin that crossed 255 in this round was saturated for the touches
+// after its (255 - before)-th in global position order: that touch's position T is found by a radix select over the records of
+// the crossing bins.
+static int shard_satmark(kmgpu_shard* s, uint64_t n_list, uint64_t n_cross, uint32_t n_pos_all)
+{
+    kmgpu_sketch* h = s->local;
+    cudaStream_t st = h->stream;
+    constexpr uint64_t WS_MIN = 1ull << 20;
+    const int sbb = BKT_SHIFT + s->GF.L.sb_shift;
+    const dim3 grid(s->n_sb_local, 8);
+    uint64_t slots = 1024;
+    const uint32_t* T = nullptr;
+    if (n_cross) {
+        slots = pow2_at_least(2 * n_cross);
+        CKR(h->d_htkeys.ensure(std::max<uint64_t>(slots, WS_MIN)));
+        CKR(h->d_htvals.ensure(std::max<uint64_t>(slots, WS_MIN)));
+        CK(cudaMemsetAsync(h->d_htkeys.p, 0xFF, slots * 8, st));
+        k_list_register<<<(unsigned)std::min<uint64_t>((n_list + 255) / 256, 148 * 8), 256, 0, st>>>(h->d_binlist.p, n_list, BL_CROSS, h->d_htkeys.p,
+                                                                                                  h->d_htvals.p, slots - 1, nullptr, 1);
+        h->all_launches += 1;
+        // the touches of the crossing bins; the buffer grows (and the pass runs again) when they do not fit
+        unsigned long long* n_pairs = &h->d_ctrl->n_events;
+        uint64_t n = 0;
+        for (int pass = 0; pass < 2; pass++) {
+            CKR(s->sel_pairs.ensure(std::max<uint64_t>(n, WS_MIN)));
+            CK(cudaMemsetAsync(n_pairs, 0, sizeof(unsigned long long), st));
+            k_shard_sel_pairs<<<grid, 256, 0, st>>>(s->geom, s->rec1, s->sb_off.p, s->sb_cnt.p, sbb, h->d_htkeys.p, slots - 1, s->sel_pairs.p,
+                                                    (unsigned long long)s->sel_pairs.cap, n_pairs);
+            h->all_launches += 1;
+            CK(cudaGetLastError());
+            CKR(read_ctrl(h));
+            n = h->h_ctrl->n_events;
+            if (n <= s->sel_pairs.cap) break;
+        }
+        if (n > s->sel_pairs.cap) return fail(KMGPU_ECUDA, "internal: crossing-bin touches overflowed");
+        CKR(h->d_sel.ensure(std::max<uint64_t>(3 * slots, WS_MIN)));
+        SelState ss{h->d_sel.p, h->d_sel.p + slots, h->d_sel.p + 2 * slots};
+        const unsigned gsl = (unsigned)((slots + 255) / 256), gp = (unsigned)std::max<uint64_t>((n + 255) / 256, 1);
+        k_sel_init<<<gsl, 256, 0, st>>>(h->d_htkeys.p, h->d_htvals.p, slots, ss);
+        int top = 0;
+        while (top < 31 && (1ull << (top + 1)) <= (uint64_t)n_pos_all) top++;
+        for (int bit = top; bit >= 0; bit--) {
+            k_sel_count_pairs<<<gp, 256, 0, st>>>(s->sel_pairs.p, n, bit, ss);
+            k_sel_update<<<gsl, 256, 0, st>>>(slots, bit, ss);
+        }
+        h->all_launches += 1 + 2 * (top + 1);
+        T = ss.prefix;
+    }
+    k_shard_satmark<<<grid, 256, 0, st>>>(s->geom, h->dev, s->rec1, s->sb_off.p, s->sb_cnt.p, sbb, h->d_htkeys.p, slots - 1, T, n_cross ? 1 : 0);
+    h->all_launches += 1;
+    CK(cudaGetLastError());
+    const unsigned long long fl = 2ull;
+    CK(cudaMemcpyAsync(s->flags, &fl, 8, cudaMemcpyHostToDevice, st));
+    CK(cudaStreamSynchronize(st));
+    return KMGPU_OK;
+}
+
 extern "C" int kmgpu_shard_apply(kmgpu_shard_t* s)
 {
     if (!s) return fail(KMGPU_EINVAL, "null shard");
     kmgpu_sketch* h = s->local;
     std::lock_guard<std::mutex> g(h->mu);
     CKR(set_device(h->device));
-    if (h->kind == BYTE && h->use_bigcount) return fail(KMGPU_EUNSUPPORTED, "bigcount is not maintained by sharded sketches");
+    const int want_cross = h->kind == BYTE && h->use_bigcount;
+    if (want_cross && h->nt > 30) return fail(KMGPU_EUNSUPPORTED, "bigcount is supported for up to 30 tables");
     cudaStream_t st = h->stream;
     const size_t n_dem = (size_t)s->n_sb_local * s->world;
     if (s->refused) {
+        // the refusal flag stays up: with bigcount on, the senders read it in kmgpu_shard_bigcount_events (kmgpu_shard_offsets
+        // writes it anew every round)
         s->refused = false;
-        CK(cudaMemsetAsync(s->flags, 0, 8, st));
         CK(cudaMemsetAsync(s->demand, 0, n_dem * 4, st));
         CK(cudaStreamSynchronize(st));
         return fail(KMGPU_ENOMEM, "rank %d was sent %llu records in one round, its arena holds %llu (this rank owns far more than its share of the "
@@ -3593,7 +3658,14 @@ extern "C" int kmgpu_shard_apply(kmgpu_shard_t* s)
     CKR(h->d_cursors.ensure(G.n_buckets));
     if (!try_ensure(h->d_records, std::max<uint64_t>((uint64_t)G.n_buckets * G.L.cap, 2)))
         return fail(KMGPU_ENOMEM, "no room for the bucket store of a sharded round");
-    CKR(h->d_binlist.ensure(1));
+    // bigcount: one crossing-list entry per bin that reaches 255 in this round, at most one per record received
+    uint64_t list_cap = 1;
+    if (want_cross) {
+        uint64_t bins = 0;
+        for (int i = 0; i < h->nt; i++) bins += h->sizes[i];
+        list_cap = std::max<uint64_t>(1, std::min<uint64_t>(s->received, bins));
+    }
+    CKR(h->d_binlist.ensure(list_cap));
     CK(cudaMemsetAsync(s->newbits, 0, (size_t)n_pos_all / 8, st));
     CK(cudaMemsetAsync(h->d_ctrl, 0, sizeof(Ctrl), st));
     CK(cudaEventRecord(h->ev0, st));
@@ -3605,7 +3677,7 @@ extern "C" int kmgpu_shard_apply(kmgpu_shard_t* s)
     memset(&P0, 0, sizeof P0);
     const HashCfg H{h->hash, h->k};
     const std::vector<Part> none;
-    if (s->received) CKR(group_turn(h, G, tn, 0, 0, H, none, P0, false, h->dev, false, 0u, n_pos_all, 1, 0, sb, &s1, s->newbits));
+    if (s->received) CKR(group_turn(h, G, tn, 0, 0, H, none, P0, false, h->dev, false, 0u, n_pos_all, list_cap, want_cross, sb, &s1, s->newbits));
     CK(cudaEventRecord(h->ev1, st));
     CKR(read_ctrl(h));
     float ms = 0;
@@ -3615,7 +3687,7 @@ extern "C" int kmgpu_shard_apply(kmgpu_shard_t* s)
         const unsigned bits = (unsigned)(h->h_ctrl->overflow & 3ull);
         CK(cudaMemsetAsync(&h->d_ctrl->overflow, 0, sizeof(unsigned long long), st));
         h->n_regroups++;
-        CKR(group_turn(h, G, tn, 0, 0, H, none, P0, false, h->dev, false, bits, n_pos_all, 1, 0, sb, &s1, s->newbits));
+        CKR(group_turn(h, G, tn, 0, 0, H, none, P0, false, h->dev, false, bits, n_pos_all, list_cap, want_cross, sb, &s1, s->newbits));
         CKR(read_ctrl(h));
         if (h->h_ctrl->overflow) return fail(KMGPU_ECUDA, "internal: regrouping run overflowed");
         // bucket regions get more slack from the next round on
@@ -3625,6 +3697,12 @@ extern "C" int kmgpu_shard_apply(kmgpu_shard_t* s)
         s->G.sparse = s->G.sparse && s->G.L.cap <= SPARSE_MAX_RECORDS;
     }
     h->n_occupied += h->h_ctrl->n_new_t[0];   // the apply kernels of the grouped path count newly occupied bins per table
+    if (want_cross) {
+        // after any regrouping run (it reads the arena's records as they were pushed); no touch found a saturated byte: nothing to mark
+        const Ctrl c = *h->h_ctrl;
+        if (c.n_events > list_cap) return fail(KMGPU_ECUDA, "internal: crossing list overflow");
+        if (c.n_sat) CKR(shard_satmark(s, c.n_events, c.n_cross, n_pos_all));
+    }
     CK(cudaMemsetAsync(s->demand, 0, n_dem * 4, st));   // ranks without reads in a later round post nothing for tables they do not reach
     CK(cudaStreamSynchronize(st));
     h->satbits_valid = false;
@@ -3673,7 +3751,6 @@ extern "C" int kmgpu_shard_lookup(kmgpu_shard_t* s)
     kmgpu_sketch* h = s->local;
     std::lock_guard<std::mutex> g(h->mu);
     CKR(set_device(h->device));
-    if (h->kind == BYTE && h->use_bigcount) return fail(KMGPU_EUNSUPPORTED, "bigcount is not maintained by sharded sketches");
     cudaStream_t st = h->stream;
     const size_t n_dem = (size_t)s->n_sb_local * s->world;
     if (s->refused) {
@@ -3719,7 +3796,7 @@ extern "C" int kmgpu_shard_pull(kmgpu_shard_t* s)
         CK(cudaMemsetAsync(&h->d_ctrl->overflow, 0, sizeof(unsigned long long), st));
         k_shard_pull<<<dim3(s->GF.n_sb, 8), 256, 0, st>>>(s->geom, src, PP, BKT_SHIFT + s->GF.L.sb_shift,
                                                          (uint32_t)((uint64_t)s->rank * s->max_positions), stride, s->planes.p,
-                                                         &h->d_ctrl->overflow);
+                                                         &h->d_ctrl->overflow, 0ull);
         h->all_launches += 1;
         CK(cudaGetLastError());
         CKR(read_ctrl(h));
@@ -3728,10 +3805,137 @@ extern "C" int kmgpu_shard_pull(kmgpu_shard_t* s)
         k_shard_fold<<<(unsigned)std::min<uint32_t>((n_pos + 255) / 256, 148 * 16), 256, 0, st>>>(s->planes.p, s->nt, stride, n_pos,
                                                                                                    h->d_counts.p);
         h->all_launches += 1;
+        if (h->kind == BYTE && h->use_bigcount) {
+            CKR(sync_big_to_device(h));
+            if (h->n_big_dev) {
+                Input in = make_input(s->q);
+                const unsigned gb = (unsigned)std::min<uint32_t>((n_pos + 255) / 256, 148 * 16);
+                if (h->hash == MURMUR) {
+                    in.hashes = h->d_hash64.p;
+                    k_shard_bigcount<TWOBIT, 1><<<gb, 256, 0, st>>>(h->d_counts.p, in, h->k, h->big_keys.p, h->big_vals.p, h->n_big_dev);
+                } else {
+                    k_shard_bigcount<TWOBIT, 0><<<gb, 256, 0, st>>>(h->d_counts.p, in, h->k, h->big_keys.p, h->big_vals.p, h->n_big_dev);
+                }
+                h->all_launches += 1;
+            }
+        }
         CK(cudaGetLastError());
         CK(cudaStreamSynchronize(st));
     }
     s->pulled = true;
+    return KMGPU_OK;
+}
+
+// bigcount events (sender, ingest rounds): after every owner has applied the round, the k-mers of MY reads whose N bytes were all
+// 255 before they arrived.  The answers of the owners that marked their arenas are pulled, ANDed over the tables and aggregated per
+// k-mer; the list (one entry per distinct hash, in the order of its first event) is kept until the next route.
+static int shard_bigcount_events(kmgpu_shard* s)
+{
+    kmgpu_sketch* h = s->local;
+    cudaStream_t st = h->stream;
+    constexpr uint64_t WS_MIN = 1ull << 20;
+    s->big_ev.clear();
+    const uint32_t n_pos = s->q.n_pos;
+    if (n_pos == 0) return KMGPU_OK;
+    unsigned long long fl[MAX_WORLD];
+    for (int q = 0; q < s->world; q++) CK(cudaMemcpyAsync(&fl[q], s->peers[q].flags, 8, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));
+    bool any = false;
+    for (int q = 0; q < s->world; q++) any |= (fl[q] & 3ull) != 0;
+    if (!any) return KMGPU_OK;   // no owner marked anything, and none refused the round
+    const uint64_t stride = s->max_positions;
+    if (!try_ensure(s->planes, (size_t)s->nt * stride)) return fail(KMGPU_ENOMEM, "no room for the bigcount answers of a round");
+    CK(cudaMemset2DAsync(s->planes.p, stride, 0, n_pos, s->nt, st));   // positions whose owners marked nothing stay 0
+    ShardPeers PP;
+    shard_peers(s, &PP);
+    const Store src = s->exact_s ? Store{s->rec_s.p, s->off_s.p, s->cur_s.p, 0, 0} : Store{s->rec_s.p, nullptr, s->cur_s.p, s->GF.L.cap1, 0};
+    CK(cudaMemsetAsync(&h->d_ctrl->overflow, 0, sizeof(unsigned long long), st));
+    k_shard_pull<<<dim3(s->GF.n_sb, 8), 256, 0, st>>>(s->geom, src, PP, BKT_SHIFT + s->GF.L.sb_shift, (uint32_t)((uint64_t)s->rank * s->max_positions),
+                                                     stride, s->planes.p, &h->d_ctrl->overflow, 2ull);
+    h->all_launches += 1;
+    CK(cudaGetLastError());
+    CKR(read_ctrl(h));
+    if (h->h_ctrl->overflow)
+        return fail(KMGPU_ENOMEM, "rank %d: an owner's arena could not hold this round (see its kmgpu_shard_apply): no bigcount events", s->rank);
+    CKR(h->d_counts.ensure(n_pos));
+    const unsigned gp = (unsigned)std::min<uint32_t>((n_pos + 255) / 256, 148 * 16);
+    k_shard_fold<<<gp, 256, 0, st>>>(s->planes.p, s->nt, stride, n_pos, h->d_counts.p);
+    h->all_launches += 1;
+    Input in = make_input(s->q);
+    if (h->hash == MURMUR) in.hashes = h->d_hash64.p;   // the route's hashes: nothing restages or rehashes before the next route
+    unsigned long long* n_ctr = &h->d_ctrl->n_events;
+    uint64_t n_rec = 0;
+    for (int pass = 0; pass < 2; pass++) {   // the event buffer grows (and the pass runs again) when the events do not fit
+        CKR(h->d_events.ensure(std::max<uint64_t>(n_rec, WS_MIN)));
+        CK(cudaMemsetAsync(n_ctr, 0, sizeof(unsigned long long), st));
+        if (h->hash == MURMUR) k_shard_events<TWOBIT, 1><<<gp, 256, 0, st>>>(h->d_counts.p, in, h->k, h->d_events.p, h->d_events.cap, n_ctr);
+        else k_shard_events<TWOBIT, 0><<<gp, 256, 0, st>>>(h->d_counts.p, in, h->k, h->d_events.p, h->d_events.cap, n_ctr);
+        h->all_launches += 1;
+        CK(cudaGetLastError());
+        CKR(read_ctrl(h));
+        n_rec = h->h_ctrl->n_events;
+        if (n_rec <= h->d_events.cap) break;
+    }
+    if (n_rec > h->d_events.cap) return fail(KMGPU_ECUDA, "internal: bigcount events overflowed");
+    if (n_rec == 0) return KMGPU_OK;
+    // aggregate per k-mer: count and first position (as the single sketch's resolution does)
+    const uint64_t evslots = pow2_at_least(2 * n_rec);
+    CKR(h->d_evkeys.ensure(std::max<uint64_t>(evslots, WS_MIN)));
+    CKR(h->d_evvals.ensure(std::max<uint64_t>(2 * evslots, 2 * WS_MIN)));
+    CK(cudaMemsetAsync(h->d_evkeys.p, 0xFF, evslots * 8, st));
+    CK(cudaMemsetAsync(h->d_evvals.p, 0, evslots * 4, st));
+    CK(cudaMemsetAsync(h->d_evvals.p + evslots, 0xFF, evslots * 4, st));
+    CK(cudaMemsetAsync(&h->d_ctrl->n_unique, 0, sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(n_ctr, 0, sizeof(unsigned long long), st));
+    EvTable ev{h->d_evkeys.p, h->d_evvals.p, h->d_evvals.p + evslots, evslots - 1};
+    k_ev_decide<<<(unsigned)((n_rec + 255) / 256), 256, 0, st>>>(h->d_events.p, n_rec, h->nt, nullptr, nullptr, 0, ev, h->d_ctrl);
+    h->all_launches += 1;
+    CK(cudaGetLastError());
+    CKR(read_ctrl(h));
+    const uint64_t n_distinct = h->h_ctrl->n_unique;
+    CKR(h->d_evout.ensure(std::max<uint64_t>(n_distinct, WS_MIN / 4)));
+    CKR(h->h_evout.ensure(std::max<uint64_t>(n_distinct, WS_MIN / 4)));
+    k_ev_compact<<<(unsigned)((evslots + 255) / 256), 256, 0, st>>>(ev, h->d_evout.p, h->d_ctrl);
+    h->all_launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h->h_evout.p, h->d_evout.p, n_distinct * sizeof(EvOut), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    s->big_ev.assign(h->h_evout.p, h->h_evout.p + n_distinct);
+    std::sort(s->big_ev.begin(), s->big_ev.end(), [](const EvOut& a, const EvOut& b) { return a.first < b.first; });
+    return KMGPU_OK;
+}
+
+extern "C" int kmgpu_shard_bigcount_events(kmgpu_shard_t* s, uint64_t* hashes, uint32_t* counts, uint64_t cap, uint64_t* n_out)
+{
+    if (!s || !n_out) return fail(KMGPU_EINVAL, "null argument");
+    *n_out = 0;
+    kmgpu_sketch* h = s->local;
+    std::lock_guard<std::mutex> g(h->mu);
+    if (!(h->kind == BYTE && h->use_bigcount)) return fail(KMGPU_EINVAL, "bigcount is off on this shard");
+    if (hashes && !counts) return fail(KMGPU_EINVAL, "null counts");
+    CKR(set_device(h->device));
+    if (!s->big_ev_ready) {
+        CKR(shard_bigcount_events(s));
+        s->big_ev_ready = true;
+    }
+    const uint64_t n = s->big_ev.size();
+    for (uint64_t i = 0; hashes && i < n && i < cap; i++) {
+        hashes[i] = s->big_ev[i].hash;
+        counts[i] = s->big_ev[i].count;
+    }
+    *n_out = n;
+    return KMGPU_OK;
+}
+
+// the events of every rank, concatenated in rank order: new keys enter the map in the order of their first event in the stream
+extern "C" int kmgpu_shard_bigcount_apply(kmgpu_shard_t* s, const uint64_t* hashes, const uint32_t* counts, uint64_t n)
+{
+    if (!s) return fail(KMGPU_EINVAL, "null shard");
+    if (n && (!hashes || !counts)) return fail(KMGPU_EINVAL, "null input");
+    kmgpu_sketch* h = s->local;
+    if (h->kind != BYTE) return fail(KMGPU_EUNSUPPORTED, "bigcount is not supported for this storage.");
+    std::lock_guard<std::mutex> g(h->mu);
+    for (uint64_t i = 0; i < n; i++) big_events(h, hashes[i], std::min<uint32_t>(counts[i], 65535u));
     return KMGPU_OK;
 }
 

@@ -611,7 +611,7 @@ k_apply2(const __grid_constant__ SketchDev S, const __grid_constant__ GroupLayou
                 }
             }
             *reinterpret_cast<uint64_t*>(slice + (size_t)g * 8) = new64;
-            if (want_cross && fullm) {
+            if (want_cross && fullm && sb.t[t]) {   // (address-sharded owners keep no bitmaps)
                 unsigned m = 0;
 #pragma unroll
                 for (int j = 0; j < 8; j++) m |= (unsigned)(((new64 >> (8 * j)) & 255u) == 255u) << j;
@@ -822,7 +822,7 @@ k_apply_sparse(const __grid_constant__ SketchDev S, const __grid_constant__ Grou
                         if (at < list_cap) binlist[at] = BL_CROSS | ((unsigned long long)before[j] << 48) | ht_key(bin[j], t);
                     }
                 }
-                if (want_cross && tt >= 255u) atomicOr(reinterpret_cast<uint32_t*>(sb.t[t]) + (bin[j] >> 5), 1u << (bin[j] & 31));
+                if (want_cross && tt >= 255u && sb.t[t]) atomicOr(reinterpret_cast<uint32_t*>(sb.t[t]) + (bin[j] >> 5), 1u << (bin[j] & 31));
             }
             if (before[j] == 0) {
                 n_new++;
@@ -1424,10 +1424,11 @@ k_shard_lookup(const __grid_constant__ ShardGeom G, const __grid_constant__ Sket
 }
 
 // sender: grid (global super-buckets, Y), the runs the push wrote; answers land in one byte plane per table (plain stores: every
-// (table, position) has exactly one record).  A run whose owner refused the round sets *refused and is not read.
+// (table, position) has exactly one record).  A run whose owner refused the round sets *refused and is not read; a run whose
+// owner's flags lack one of the bits of `need` is not read either (bigcount events: owners that marked nothing).
 __global__ void __launch_bounds__(256)
 k_shard_pull(const __grid_constant__ ShardGeom G, Store src, const __grid_constant__ ShardPeers P, int sb_bin_shift, uint32_t pos_base,
-             uint64_t plane_stride, uint8_t* __restrict__ planes, unsigned long long* refused)
+             uint64_t plane_stride, uint8_t* __restrict__ planes, unsigned long long* refused, unsigned long long need)
 {
     const uint32_t g = blockIdx.x;
     uint32_t c = src.cursor[g];
@@ -1437,10 +1438,12 @@ k_shard_pull(const __grid_constant__ ShardGeom G, Store src, const __grid_consta
     int q;
     uint32_t j;
     shard_owner(G, g, &q, &j);
-    if (*P.flags[q] & 1ull) {
+    const unsigned long long fl = *P.flags[q];
+    if (fl & 1ull) {
         if (blockIdx.y == 0 && threadIdx.x == 0) atomicOr(refused, 1ull);
         return;
     }
+    if ((fl & need) != need) return;
     int t = 0;
 #pragma unroll 1
     for (int i = 1; i < G.n_tables; i++)
@@ -1461,6 +1464,133 @@ __global__ void k_shard_fold(const uint8_t* __restrict__ planes, int n_tables, u
         uint32_t m = planes[p];
         for (int t = 1; t < n_tables; t++) m = min(m, (uint32_t)planes[(size_t)t * plane_stride + p]);
         counts[p] = (uint16_t)m;
+    }
+}
+
+// ---- bigcount in sharded rounds (ByteStorage::add, storage.hh:606-617).  A touch is a bigcount event iff all N of its bytes were
+//      255 before it, in the order of global positions.  Each owner answers that for its own bins (k_shard_satmark, in place as
+//      k_shard_lookup does: 1 = "this byte was 255 before this touch"); the sender ANDs the answers over the tables (k_shard_pull +
+//      k_shard_fold: min 1) and aggregates its events per k-mer (k_shard_events, then k_ev_decide / k_ev_compact).
+
+// owner: (global position, crossing-bin slot) of every received record whose bin reached 255 in this round, for the radix select
+// of the saturating touch (k_sel_init / k_sel_count_pairs / k_sel_update).  Grid (local super-buckets, Y).
+__global__ void __launch_bounds__(256)
+k_shard_sel_pairs(const __grid_constant__ ShardGeom G, const unsigned long long* __restrict__ arena, const unsigned long long* __restrict__ sb_off,
+                  const uint32_t* __restrict__ sb_cnt, int sb_bin_shift, const uint64_t* __restrict__ keys, uint64_t mask, uint2* __restrict__ out,
+                  unsigned long long cap, unsigned long long* n_out)
+{
+    const uint32_t j = blockIdx.x;
+    const uint32_t c = sb_cnt[j];
+    if (c == 0) return;
+    int t = 0;
+#pragma unroll 1
+    for (int i = 1; i < G.n_tables; i++)
+        if (j >= G.local_first[i]) t = i;
+    const unsigned long long bmask = (1ull << sb_bin_shift) - 1;
+    const uint64_t bin0 = (uint64_t)(j - G.local_first[t]) << sb_bin_shift;
+    const unsigned long long* rec = arena + sb_off[j];
+    const uint32_t lane = threadIdx.x & 31;
+    for (uint32_t e0 = blockIdx.y * 256u; e0 < c; e0 += gridDim.y * 256u) {   // uniform per warp: one reservation per warp
+        const uint32_t e = e0 + threadIdx.x;
+        unsigned long long r = 0;
+        uint64_t sl = ~0ull;
+        if (e < c) {
+            r = rec[e];
+            sl = ht_find(keys, mask, ht_key(bin0 | (r & bmask), t));
+        }
+        const unsigned m = __ballot_sync(0xffffffffu, sl != ~0ull);
+        if (!m) continue;
+        const int lead = __ffs(m) - 1;
+        unsigned long long at = 0;
+        if ((int)lane == lead) at = atomicAdd(n_out, (unsigned long long)__popc(m));
+        at = __shfl_sync(0xffffffffu, at, lead) + __popc(m & ((1u << lane) - 1u));
+        if (sl != ~0ull && at < cap) out[at] = make_uint2((uint32_t)(r >> sb_bin_shift), (uint32_t)sl);
+    }
+}
+
+// k_sel_count over (position, slot) pairs
+__global__ void k_sel_count_pairs(const uint2* __restrict__ pairs, uint64_t n, int bit, SelState st)
+{
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint2 pr = pairs[i];
+    if ((pr.x >> bit) & 1u) return;
+    if (bit == 31 || (pr.x >> (bit + 1)) == (st.prefix[pr.y] >> (bit + 1))) atomicAdd(&st.cnt[pr.y], 1u);
+}
+
+// owner, after the apply: every record's low bits become 1 iff its byte was 255 before it arrived — the byte is 255 now and either
+// did not cross in this round or crossed at an earlier touch (position > T of its slot).  Position bits stay.
+__global__ void __launch_bounds__(256)
+k_shard_satmark(const __grid_constant__ ShardGeom G, const __grid_constant__ SketchDev S, unsigned long long* __restrict__ arena,
+                const unsigned long long* __restrict__ sb_off, const uint32_t* __restrict__ sb_cnt, int sb_bin_shift, const uint64_t* __restrict__ keys,
+                uint64_t mask, const uint32_t* __restrict__ T, int have_cross)
+{
+    const uint32_t j = blockIdx.x;
+    const uint32_t c = sb_cnt[j];
+    if (c == 0) return;
+    int t = 0;
+#pragma unroll 1
+    for (int i = 1; i < G.n_tables; i++)
+        if (j >= G.local_first[i]) t = i;
+    const unsigned long long bmask = (1ull << sb_bin_shift) - 1;
+    const uint64_t bin0 = (uint64_t)(j - G.local_first[t]) << sb_bin_shift;
+    const uint8_t* tab = S.tables[t];
+    unsigned long long* rec = arena + sb_off[j];
+    const uint32_t step = gridDim.y * 256u;
+    for (uint32_t e0 = blockIdx.y * 256u + threadIdx.x; e0 < c; e0 += 4 * step) {   // four random table loads in flight per thread
+        unsigned long long r[4];
+        uint32_t v[4];
+#pragma unroll
+        for (int u = 0; u < 4; u++) r[u] = e0 + u * step < c ? rec[e0 + u * step] : 0ull;
+#pragma unroll
+        for (int u = 0; u < 4; u++) v[u] = e0 + u * step < c ? tab[bin0 | (r[u] & bmask)] : 0u;
+#pragma unroll
+        for (int u = 0; u < 4; u++) {
+            if (e0 + u * step >= c) continue;
+            unsigned long long sat = v[u] == 255u;
+            if (sat && have_cross) {
+                const uint64_t sl = ht_find(keys, mask, ht_key(bin0 | (r[u] & bmask), t));
+                if (sl != ~0ull) sat = (uint32_t)(r[u] >> sb_bin_shift) > T[sl];
+            }
+            rec[e0 + u * step] = (r[u] & ~bmask) | sat;
+        }
+    }
+}
+
+// sender: an Event for every position whose touches all found their bytes saturated (counts[p] == 1 after the fold); position p is
+// relative to this rank's reads, so that the first event of a k-mer is its first in stream order
+template <int HK, int SRC>
+__global__ void __launch_bounds__(256)
+k_shard_events(const uint16_t* __restrict__ counts, Input in, int k, Event* __restrict__ out, unsigned long long cap, unsigned long long* n_out)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    for (uint32_t p0 = blockIdx.x * 256u; p0 < in.n_pos; p0 += gridDim.x * 256u) {
+        const uint32_t p = p0 + threadIdx.x;
+        const bool ev = p < in.n_pos && counts[p] != 0;
+        const unsigned m = __ballot_sync(0xffffffffu, ev);
+        if (!m) continue;
+        const int lead = __ffs(m) - 1;
+        unsigned long long at = 0;
+        if ((int)lane == lead) at = atomicAdd(n_out, (unsigned long long)__popc(m));
+        at = __shfl_sync(0xffffffffu, at, lead) + __popc(m & ((1u << lane) - 1u));
+        if (ev && at < cap) {
+            Event e;
+            e.hash = hash_at<HK, SRC>(in, k, p);
+            e.pos = p;
+            e.info = 1u << 30;   // all bytes saturated, no crossing bins left to check (k_ev_decide)
+            out[at] = e;
+        }
+    }
+}
+
+// sender, query rounds with bigcount: a k-mer counted 255 takes its value from the bigcount map when the map holds it
+template <int HK, int SRC>
+__global__ void k_shard_bigcount(uint16_t* __restrict__ counts, Input in, int k, const uint64_t* __restrict__ big_keys,
+                                 const uint16_t* __restrict__ big_vals, uint32_t n_big)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < in.n_pos; p += gridDim.x * blockDim.x) {
+        if (counts[p] != 255u || !((in.valid[p >> 5] >> (p & 31)) & 1u)) continue;   // (the planes of other positions are stale)
+        counts[p] = (uint16_t)big_lookup(big_keys, big_vals, n_big, hash_at<HK, SRC>(in, k, p), 255u);
     }
 }
 

@@ -190,6 +190,18 @@ struct Event {
     uint32_t info;  // crossmask | allsat_after << 30
 };
 
+// the value of k-mer h in the sorted device copy of the bigcount map (storage.hh:640-647); c when the map does not hold it
+__device__ __forceinline__ uint32_t big_lookup(const uint64_t* __restrict__ big_keys, const uint16_t* __restrict__ big_vals, uint32_t n_big,
+                                               uint64_t h, uint32_t c)
+{
+    uint32_t lo = 0, hi = n_big;
+    while (lo < hi) {
+        uint32_t mid = (lo + hi) >> 1;
+        if (big_keys[mid] < h) lo = mid + 1; else hi = mid;
+    }
+    return lo < n_big && big_keys[lo] == h ? big_vals[lo] : c;
+}
+
 // ---- queries ---------------------------------------------------------------------------------------
 // Storage::get_count per position (min over tables; saturated bytes looked up in the sorted device copy
 // of the bigcount map, storage.hh:640-647), optionally also the hash.
@@ -221,14 +233,7 @@ k_counts(SketchDev S, HashCfg H, Input in, const uint64_t* __restrict__ big_keys
 #pragma unroll
             for (int j = 0; j < 4; j++) mn = c[j] < mn ? c[j] : mn;
         }
-        if (KIND == BYTE && mn == 255u && n_big && t_hi == S.n_tables) {
-            uint32_t lo = 0, hi = n_big;
-            while (lo < hi) {
-                uint32_t mid = (lo + hi) >> 1;
-                if (big_keys[mid] < h) lo = mid + 1; else hi = mid;
-            }
-            if (lo < n_big && big_keys[lo] == h) mn = big_vals[lo];
-        }
+        if (KIND == BYTE && mn == 255u && n_big && t_hi == S.n_tables) mn = big_lookup(big_keys, big_vals, n_big, h, mn);
         counts[p] = (uint16_t)mn;
     }
 }

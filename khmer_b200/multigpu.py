@@ -263,12 +263,18 @@ class ShardedGroup:
     over NVLink peer memory (push), owners apply what they received (apply); every rank counts which of its k-mers were new
     (count_new).  A query round takes the same first three steps, then the owners answer every record with its counter in place
     (lookup) and the senders read the answers back, keeping the minimum over the tables per k-mer (pull).  Only the barriers
-    between the phases come from `comm`."""
+    between the phases come from `comm`.
+
+    With bigcount on (set_use_bigcount, ByteStorage), an ingest round also lists, on every rank, its k-mers whose N bytes were
+    all 255 before they arrived (bigcount_events); the ranks exchange the lists and every rank applies all of them in rank order,
+    so every rank holds the bigcount map of one sketch fed the rounds in stream order."""
 
     def __init__(self, shard, comm=None, device=None):
         self.shard = shard
         self.comm = _as_comm(comm, device)
         self.rank, self.world = self.comm.rank, self.comm.world
+        get = getattr(shard, "get_use_bigcount", None)
+        self.bigcount = bool(get()) if get else False   # the ranks' common setting (set_use_bigcount)
 
     def barrier(self):
         self.comm.barrier()
@@ -289,6 +295,20 @@ class ShardedGroup:
         empty = (np.zeros(0, dtype=np.uint8), np.zeros(1, dtype=np.uint64))
         return [(buf, off[r0:r1 + 1]) for r0, r1 in runs] + [empty] * (rounds - len(runs))
 
+    def set_use_bigcount(self, on):
+        """Collective: bigcount on or off for the whole sketch from the next round on.  Every rank must pass the same value;
+        if they disagree, every rank raises and nothing changes."""
+        on = bool(on)
+        votes = [bool(p[0]) for p in self.comm.all_gather_bytes(bytes([on]))]
+        if len(set(votes)) > 1:
+            raise ValueError("set_use_bigcount: the ranks disagree (%s)" % ", ".join("rank %d: %s" % (r, v) for r, v in enumerate(votes)))
+        self.shard.set_use_bigcount(on)
+        self.bigcount = on
+
+    def bigcounts(self):
+        """The bigcount map, identical on every rank, in its iteration order (that of a .ct file's trailer): (hashes, counts)."""
+        return self.shard.bigcounts()
+
     def _ingest_round(self, run, clean):
         n = self.shard.route(run, clean=clean)
         self.barrier()          # every owner knows what it will be sent
@@ -296,11 +316,47 @@ class ShardedGroup:
         self.barrier()          # every sender can read where its runs go
         self.shard.push()
         self.barrier()          # every update of this round sits in its owner's arena
-        self.shard.apply()
-        self.barrier()          # every owner has marked the new positions of the round
+        if not self.bigcount:
+            self.shard.apply()
+            self.barrier()      # every owner has marked the new positions of the round
+            self.shard.count_new()
+            self.barrier()      # nobody reads a peer's bitmap or store any more: the next round may start
+            return n
+        from . import cabi
+        err = None
+        try:
+            self.shard.apply()
+        except cabi.KmgpuError as e:
+            err = e
+        # (also the barrier after apply: every owner has marked the new positions and the saturated touches of the round)
+        if self.comm.all_reduce_sum(err is not None):
+            raise err or cabi.KmgpuError(4, "another rank's arena could not hold this round")
         self.shard.count_new()
-        self.barrier()          # nobody reads a peer's bitmap or store any more: the next round may start
+        self._exchange_bigcount()
         return n
+
+    def _exchange_bigcount(self):
+        """every rank's events of the round -> every rank, applied in rank order.  The exchange is also the barrier that ends
+        the round: nobody reads a peer's store any more."""
+        from . import cabi
+        hashes, counts = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+        err = None
+        try:
+            hashes, counts = self.shard.bigcount_events()
+        except cabi.KmgpuError as e:
+            err = e
+        heads = [struct.unpack("<qq", p) for p in self.comm.all_gather_bytes(struct.pack("<qq", len(hashes), err is not None))]
+        if any(failed for _, failed in heads):
+            raise err or cabi.KmgpuError(4, "another rank could not read the bigcount marks of this round")
+        most = max(n for n, _ in heads)
+        if most == 0:
+            return
+        # equal lengths on every rank (TorchComm gathers equal-sized tensors)
+        blob = hashes.tobytes() + counts.tobytes()
+        parts = self.comm.all_gather_bytes(blob + bytes(12 * most - len(blob)))
+        hs = [np.frombuffer(p, dtype=np.uint64, count=n) for p, (n, _) in zip(parts, heads)]
+        cs = [np.frombuffer(p, dtype=np.uint32, count=n, offset=8 * n) for p, (n, _) in zip(parts, heads)]
+        self.shard.bigcount_apply(np.concatenate(hs), np.concatenate(cs))
 
     def _query_round(self, run, clean):
         """route | offsets | push | lookup | pull: afterwards the shard's getters answer for `run`.  A round an owner refused
