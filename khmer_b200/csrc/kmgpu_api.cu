@@ -1217,10 +1217,22 @@ static int ingest_chunk(kmgpu_sketch* h, int src, HashCfg H, const std::vector<P
     GroupPlan G;   // the regions are sized for this chunk's positions
     if (path == Path::Choose) path = choose_path(h, n_pos, h->ft_on, &G);
     else if (path == Path::Grouped && !plan_group(h, n_pos, &G)) return fail(KMGPU_ECUDA, "internal: grouped plan changed between chunks");
-    if (path == Path::Grouped) return ingest_chunk_grouped(h, G, src, H, parts, P, pred, M, res, between);
+    static const bool dbg = env_u64("KMGPU_DEBUG", 0) != 0;
+    if (path == Path::Grouped) {
+        if (dbg)
+            fprintf(stderr, "[kmgpu] chunk: path=grouped delta_blocks=0 levels=%d sb_shift=%d apply=%s n_pos=%u\n", G.L.two_level ? 2 : 1,
+                    G.L.two_level ? (int)G.L.sb_shift : 0, G.sparse ? "sparse" : G.split == 4 ? "split4" : G.split == 2 ? "split2" : "dense", n_pos);
+        return ingest_chunk_grouped(h, G, src, H, parts, P, pred, M, res, between);
+    }
     std::vector<DeltaPass> dp;
     if (path == Path::Unsupported || !plan_delta(h, dp))
         return fail(KMGPU_EUNSUPPORTED, "no ingestion path can take this sketch (%d tables; more than %d need the grouped path)", h->nt, F_MAXT);
+    if (dbg) {
+        BucketLayout BL;   // ingest_chunk_delta takes the bins path whenever the buckets can be planned
+        const bool bins = plan_buckets(h, n_pos, &BL);
+        fprintf(stderr, "[kmgpu] chunk: path=%s delta_blocks=%zu levels=0 sb_shift=0 apply=- n_pos=%u\n", bins ? "bins" : "delta", bins ? (size_t)0 : dp.size(),
+                n_pos);
+    }
     return ingest_chunk_delta(h, dp, src, H, parts, P, pred, M, res, between);
 }
 
